@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path on the host cores
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR  # also write B / residual / band sums of the last timed pass
 
 A step is ONE gather pass (residual <- M (F residual); B += residual, reference Lightning.h:196-226) over the
 resident dense FP32 form-factor matrix of the workload.  Before the timed passes the matrix is built by the fused
@@ -44,6 +45,14 @@ WORKLOADS = {
 FIXTURE_SCENES = ("cornellbox_blacklight", "colorballs")
 # the matrix depends on the geometry only: workloads that differ in bands / materials share the committed digests and ncu captures
 SAME_MATRIX_AS = {"fluor_32k_k16": "cornell_32k"}
+
+
+def row_digest32(wsum):
+    """One uint32 per matrix row, as committed in tests/golden/rowdigest_<workload>.npz: the low 32 bits of the device's
+    position-weighted sum of the row's bit patterns (sum of bits_c * (2c + 1) mod 2^64).  Every weight is odd, hence invertible
+    mod 2^32, so a change of any single entry always changes it; 4 bytes per row keep the largest workload's file under 1 MB.
+    The device's xor digest is not used: xor-ing it in lets the two cancel for a one-ulp change of the same entry."""
+    return (np.asarray(wsum, np.uint64) & np.uint64(0xFFFFFFFF)).astype(np.uint32)
 
 
 def parity_rows(N):
@@ -292,8 +301,8 @@ def parity_block(optixP, solver, sc, uv, E, M, K, world, rank, torch, name, stop
     dpath = os.path.join(ROOT, "tests", "golden", f"rowdigest_{SAME_MATRIX_AS.get(name, name)}.npz")
     if os.path.exists(dpath) and r1 > r0:
         g = np.load(dpath)
-        dx, dw = rm.row_digest()
-        bad = int(np.count_nonzero((dx != g["xor"][r0:r1]) | (dw != g["wsum"][r0:r1])))
+        _, dw = rm.row_digest()
+        bad = int(np.count_nonzero(row_digest32(dw) != g["digest"][r0:r1]))
         out["digest"] = {"file": os.path.relpath(dpath, ROOT), "rows_checked": int(allsum(r1 - r0)), "row_mismatches": int(allsum(bad))}
     elif os.path.exists(dpath):
         out["digest"] = {"file": os.path.relpath(dpath, ROOT), "rows_checked": int(allsum(0)), "row_mismatches": int(allsum(0))}
@@ -407,6 +416,30 @@ def optixP_rows_per_rank(optixP):
     return n.value
 
 
+def dump_outputs(out_dir, optixP, solver, K, N, world, rank, torch):
+    """Writes what a caller of the solver receives after the last timed pass: B.npy and residual.npy (K x N float32, every
+    patch, gathered from all ranks) and band_sums.npy (K float64).  The inputs are fixed by the workload, so two builds run
+    with the same arguments can be compared array for array.  The largest workload (65536 patches, K = 32) writes 16 MB."""
+    B, R = solver.read_local()
+    sums = solver.band_sums()
+    if world > 1:
+        n = optixP_rows_per_rank(optixP)
+
+        def gather(X):
+            mine = torch.zeros((K, n), dtype=torch.float32, device="cuda")
+            mine[:, :X.shape[1]] = torch.from_numpy(X).cuda()
+            parts = [torch.empty_like(mine) for _ in range(world)]
+            torch.distributed.all_gather(parts, mine)
+            return torch.cat(parts, 1)[:, :N].cpu().numpy()
+
+        B, R = gather(B), gather(R)
+    if rank == 0:
+        assert B.nbytes + R.nbytes + sums.nbytes <= 64 << 20
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in (("B", B), ("residual", R), ("band_sums", sums)):
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -499,6 +532,8 @@ def run_ours(args):
     ms_total = allmax(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     value = 1e3 / ms_step
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, optixP, solver, K, N, world, rank, torch)
     if chained:
         _lib.check(L.daisy_solver_set_chained(solver._s, 0))
 
@@ -718,7 +753,12 @@ def main():
     ap.add_argument("--no-chained", action="store_true", help="one GPU: per-pass events and plain stream order between passes (no programmatic dependent launch)")
     ap.add_argument("--no-fused", action="store_true", help="multi-GPU: NCCL all-gather per pass instead of the epilogue kernel's peer stores")
     ap.add_argument("--no-peer-tiles", action="store_true", help="multi-GPU: trace every tile touching this rank's rows instead of exchanging mirrored tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write B, residual and band sums after the last timed pass as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

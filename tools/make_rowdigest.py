@@ -18,9 +18,9 @@ for name in sys.argv[1:]:
     uv = dz.msvc_sample_pattern(1)
     p = dz.OptixPrimeFunctionality(dz.MeshS.from_scene(sc), rands=uv)
     rm = p.cudaCalculateRadiosityMatrix()
-    x, w = rm.row_digest()
+    _, w = rm.row_digest()
     st = p.stats()
     out = os.path.join("gpurun_out", f"rowdigest_{name}.npz")
-    np.savez_compressed(out, xor=x, wsum=w, pairs=np.int64(st["pairs_traced"]), patches=np.int64(sc.numtriangles))
+    np.savez_compressed(out, digest=bench.row_digest32(w), pairs=np.int64(st["pairs_traced"]), patches=np.int64(sc.numtriangles))
     print(name, "pairs", st["pairs_traced"], "ff_ms %.1f" % st["ff_ms"], "->", out, os.path.getsize(out), "bytes", flush=True)
     p.close()
