@@ -74,6 +74,8 @@ SYMBOLS = {
     "daisy_solver_write_partitioned": (_i, [_vp, _fp, _fp]),
     "daisy_solver_write_slices": (_i, [_vp, _fp, _fp]),
     "daisy_solver_launches_per_pass": (_i, [_vp]),
+    "daisy_solver_tile_map": (_i, [_vp, _ip, C.POINTER(C.c_uint8), C.c_int64, _i64p, _dp]),
+    "daisy_gather_plan_dump": (_i, [C.POINTER(C.c_uint8), _i, _i, _i, _ip, _ip, _ip, _ip, C.c_int64]),
     "daisy_group_create": (_i, [_fp, _i, _fp, _i, _ip, _i, _ip, _i, C.POINTER(_vp)]),
     "daisy_group_destroy": (None, [_vp]),
     "daisy_group_size": (_i, [_vp]),

@@ -484,6 +484,7 @@ extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     if (rc) return rc;
     if (timing) fprintf(stderr, "daisy_formfactors_build: tile list + kernel + clean-up %.3f s (kernel %.3f s)\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t1).count(), ctx->ff_ms * 1e-3);
     ctx->have_F = true;
+    ctx->F_version++;
     return DAISY_OK;
 }
 
@@ -565,6 +566,7 @@ extern "C" int daisy_formfactors_write_rows(daisy_ctx *ctx, int row0, int nrows,
                                   sizeof(float) * (size_t)ctx->N, (size_t)nrows, cudaMemcpyHostToDevice, ctx->stream));
     DZ_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->have_F = true;
+    ctx->F_version++;
     return DAISY_OK;
 }
 

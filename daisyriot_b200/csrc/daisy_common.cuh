@@ -313,6 +313,7 @@ struct daisy_ctx {
     float *d_F = nullptr; // (row1-row0) x ldF
     int64_t ldF = 0;
     bool have_F = false;
+    uint64_t F_version = 0;         // bumped by every write of F through this library (a solver rescans its tile map when it changes)
     float *peerF[16] = { nullptr }; // every rank's F (own pointer or CUDA-IPC mapping), set by daisy_formfactors_set_peers
     bool peers_set = false;
     bool peers_ipc = false;         // the peer pointers are CUDA-IPC mappings this context has to close (one process per GPU)

@@ -49,6 +49,17 @@ struct daisy_solver {
     unsigned long long timeout_ns = 30000000000ull;                  // how long a pass waits for a peer's block (DAISY_EXCHANGE_TIMEOUT_MS)
     int R = 8, nsplit = 1, grid = 148, colw = 0;
     int sk_S = 0, sk_L = 0, sk_total = 0, sk_grid = 0, sk_maxp = 1; // stream-K decomposition of the fused TMA kernel (plan())
+    int partial_splits = 0;             // d_partial holds partial_splits x nloc x Kp floats
+    // tile skipping (fused K <= 9 kernel, DAISY_GATHER_SKIP=0 turns it off): the stream-K sequence holds only the F tiles with a
+    // non-zero entry.  d_sk_list = column step of every entry (-1: the single null entry of a row block without any), d_sk_off =
+    // nrb + 1 offsets of the row blocks' entries.  Rebuilt whenever ctx->F_version moves away from scanned_version.
+    bool skip = false;
+    uint64_t scanned_version = 0;
+    int *d_sk_list = nullptr, *d_sk_off = nullptr;
+    int64_t sk_list_cap = 0;
+    std::vector<unsigned char> occ;     // tile map of the last scan: nrb_tma x sk_S
+    int64_t occupied = 0;
+    double scan_ms = 0.0;
     bool use_tma = true;
     bool use_mma = false;               // K = 16 / 32: tcgen05 3xTF32 path (gather_mma.cuh)
     bool fused_epi = false;             // k_gather_tma does the epilogue (and the exchange wait) itself: one launch per pass
@@ -133,14 +144,17 @@ struct GatherParams {
     // gets the same number of steps whatever the matrix shape, and a row block is shared by at most a few CTAs ("pieces")
     int sk;                 // 1: stream-K pieces, 0: (row block, column split) items
     int sk_S, sk_L, sk_total; // steps per row block, steps per CTA, steps in total
+    // tile skipping (sk_off != null): the sequence is the list of occupied tiles instead, sk_total entries, row block rb owning
+    // entries [sk_off[rb], sk_off[rb+1]) whose column steps are sk_list[]; CTA c streams the entries [c T / grid, (c+1) T / grid)
+    const int *sk_list, *sk_off;
     // L2 residency: the F tiles whose step number s has (s * 11 + rb * 5) % 16 < pin16 are loaded evict_last, the others
     // evict_first -- a fixed subset of the matrix, spread evenly over the CTAs, that stays in L2 from pass to pass when the
     // matrix is not much larger than L2 (the reference's own scenes: 164 / 238 MB against 126 MB of L2)
     int pin16;
 };
 
-// one unit of work of k_gather_tma: steps [s0, s1) of row block rb; idx / np = this piece's ordinal among / number of the
-// pieces that make up the row block (their partial sums are added in idx order)
+// one unit of work of k_gather_tma: steps [s0, s1) of row block rb (tile skipping: entries [s0, s1) of sk_list); idx / np =
+// this piece's ordinal among / number of the pieces that make up the row block (their partial sums are added in idx order)
 struct Piece { int rb, s0, s1, idx, np; };
 
 // stage the K bands of columns [j0, j0+w) of the exchange buffer into tile[k][0..w)
@@ -319,10 +333,74 @@ struct FusedEpi {
     unsigned long long timeout_ns;
 };
 
+// acquire flag[g] >= wait_seq: rank g's block of the previous pass has landed here and rank g has finished reading the buffer
+// this pass writes into.  A peer that does not show up within timeout_ns sets the abort markers instead.
+__device__ __forceinline__ void wait_flag(const FusedEpi &E, int g) {
+    unsigned long long t0, t1, v;
+    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0));
+    while (true) {
+        asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(E.flags + g) : "memory");
+        if (v >= E.wait_seq) break;
+        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1));
+        if (t1 - t0 > E.timeout_ns) {
+            E.flags[16] = E.seq;
+            if (E.host_abort) *reinterpret_cast<volatile unsigned long long *>(E.host_abort) = E.seq;
+            __threadfence_system();
+            break;
+        }
+        __nanosleep(100);
+    }
+}
 
-// the i-th piece of CTA `cta` (cursor: running position, start at 0); false when the CTA has no more work
+
+#ifdef __CUDA_ARCH__
+#define DZ_ASSERT_HD(cond) DZ_ASSERT(cond)
+#define DZ_LDG(p) __ldg(p)
+#else
+#define DZ_ASSERT_HD(cond) do { } while (0)
+#define DZ_LDG(p) (*(p))
+#endif
+// tile skipping: CTA c of ncta streams the entries [sk_bound(c), sk_bound(c+1)) -- lengths differ by at most one; sk_owner(e) is
+// the CTA whose range holds entry e
+__host__ __device__ __forceinline__ int sk_bound(int c, int T, int ncta) { return (int)((long long)c * T / ncta); }
+__host__ __device__ __forceinline__ int sk_owner(int e, int T, int ncta) { return (int)((((long long)e + 1) * ncta - 1) / T); }
+// column step of position e of a piece's range
+__device__ __forceinline__ int piece_step(const GatherParams &P, int e) {
+    const int s = P.sk_list ? __ldg(P.sk_list + e) : e;
+    DZ_ASSERT(s >= 0 && s < P.sk_S && (!P.sk_list || e < P.sk_total));
+    return s;
+}
+
+// the i-th piece of CTA `cta` (cursor: running position, start at 0; p: the piece the previous call returned); false when the
+// CTA has no more work.  Host-callable for daisy_gather_plan_dump.
 template <int T_COLS>
-__device__ __forceinline__ bool next_piece(const GatherParams &P, int cta, int ncta, int &cursor, Piece &p) {
+__host__ __device__ __forceinline__ bool next_piece(const GatherParams &P, int cta, int ncta, int &cursor, Piece &p) {
+    if (P.sk_off) {
+        const int c1 = sk_bound(cta + 1, P.sk_total, ncta), g0 = sk_bound(cta, P.sk_total, ncta) + cursor;
+        if (g0 >= c1) return false;
+        int rb;
+        if (cursor == 0) { // largest rb with sk_off[rb] <= g0
+            int lo = 0, hi = P.nrb - 1;
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (DZ_LDG(P.sk_off + mid) <= g0) lo = mid; else hi = mid - 1;
+            }
+            rb = lo;
+        } else {
+            rb = p.rb + 1; // a CTA's range is contiguous and every row block owns at least one entry
+        }
+        const int e0 = DZ_LDG(P.sk_off + rb), e1 = DZ_LDG(P.sk_off + rb + 1);
+        DZ_ASSERT_HD(rb >= 0 && rb < P.nrb && e0 <= g0 && g0 < e1 && e1 <= P.sk_total);
+        p.rb = rb;
+        p.s0 = g0;
+        p.s1 = e1 < c1 ? e1 : c1;
+        const int first = sk_owner(e0, P.sk_total, ncta);
+        p.idx = cta - first;
+        p.np = sk_owner(e1 - 1, P.sk_total, ncta) - first + 1;
+        cursor += p.s1 - p.s0;
+        if (DZ_LDG(P.sk_list + e0) < 0) p.s1 = p.s0; // the null entry of a row block without an occupied tile: nothing to stream
+        return true;
+    }
     if (P.sk) {
         const int g0 = cta * P.sk_L + cursor, g1 = min(P.sk_total, (cta + 1) * P.sk_L);
         if (g0 >= g1) return false;
@@ -384,10 +462,20 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
         const int et = tid - (NCW + 1) * 32, ewarp = et >> 5;
         auto esync = [&]() { asm volatile("bar.sync 1, 64;" ::: "memory"); };
         unsigned nitem_done = 0;
+        // fused exchange: the stores below go into the buffer every peer read in the previous pass.  The pieces of a row block
+        // need not have streamed a tile of every rank's block (tile skipping), so before its first peer store the CTA observes
+        // every rank's flag itself
+        bool flags_seen = E.npeers == 0 || E.wait_seq == 0ull;
         for (; next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cursor, pc); nitem_done++) {
             const int rb = pc.rb;
             const int buf = (int)(nitem_done & 1u);
             DZ_ASSERT(rb >= 0 && rb < P.nrb && pc.idx >= 0 && pc.idx < pc.np);
+            if (!flags_seen) {
+                if (et == 0)
+                    for (int g = 0; g < E.G; g++) wait_flag(E, g);
+                esync();
+                flags_seen = true;
+            }
             asm volatile("bar.sync %0, %1;" ::"r"(2 + buf), "n"(NCW * 32 + 64) : "memory"); // the consumers have written this item's sums
             bool last = true;
             if (pc.np > 1) {
@@ -517,7 +605,8 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
                 int cur2 = 0;
                 Piece p2;
                 while (pre < (uint32_t)NST && next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cur2, p2))
-                    for (int s = p2.s0; s < p2.s1 && pre < (uint32_t)NST; s++, pre++) {
+                    for (int e = p2.s0; e < p2.s1 && pre < (uint32_t)NST; e++, pre++) {
+                        const int s = piece_step(P, e);
                         mbar_expect_tx(&full[pre], (uint32_t)tma_stage_bytes<K>());
                         tma_load_2d_hint(stages + (size_t)pre * STAGE_F, &tmF, s * T_COLS, p2.rb * T_ROWS, &full[pre], pol(p2.rb, s));
                     }
@@ -525,8 +614,9 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
             asm volatile("griddepcontrol.wait;" ::: "memory");
             while (next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cursor, pc)) {
                 const int row0 = pc.rb * T_ROWS;
-                for (int s = pc.s0; s < pc.s1; s++, it++) {
+                for (int e = pc.s0; e < pc.s1; e++, it++) {
                     const int st = it % NST;
+                    const int s = piece_step(P, e);
                     const int col0 = s * T_COLS;
                     float *sf = stages + (size_t)st * STAGE_F;
                     if (it >= pre) {
@@ -537,20 +627,7 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
                     const int g = col0 / P.n, jl = col0 - g * P.n;
                     DZ_ASSERT(g >= 0 && g < 32 && col0 < P.ncols && row0 < P.nloc + T_ROWS);
                     if (!((ready >> g) & 1u)) {
-                        unsigned long long t0, t1, v;
-                        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0));
-                        while (true) {
-                            asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(E.flags + g) : "memory");
-                            if (v >= E.wait_seq) break;
-                            asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1));
-                            if (t1 - t0 > E.timeout_ns) {
-                                E.flags[16] = E.seq;
-                                if (E.host_abort) *reinterpret_cast<volatile unsigned long long *>(E.host_abort) = E.seq;
-                                __threadfence_system();
-                                break;
-                            }
-                            __nanosleep(100);
-                        }
+                        wait_flag(E, g);
                         ready |= 1u << g;
                         asm volatile("fence.proxy.async;" ::: "memory"); // the peer's stores, seen by the acquire above, before the TMA reads below
                     }
@@ -774,6 +851,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
     P.res = s->d_res[s->cur]; P.bstride = s->bstride; P.partial = s->d_partial;
     P.nsplit = s->nsplit; P.colw = s->colw; P.nrb = (s->nloc + G_WARPS * s->R - 1) / (G_WARPS * s->R);
     P.sk = 0; P.sk_S = P.sk_L = P.sk_total = 0; P.pin16 = 0;
+    P.sk_list = P.sk_off = nullptr;
     int rc;
     if (s->use_mma && (K == 16 || K == 32)) {
         if constexpr (K == 16 || K == 32) {
@@ -800,6 +878,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
         }
         P.nrb = (s->nloc + tma_rows<K>() - 1) / tma_rows<K>();
         P.sk = s->fused_epi ? 1 : 0; P.sk_S = s->sk_S; P.sk_L = s->sk_L; P.sk_total = s->sk_total;
+        if (s->skip) { P.sk_list = s->d_sk_list; P.sk_off = s->d_sk_off; }
         P.pin16 = s->pin16;
         const int grid = s->fused_epi ? s->sk_grid : s->grid;
         FusedEpi F;
@@ -867,7 +946,13 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
     return DAISY_OK;
 }
 
+static int scan_and_plan(daisy_solver *s);
+
 static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull) {
+    if (s->skip && s->scanned_version != s->ctx->F_version) { // F was written since the last scan (a host integer compare per pass)
+        int rc = scan_and_plan(s);
+        if (rc) return rc;
+    }
     switch (s->Kp) {
     case 1: return launch_pass_K<1>(s, wait_seq);
     case 3: return launch_pass_K<3>(s, wait_seq);
@@ -940,6 +1025,21 @@ static int make_maps(daisy_solver *s) {
     return DAISY_OK;
 }
 
+// L2 residency (GatherParams::pin16) for a pass that streams fbytes of F: keep ~45 % of the L2 filled with F tiles that are read
+// again next pass; the rest of the matrix streams through evict_first (which by itself is worth 9 % on the 164 MB matrix: the
+// stream no longer pushes the residual vectors out).  Measured on the reference's scenes (164 / 238 MB): best at 61 / 45 MB
+// pinned, worse from ~70 MB on (the two L2 halves mirror lines read from both dies).  DAISY_GATHER_PIN16 = 0..16 overrides.
+static int pin16_for(const daisy_solver *s, double fbytes) {
+    int l2 = 0;
+    cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, s->ctx->device);
+    int p16 = fbytes > 0.0 ? (int)floor(16.0 * 0.45 * (double)l2 / fbytes) : 0;
+    if (p16 > 16) p16 = 16;
+    if (p16 < 0) p16 = 0;
+    const char *e3 = getenv("DAISY_GATHER_PIN16");
+    if (e3) { p16 = atoi(e3); if (p16 < 0) p16 = 0; if (p16 > 16) p16 = 16; }
+    return p16;
+}
+
 // choose rows-per-warp and the column split so that (row blocks x splits) fills the persistent grid evenly
 static void plan(daisy_solver *s) {
     int sms = s->ctx->num_sms;
@@ -951,6 +1051,8 @@ static void plan(daisy_solver *s) {
     {
         const char *e2 = getenv("DAISY_GATHER_EPI"); // "split": keep the separate epilogue kernel (A/B switch)
         s->fused_epi = s->use_tma && !s->use_mma && !(e2 && strcmp(e2, "split") == 0);
+        const char *e4 = getenv("DAISY_GATHER_SKIP"); // "0": stream every tile of F (the dense plan, A/B switch)
+        s->skip = s->fused_epi && s->Kp <= 9 && !(e4 && strcmp(e4, "0") == 0);
     }
     int Rs[2];
     if (s->use_mma) { Rs[0] = Rs[1] = MM_ROWS / G_WARPS; } // 128-row tiles
@@ -988,22 +1090,108 @@ static void plan(daisy_solver *s) {
         s->sk_L = (s->sk_total + s->sk_grid - 1) / s->sk_grid;
         if (s->sk_L < 1) s->sk_L = 1;
         s->sk_maxp = s->sk_S / s->sk_L + 2;
-        // L2 residency (GatherParams::pin16): keep ~45 % of the L2 filled with F tiles that are read again next pass; the rest
-        // of the matrix streams through evict_first (which by itself is worth 9 % on the 164 MB matrix: the stream no longer
-        // pushes the residual vectors out).  Measured on the reference's scenes (164 / 238 MB): best at 61 / 45 MB pinned, worse
-        // from ~70 MB on (the two L2 halves mirror lines read from both dies).  DAISY_GATHER_PIN16 = 0..16 overrides.
-        {
-            int l2 = 0;
-            cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, s->ctx->device);
-            const double fbytes = (double)s->nloc * (double)ncols * 4.0;
-            int p16 = fbytes > 0.0 ? (int)floor(16.0 * 0.45 * (double)l2 / fbytes) : 0;
-            if (p16 > 16) p16 = 16;
-            if (p16 < 0) p16 = 0;
-            const char *e3 = getenv("DAISY_GATHER_PIN16");
-            if (e3) { p16 = atoi(e3); if (p16 < 0) p16 = 0; if (p16 > 16) p16 = 16; }
-            s->pin16 = p16;
-        }
+        s->pin16 = pin16_for(s, (double)s->nloc * (double)ncols * 4.0); // tile skipping rebases it on the occupied tiles
     }
+}
+
+// ---- tile skipping ------------------------------------------------------------------------------------------------
+// occ[rb * S + s] = 1 iff tile (rb, s) -- rows [rb T_ROWS, +T_ROWS) x columns [s T_COLS, +T_COLS), clipped to the nloc x ldF
+// extent the F tensor map covers, i.e. exactly what the producer would load -- holds an entry whose bits other than the sign
+// are not all zero (NaN and Inf tiles are kept).  One CTA per tile, 4 rows x 256 columns per load.
+__global__ void __launch_bounds__(256) k_tile_scan(const float *F, int64_t ldF, int nloc, int trows, int tcols, int S, unsigned char *occ) {
+    const int s = blockIdx.x, rb = blockIdx.y, lanes = tcols / 4;
+    const int64_t col = (int64_t)s * tcols + (threadIdx.x % lanes) * 4;
+    const int r1 = min(nloc, (rb + 1) * trows);
+    unsigned any = 0u;
+    if (col < ldF) // ldF is a multiple of 32: a float4 is either inside or outside
+        for (int r = rb * trows + (int)threadIdx.x / lanes; r < r1; r += 256 / lanes) {
+            const float4 v = ldg_stream(F + (size_t)r * ldF + col);
+            any |= (__float_as_uint(v.x) | __float_as_uint(v.y) | __float_as_uint(v.z) | __float_as_uint(v.w)) & 0x7fffffffu;
+        }
+    any = __syncthreads_or(any != 0u);
+    if (threadIdx.x == 0) occ[(size_t)rb * S + s] = any ? 1 : 0;
+}
+
+// the compacted stream-K plan over the occupied tiles of an nrb x S map: the entries of every row block in column order, a
+// row block without an occupied tile gets one null entry (-1: nothing streamed, its epilogue still runs)
+struct SkipPlan {
+    std::vector<int> list, off;
+    int total = 0, grid = 1, L = 0, maxp = 1;
+    int64_t occupied = 0;
+};
+static void build_skip_plan(const unsigned char *occ, int nrb, int S, int sms, SkipPlan &sp) {
+    sp.list.clear();
+    sp.off.assign((size_t)nrb + 1, 0);
+    sp.occupied = 0;
+    for (int rb = 0; rb < nrb; rb++) {
+        sp.off[(size_t)rb] = (int)sp.list.size();
+        for (int st = 0; st < S; st++)
+            if (occ[(size_t)rb * S + st]) sp.list.push_back(st);
+        sp.occupied += (int64_t)sp.list.size() - sp.off[(size_t)rb];
+        if ((int)sp.list.size() == sp.off[(size_t)rb]) sp.list.push_back(-1);
+    }
+    sp.off[(size_t)nrb] = (int)sp.list.size();
+    sp.total = (int)sp.list.size();
+    sp.grid = sp.total < sms ? (sp.total > 0 ? sp.total : 1) : sms;
+    sp.L = sp.total > 0 ? (sp.total + sp.grid - 1) / sp.grid : 1;
+    sp.maxp = 1;
+    for (int rb = 0; rb < nrb; rb++) {
+        const int np = sk_owner(sp.off[(size_t)rb + 1] - 1, sp.total, sp.grid) - sk_owner(sp.off[(size_t)rb], sp.total, sp.grid) + 1;
+        if (np > sp.maxp) sp.maxp = np;
+    }
+}
+
+// scan F, rebuild the plan and upload it.  Runs at solver creation and before the first pass after F changed.
+static int scan_and_plan(daisy_solver *s) {
+    daisy_ctx *c = s->ctx;
+    const int trows = 64, tcols = 256; // = tma_rows<K>() x TmaCfg<K>::COLS for K <= 9
+    const int nrb = (s->nloc + trows - 1) / trows, S = s->sk_S;
+    cudaStream_t st = c->stream;
+    s->occ.assign((size_t)nrb * S, 0);
+    if (s->nloc > 0 && S > 0) {
+        unsigned char *d_occ = nullptr;
+        cudaEvent_t t0 = nullptr, t1 = nullptr;
+        int rc = DAISY_OK;
+        auto ok = [&](cudaError_t e, const char *what) {
+            if (e != cudaSuccess && !rc) { daisy_set_error("tile scan: %s -> %s", what, cudaGetErrorString(e)); rc = DAISY_E_CUDA; }
+            return rc == DAISY_OK;
+        };
+        if (ok(cudaMalloc(&d_occ, s->occ.size()), "cudaMalloc") && ok(cudaEventCreate(&t0), "cudaEventCreate") && ok(cudaEventCreate(&t1), "cudaEventCreate") &&
+            ok(cudaEventRecord(t0, st), "cudaEventRecord")) {
+            k_tile_scan<<<dim3((unsigned)S, (unsigned)nrb), 256, 0, st>>>(c->d_F, c->ldF, s->nloc, trows, tcols, S, d_occ);
+            if (ok(cudaGetLastError(), "k_tile_scan") && ok(cudaEventRecord(t1, st), "cudaEventRecord") &&
+                ok(cudaMemcpyAsync(s->occ.data(), d_occ, s->occ.size(), cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync") &&
+                ok(cudaStreamSynchronize(st), "cudaStreamSynchronize")) {
+                float ms = 0.f;
+                if (ok(cudaEventElapsedTime(&ms, t0, t1), "cudaEventElapsedTime")) s->scan_ms = ms;
+            }
+        }
+        if (t0) cudaEventDestroy(t0);
+        if (t1) cudaEventDestroy(t1);
+        cudaFree(d_occ);
+        if (rc) return rc;
+    }
+    SkipPlan sp;
+    build_skip_plan(s->occ.data(), nrb, S, c->num_sms, sp);
+    // the stream is idle here (synchronised above): no pass can still read the arrays about to be replaced
+    if ((int64_t)sp.list.size() > s->sk_list_cap) {
+        cudaFree(s->d_sk_list); s->d_sk_list = nullptr; s->sk_list_cap = 0;
+        DZ_CUDA(cudaMalloc(&s->d_sk_list, sizeof(int) * sp.list.size()));
+        s->sk_list_cap = (int64_t)sp.list.size();
+    }
+    if (!s->d_sk_off) DZ_CUDA(cudaMalloc(&s->d_sk_off, sizeof(int) * ((size_t)nrb + 1)));
+    if (sp.maxp > s->partial_splits) {
+        cudaFree(s->d_partial); s->d_partial = nullptr; s->partial_splits = 0;
+        DZ_CUDA(cudaMalloc(&s->d_partial, sizeof(float) * (size_t)sp.maxp * (s->nloc > 0 ? s->nloc : 1) * s->Kp));
+        s->partial_splits = sp.maxp;
+    }
+    DZ_CUDA(cudaMemcpy(s->d_sk_list, sp.list.data(), sizeof(int) * sp.list.size(), cudaMemcpyHostToDevice));
+    DZ_CUDA(cudaMemcpy(s->d_sk_off, sp.off.data(), sizeof(int) * sp.off.size(), cudaMemcpyHostToDevice));
+    s->sk_total = sp.total; s->sk_grid = sp.grid; s->sk_L = sp.L; s->sk_maxp = sp.maxp;
+    s->occupied = sp.occupied;
+    s->pin16 = pin16_for(s, (double)sp.occupied * trows * tcols * 4.0); // the bytes a pass actually streams
+    s->scanned_version = c->F_version;
+    return DAISY_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1022,6 +1210,7 @@ static void free_solver(daisy_solver *s) {
     cudaFree(s->d_res[0]); cudaFree(s->d_res[1]); cudaFree(s->d_B); cudaFree(s->d_E); cudaFree(s->d_M); cudaFree(s->d_mat);
     cudaFree(s->d_partial); cudaFree(s->d_cta_sums); cudaFree(s->d_done); cudaFree(s->d_split);
     cudaFree(s->d_rb_arrive); cudaFree(s->d_rb_sums);
+    cudaFree(s->d_sk_list); cudaFree(s->d_sk_off);
     if (s->h_abort) cudaFreeHost(s->h_abort);
     if (s->e0) cudaEventDestroy(s->e0);
     if (s->e1) cudaEventDestroy(s->e1);
@@ -1083,7 +1272,8 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     SC(cudaMalloc(&s->d_B, sizeof(float) * (size_t)s->Kp * s->n));
     SC(cudaMalloc(&s->d_M, sizeof(float) * (size_t)nmat * s->Kp * s->Kp));
     SC(cudaMalloc(&s->d_mat, sizeof(int) * (size_t)(s->nloc > 0 ? s->nloc : 1)));
-    SC(cudaMalloc(&s->d_partial, sizeof(float) * (size_t)(s->nsplit > s->sk_maxp ? s->nsplit : s->sk_maxp) * (s->nloc > 0 ? s->nloc : 1) * s->Kp));
+    s->partial_splits = s->nsplit > s->sk_maxp ? s->nsplit : s->sk_maxp;
+    SC(cudaMalloc(&s->d_partial, sizeof(float) * (size_t)s->partial_splits * (s->nloc > 0 ? s->nloc : 1) * s->Kp));
     SC(cudaMalloc(&s->d_cta_sums, sizeof(double) * 148 * s->Kp));
     SC(cudaMalloc(&s->d_done, sizeof(unsigned int)));
     SC(cudaMemset(s->d_done, 0, sizeof(unsigned int)));
@@ -1127,6 +1317,7 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     // the set-up above used synchronous copies and legacy-stream memsets; the solver's kernels run on ctx->stream, which may be
     // a non-blocking stream (daisy_ctx_set_stream): make sure everything has landed before anything is enqueued there
     { cudaError_t e_ = cudaDeviceSynchronize(); if (e_ != cudaSuccess) { daisy_set_error("daisy_solver_create: %s", cudaGetErrorString(e_)); free_solver(s); return DAISY_E_CUDA; } }
+    if (s->skip) { rc = scan_and_plan(s); if (rc) { free_solver(s); return rc; } }
     compute_sums_from_host(s, E);
     s->e_sums = s->sums;
     *out = s;
@@ -1471,5 +1662,53 @@ extern "C" int daisy_solver_launches_per_pass(daisy_solver *s) {
 extern "C" int daisy_solver_last_step_ms(daisy_solver *s, double *ms) {
     DZ_REQUIRE(s && ms, DAISY_E_INVALID, "daisy_solver_last_step_ms: null argument");
     *ms = s->last_ms;
+    return DAISY_OK;
+}
+
+// tile map of the last scan (tile skipping): dims2 = row blocks, column steps (0, 0 when the solver streams the dense plan);
+// occ (may be NULL) receives the nrb x S map if capacity allows; occupied = tiles with a non-zero entry; scan_ms = device time
+// of the scan kernel
+extern "C" int daisy_solver_tile_map(daisy_solver *s, int32_t *dims2, uint8_t *occ, int64_t capacity, int64_t *occupied, double *scan_ms) {
+    DZ_REQUIRE(s && dims2, DAISY_E_INVALID, "daisy_solver_tile_map: null argument");
+    const bool have = s->skip && !s->occ.empty();
+    dims2[0] = have ? (int32_t)(s->occ.size() / (size_t)s->sk_S) : 0;
+    dims2[1] = have ? s->sk_S : 0;
+    if (occ && have) {
+        DZ_REQUIRE(capacity >= (int64_t)s->occ.size(), DAISY_E_INVALID, "daisy_solver_tile_map: buffer too small");
+        memcpy(occ, s->occ.data(), s->occ.size());
+    }
+    if (occupied) *occupied = have ? s->occupied : 0;
+    if (scan_ms) *scan_ms = have ? s->scan_ms : 0.0;
+    return DAISY_OK;
+}
+
+// diagnostic, host only: the compacted stream-K plan k_gather_tma runs for an nrb x S tile map on `sms` SMs, with the pieces every
+// CTA takes as the kernel's own next_piece computes them
+extern "C" int daisy_gather_plan_dump(const uint8_t *occ, int nrb, int S, int sms, int32_t *info5, int32_t *list, int32_t *off, int32_t *pieces6,
+                                      int64_t capacity) {
+    DZ_REQUIRE(occ && info5 && nrb >= 0 && S >= 0 && sms >= 1, DAISY_E_INVALID, "daisy_gather_plan_dump: bad argument");
+    SkipPlan sp;
+    build_skip_plan(occ, nrb, S, sms, sp);
+    GatherParams P;
+    memset(&P, 0, sizeof(P));
+    P.nrb = nrb; P.sk = 1; P.sk_S = S; P.sk_L = sp.L; P.sk_total = sp.total;
+    P.sk_list = sp.list.data(); P.sk_off = sp.off.data();
+    std::vector<int32_t> pcs;
+    for (int c = 0; c < sp.grid && sp.total > 0; c++) {
+        int cursor = 0;
+        Piece p;
+        memset(&p, 0, sizeof(p));
+        while (next_piece<256>(P, c, sp.grid, cursor, p)) {
+            const int32_t rec[6] = { c, p.rb, p.s0, p.s1, p.idx, p.np };
+            pcs.insert(pcs.end(), rec, rec + 6);
+        }
+    }
+    info5[0] = sp.total; info5[1] = sp.grid; info5[2] = sp.L; info5[3] = sp.maxp; info5[4] = (int32_t)(pcs.size() / 6);
+    if (list || off || pieces6)
+        DZ_REQUIRE(capacity >= (int64_t)pcs.size() && capacity >= (int64_t)sp.total && capacity >= (int64_t)nrb + 1, DAISY_E_INVALID,
+                   "daisy_gather_plan_dump: buffers too small");
+    if (list) memcpy(list, sp.list.data(), sizeof(int32_t) * sp.list.size());
+    if (off) memcpy(off, sp.off.data(), sizeof(int32_t) * sp.off.size());
+    if (pieces6) memcpy(pieces6, pcs.data(), sizeof(int32_t) * pcs.size());
     return DAISY_OK;
 }

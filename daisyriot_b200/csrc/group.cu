@@ -133,6 +133,8 @@ extern "C" int daisy_group_formfactors_build(daisy_group *g, int variant) {
     // every device traces its share of the tiles and stores into the owners' rows; the join below is the barrier after
     // which every row block is complete
     if (!rc) rc = for_each_device(g, "daisy_group_formfactors_build", [&](int i) { return daisy_formfactors_build(g->ctx[(size_t)i], variant); });
+    // the devices also wrote into each other's rows: every matrix changed after the join, whichever device finished last
+    for (int i = 0; i < g->ndev; i++) g->ctx[(size_t)i]->F_version++;
     nvtxRangePop();
     return rc;
 }

@@ -187,6 +187,21 @@ int daisy_solver_last_step_ms(daisy_solver *s, double *ms);
 int daisy_solver_set_chained(daisy_solver *s, int on);
 /* kernels one pass launches in this solver's configuration: 1 for K <= 9 (streaming, epilogue and exchange wait in one kernel) */
 int daisy_solver_launches_per_pass(daisy_solver *s);
+/* Tile skipping (K <= 9; DAISY_GATHER_SKIP=0 streams the whole matrix instead): a pass streams only the 64-row x 256-column tiles
+ * of F that hold an entry other than +-0.  The solver scans F for them at daisy_solver_create and again before the first pass
+ * after F changed through daisy_formfactors_build, daisy_formfactors_write_rows or daisy_group_formfactors_build of this
+ * process.  A write into this context's rows made by another process through a CUDA-IPC mapping of F after the solver exists
+ * is NOT seen: create the solver after the build's barrier (dist.py does).
+ * daisy_solver_tile_map: dims2 = row blocks, column steps of the last scan (0, 0 on the dense plan); occ (may be NULL) = that
+ * map, 1 = streamed, if capacity >= dims2[0] * dims2[1]; occupied = tiles streamed per pass; scan_ms = device time of the scan. */
+int daisy_solver_tile_map(daisy_solver *s, int32_t *dims2, uint8_t *occ, int64_t capacity, int64_t *occupied, double *scan_ms);
+/* diagnostic, host only: the plan a pass runs for an nrb x S tile map on `sms` SMs.  info5 = entries, CTAs, longest CTA range,
+ * most pieces of one row block, pieces; list = column step of every entry (-1: the null entry of a row block without an
+ * occupied tile), off = nrb + 1 entry offsets of the row blocks, pieces6 = {cta, row block, first entry, end entry, idx, np}
+ * per piece in CTA order (a null entry's piece has first == end).  list / off / pieces6 may be NULL; capacity = int32 elements
+ * each of them holds. */
+int daisy_gather_plan_dump(const uint8_t *occ, int nrb, int S, int sms, int32_t *info5, int32_t *list, int32_t *off, int32_t *pieces6,
+                           int64_t capacity);
 
 /* Fused exchange (replaces the NCCL all-gather of the loop above when all ranks sit in one NVLink domain):
  *   daisy_solver_ipc_handles: 3 x 64-byte CUDA-IPC handles of this rank's two exchange buffers and its flag array
