@@ -876,7 +876,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
             DZ_CUDA(cudaFuncSetAttribute(k_gather_tma<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             attr_done[c->device & 63] = true;
         }
-        P.nrb = (s->nloc + tma_rows<K>() - 1) / tma_rows<K>();
+        P.nrb = s->nrb_tma; // (nloc + tma_rows<K>() - 1) / tma_rows<K>(), and 1 for a rank without rows (plan())
         P.sk = s->fused_epi ? 1 : 0; P.sk_S = s->sk_S; P.sk_L = s->sk_L; P.sk_total = s->sk_total;
         if (s->skip) { P.sk_list = s->d_sk_list; P.sk_off = s->d_sk_off; }
         P.pin16 = s->pin16;
@@ -1080,11 +1080,16 @@ static void plan(daisy_solver *s) {
     int colw = (ncols + s->nsplit - 1) / s->nsplit;
     s->colw = ((colw + G_TC - 1) / G_TC) * G_TC; // multiple of 512 columns (and of the 128-column TMA step)
     s->nsplit = (ncols + s->colw - 1) / s->colw;
+    // column steps of a row block of k_gather_tma, whatever the plan: every step a piece streams lies below it (piece_step)
+    const int tcols = (s->Kp <= 9) ? 256 : 128; // = TmaCfg<Kp>::COLS
+    s->sk_S = (ncols + tcols - 1) / tcols;
     if (s->fused_epi) {
         // stream-K: the (row block, column step) sequence cut into one contiguous, equally long range per SM
-        const int trows = (s->Kp == 32) ? 32 : 64, tcols = (s->Kp <= 9) ? 256 : 128; // = tma_rows<Kp>() x TmaCfg<Kp>::COLS
-        const int nrb = (s->nloc + trows - 1) / trows;
-        s->sk_S = (ncols + tcols - 1) / tcols;
+        const int trows = (s->Kp == 32) ? 32 : 64; // = tma_rows<Kp>()
+        // a rank that owns no rows (the last ranks of a partition whose blocks are rounded up to 256) still gets one row block
+        // over zero rows: only the epilogue of a pass's last row block publishes the rank's band sums and raises its flag,
+        // which every peer's next pass waits for
+        const int nrb = s->nloc > 0 ? (s->nloc + trows - 1) / trows : 1;
         s->sk_total = nrb * s->sk_S;
         s->sk_grid = s->sk_total < sms ? (s->sk_total > 0 ? s->sk_total : 1) : sms;
         s->sk_L = (s->sk_total + s->sk_grid - 1) / s->sk_grid;
@@ -1145,7 +1150,7 @@ static void build_skip_plan(const unsigned char *occ, int nrb, int S, int sms, S
 static int scan_and_plan(daisy_solver *s) {
     daisy_ctx *c = s->ctx;
     const int trows = 64, tcols = 256; // = tma_rows<K>() x TmaCfg<K>::COLS for K <= 9
-    const int nrb = (s->nloc + trows - 1) / trows, S = s->sk_S;
+    const int nrb = s->nrb_tma, S = s->sk_S; // a rank without rows: one row block, whose null entry runs the epilogue (plan())
     cudaStream_t st = c->stream;
     s->occ.assign((size_t)nrb * S, 0);
     if (s->nloc > 0 && S > 0) {
@@ -1280,7 +1285,7 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     {
         const int trows = (s->Kp == 32) ? 32 : 64; // = tma_rows<Kp>()
         s->nrb_tma = (s->nloc + trows - 1) / trows;
-        if (s->nrb_tma < 1) s->nrb_tma = 1;
+        if (s->nrb_tma < 1) s->nrb_tma = 1; // a rank without rows runs one row block over zero rows (plan())
         SC(cudaMalloc(&s->d_rb_arrive, sizeof(unsigned int) * (size_t)s->nrb_tma));
         SC(cudaMemset(s->d_rb_arrive, 0, sizeof(unsigned int) * (size_t)s->nrb_tma));
         SC(cudaMalloc(&s->d_rb_sums, sizeof(double) * (size_t)s->nrb_tma * s->Kp));

@@ -170,6 +170,14 @@ extern "C" int daisy_group_formfactors_write_rows(daisy_group *g, int row0, int 
         if (rc) return rc;
         r = r1;
     }
+    // a device that owns no rows (blocks of rows_per_rank rounded up to 256 can leave the last ones empty) receives none of
+    // them above, yet its solver still needs a matrix (the one-row allocation its tensor map points at) and have_F: a write
+    // of zero rows gives it both
+    for (daisy_ctx *c : g->ctx)
+        if (c->row1 == c->row0) {
+            int rc = daisy_formfactors_write_rows(c, c->row0, 0, nullptr);
+            if (rc) return rc;
+        }
     return DAISY_OK;
 }
 
