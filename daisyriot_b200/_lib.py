@@ -66,6 +66,7 @@ SYMBOLS = {
     "daisy_solver_reset": (_i, [_vp]),
     "daisy_solver_step": (_i, [_vp, _dp]),
     "daisy_solver_converge": (_i, [_vp, C.c_double, _i, _i, _ip]),
+    "daisy_solver_converge_device": (_i, [_vp, C.c_double, _i, _i, _ip]),
     "daisy_solver_numpasses": (_i, [_vp]),
     "daisy_solver_band_sums": (_i, [_vp, _dp]),
     "daisy_solver_read": (_i, [_vp, _fp, _fp]),
@@ -91,6 +92,7 @@ SYMBOLS = {
     "daisy_group_solver_reset": (_i, [_vp]),
     "daisy_group_solver_step": (_i, [_vp, _dp]),
     "daisy_group_solver_converge": (_i, [_vp, C.c_double, _i, _i, _ip]),
+    "daisy_group_solver_converge_device": (_i, [_vp, C.c_double, _i, _i, _ip]),
     "daisy_group_solver_numpasses": (_i, [_vp]),
     "daisy_group_solver_band_sums": (_i, [_vp, _dp]),
     "daisy_group_solver_read": (_i, [_vp, _fp, _fp]),

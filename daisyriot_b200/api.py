@@ -381,9 +381,12 @@ class GroupSolver:
         _lib.check(_lib.lib().daisy_group_solver_band_sums(self._s, sums.ctypes.data_as(C.POINTER(C.c_double))), "group_solver_band_sums")
         return sums
 
-    def converge(self, threshold: float, per_band: bool, max_passes: int = 0) -> int:
+    def converge(self, threshold: float, per_band: bool, max_passes: int = 0, on_device: bool = False) -> int:
+        """``on_device=True``: the pass kernels apply the stop rule themselves and the passes follow each other without a host
+        decision in between (``daisy_group_solver_converge_device``); same passes and bit-identical results."""
         passes = C.c_int()
-        _lib.check(_lib.lib().daisy_group_solver_converge(self._s, float(threshold), int(per_band), max_passes, C.byref(passes)), "group_solver_converge")
+        fn = _lib.lib().daisy_group_solver_converge_device if on_device else _lib.lib().daisy_group_solver_converge
+        _lib.check(fn(self._s, float(threshold), int(per_band), max_passes, C.byref(passes)), "group_solver_converge")
         return passes.value
 
     @property
@@ -564,10 +567,12 @@ class Lightning:
         self._after_update()
         return sums
 
-    def converge_lightning(self, max_passes: int = 0):
+    def converge_lightning(self, max_passes: int = 0, on_device: bool = False):
+        """``on_device=True``: the pass kernels apply the stop rule themselves and the passes follow each other without a host
+        decision in between (``daisy_solver_converge_device``); same passes and bit-identical results."""
         passes = C.c_int()
-        _lib.check(_lib.lib().daisy_solver_converge(self._s, float(self.threshold), int(self.per_band), max_passes, C.byref(passes)),
-                   "solver_converge")
+        fn = _lib.lib().daisy_solver_converge_device if on_device else _lib.lib().daisy_solver_converge
+        _lib.check(fn(self._s, float(self.threshold), int(self.per_band), max_passes, C.byref(passes)), "solver_converge")
         self._after_update()
         return passes.value
 

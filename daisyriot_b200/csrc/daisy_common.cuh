@@ -339,4 +339,6 @@ struct daisy_solver;
 int dz_ctx_set_peer_pointers(daisy_ctx *ctx, float *const *F, int nranks);                                           // api.cu
 int dz_solver_get_buffers(daisy_solver *s, float **res0, float **res1, unsigned long long **flags);                  // gather.cu
 int dz_solver_set_peer_pointers(daisy_solver *s, float *const *res0, float *const *res1, unsigned long long *const *flags, int nranks); // gather.cu
+// converge with the stop rule on the device over n solvers issued from one thread (one GPU, or a group's devices)   // gather.cu
+int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per_band, int max_passes);
 int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F); // formfactor.cu

@@ -20,6 +20,8 @@
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
+#include <cmath>
 #include <vector>
 
 #define G_WARPS 8
@@ -86,6 +88,8 @@ struct daisy_solver {
     int pin16 = 0;                      // sixteenths of the local F rows kept in L2 across passes (plan())
     bool events_recorded = false;       // e0 / e1 bracket the most recent pass
     bool chained = false;               // daisy_solver_set_chained: passes launched back to back without per-pass events
+    unsigned int *d_stop = nullptr;     // device converge: {stopped, passes} (DevStop::state), allocated by the first call
+    void *h_stop = nullptr;             // pinned: that word, then the G x Kp band sums of the batch's last pass
 };
 
 // ---------------------------------------------------------------------------------------------------------
@@ -129,6 +133,41 @@ __device__ __forceinline__ float4 ldg_stream(const float *p) {
     return r;
 }
 
+// Device converge (daisy_solver_converge_device, DESIGN 3.3): the passes of one call are launched back to back and every pass
+// but the first applies converge_lightning's stop rule to the band sums the previous pass left in the tails of the buffer it
+// reads.  state == null: an ordinary pass (one branch on a kernel parameter).
+struct DevStop {
+    unsigned int *state;   // {stopped, passes}: cleared by the host at the start of the call
+    const double *tails;   // rank g's K band sums of the residual this pass reads: tails[g * tstride + k]
+    int64_t tstride;
+    int G, K;              // ranks, bands that count (not the padded Kp)
+    int rule;              // -1: no test (the host decided the first pass), 0: total over bands, 1: per band
+    double threshold;
+};
+
+// converged(): the host loop's unconverged() negated, on the totals fetch_sums forms -- the same doubles added in the same order
+__device__ __forceinline__ bool stop_converged(const DevStop &S) {
+    const volatile double *t = S.tails;
+    double tot = 0.0;
+    bool over = false;
+    for (int k = 0; k < S.K; k++) {
+        double v = 0.0;
+        for (int g = 0; g < S.G; g++) v += t[(size_t)g * S.tstride + k];
+        over = over || v > S.threshold;
+        tot += v;
+    }
+    return S.rule ? !over : !(tot > S.threshold);
+}
+__device__ __forceinline__ bool stop_stopped(const DevStop &S) { return *reinterpret_cast<volatile unsigned int *>(S.state) != 0u; }
+// the decision of a pass (every thread that asks gets the same answer): true = do nothing.  A pass that finds the residual
+// converged says so in state[0] for the launches behind it, whose buffers are stale and must not be tested.
+__device__ __forceinline__ bool stop_decide(const DevStop &S) {
+    if (stop_stopped(S)) return true;
+    if (S.rule < 0 || !stop_converged(S)) return false;
+    *reinterpret_cast<volatile unsigned int *>(S.state) = 1u;
+    return true;
+}
+
 struct GatherParams {
     const float *F; int64_t ldF;
     int nloc;               // local rows
@@ -151,6 +190,7 @@ struct GatherParams {
     // evict_first -- a fixed subset of the matrix, spread evenly over the CTAs, that stays in L2 from pass to pass when the
     // matrix is not much larger than L2 (the reference's own scenes: 164 / 238 MB against 126 MB of L2)
     int pin16;
+    DevStop stop;
 };
 
 // one unit of work of k_gather_tma: steps [s0, s1) of row block rb (tile skipping: entries [s0, s1) of sk_list); idx / np =
@@ -175,13 +215,16 @@ __global__ void __launch_bounds__(G_THREADS, 1) k_gather_partial(GatherParams P)
     extern __shared__ __align__(128) unsigned char g_smem[];
     float *tiles = reinterpret_cast<float *>(g_smem);                 // 2 x K x G_TC
     uint64_t *bars = reinterpret_cast<uint64_t *>(g_smem + 2 * K * G_TC * sizeof(float));
+    int *s_stop = reinterpret_cast<int *>(bars + 2);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) {
         mbar_init(&bars[0], 1);
         mbar_init(&bars[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        if (P.stop.state) *s_stop = stop_decide(P.stop);
     }
     __syncthreads();
+    if (P.stop.state && *s_stop) return; // device converge: no load has been issued yet
     uint32_t phase[2] = { 0, 0 };
     const int nitems = P.nrb * P.nsplit;
     for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
@@ -352,6 +395,18 @@ __device__ __forceinline__ void wait_flag(const FusedEpi &E, int g) {
     }
 }
 
+// the device-converge decision of k_gather_tma.  Fused exchange: the test needs every rank's sums of the previous pass, so
+// all G flags are awaited first (a pass that stops raises no flag, so a stopped launch must not wait for any)
+__device__ __forceinline__ bool tma_stop_decide(const DevStop &S, const FusedEpi &E) {
+    if (stop_stopped(S)) return true;
+    if (S.rule < 0) return false;
+    if (E.enabled && E.npeers > 0 && E.wait_seq != 0ull) {
+        for (int g = 0; g < E.G; g++) wait_flag(E, g);
+        if (*reinterpret_cast<volatile unsigned long long *>(E.flags + 16) != 0ull) return true; // gave up on a peer: the host reports it
+    }
+    return stop_decide(S);
+}
+
 
 #ifdef __CUDA_ARCH__
 #define DZ_ASSERT_HD(cond) DZ_ASSERT(cond)
@@ -438,6 +493,7 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
     float *s_out = reinterpret_cast<float *>(empty + NST + 2);              // 2 x T_ROWS x K sums of a block (single split), double-buffered
     double *s_red = reinterpret_cast<double *>(s_out + 2 * tma_rows<K>() * K); // 2 KB: ordered reductions
     int *s_flag = reinterpret_cast<int *>(empty + NST);
+    int *s_stop = s_flag + 1;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (E.enabled && *reinterpret_cast<volatile unsigned long long *>(E.flags + 16) != 0ull) return; // an earlier pass gave up on a peer
     if (tid == 0) {
@@ -453,6 +509,42 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
     uint32_t it = 0; // global step counter: stage = it % NST, phase = (it / NST) & 1
     int cursor = 0;
     Piece pc;
+    // producer lane: the F tiles of the first NST steps go out before the previous pass is known to be complete; returns how many
+    uint32_t pre = 0;
+    auto issue_first_tiles = [&]() {
+        uint64_t pl, pf;
+        asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pl));
+        asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pf));
+        uint32_t n = 0;
+        int cur2 = 0;
+        Piece p2;
+        while (n < (uint32_t)NST && next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cur2, p2))
+            for (int e = p2.s0; e < p2.s1 && n < (uint32_t)NST; e++, n++) {
+                const int s = piece_step(P, e);
+                mbar_expect_tx(&full[n], (uint32_t)tma_stage_bytes<K>());
+                tma_load_2d_hint(stages + (size_t)n * STAGE_F, &tmF, s * T_COLS, p2.rb * T_ROWS, &full[n],
+                                 (((s * 11 + p2.rb * 5) & 15) < P.pin16) ? pl : pf);
+            }
+        return n;
+    };
+    if (P.stop.state) {
+        // device converge: the whole CTA takes the stop decision once the previous pass is complete.  A pass that does not run
+        // leaves when the F tiles already in flight have landed: their stages expected the residual bytes too, which are
+        // completed here instead of loaded.
+        if (warp == NCW && lane == 0) pre = issue_first_tiles();
+        asm volatile("griddepcontrol.wait;" ::: "memory");
+        if (tid == 0) *s_stop = tma_stop_decide(P.stop, E);
+        __syncthreads();
+        if (*s_stop) {
+            if (warp == NCW && lane == 0)
+                for (uint32_t i = 0; i < pre; i++) {
+                    asm volatile("mbarrier.complete_tx.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&full[i])), "r"((uint32_t)(K * T_COLS * 4)) : "memory");
+                    mbar_wait(&full[i], 0);
+                }
+            return;
+        }
+        if (warp == NCW && lane == 0) asm volatile("fence.proxy.async;" ::: "memory"); // the peers' blocks seen by tid 0, before the TMA reads
+    }
     if (warp != NCW) asm volatile("griddepcontrol.wait;" ::: "memory");
     if (warp > NCW) {
         // ------------------------------- epilogue warps (64 threads) -------------------------------
@@ -574,7 +666,10 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
                         if (E.npeers > 0) { for (int g = 0; g < E.npeers; g++) E.peer_sums[g][et] = v; }
                         else E.block_sums[et] = v;
                     }
-                    if (et == 0) *E.done = 0u;
+                    if (et == 0) {
+                        *E.done = 0u;
+                        if (P.stop.state) P.stop.state[1]++; // device converge: this pass ran
+                    }
                     if (E.npeers > 0) {
                         __threadfence_system();
                         esync();
@@ -594,23 +689,13 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
         // of the residual bands (tiles never straddle an exchange block: n is a multiple of 256 when G > 1, and a
         // single block's tail beyond n is zero-filled by the TMA unit)
         if (lane == 0) {
-            unsigned ready = (E.enabled && E.wait_seq != 0ull) ? 0u : 0xffffffffu; // ranks whose block of the previous pass is known to be here
+            // ranks whose block of the previous pass is known to be here (a tested device-converge pass has awaited them all)
+            unsigned ready = (E.enabled && E.wait_seq != 0ull && !(P.stop.state && P.stop.rule >= 0)) ? 0u : 0xffffffffu;
             uint64_t pol_last, pol_first;
             asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_last));
             asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_first));
             auto pol = [&](int rb, int s) -> uint64_t { return (((s * 11 + rb * 5) & 15) < P.pin16) ? pol_last : pol_first; };
-            // the F tiles of the first NST steps go out before the previous pass is known to be complete
-            uint32_t pre = 0;
-            {
-                int cur2 = 0;
-                Piece p2;
-                while (pre < (uint32_t)NST && next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cur2, p2))
-                    for (int e = p2.s0; e < p2.s1 && pre < (uint32_t)NST; e++, pre++) {
-                        const int s = piece_step(P, e);
-                        mbar_expect_tx(&full[pre], (uint32_t)tma_stage_bytes<K>());
-                        tma_load_2d_hint(stages + (size_t)pre * STAGE_F, &tmF, s * T_COLS, p2.rb * T_ROWS, &full[pre], pol(p2.rb, s));
-                    }
-            }
+            if (!P.stop.state) pre = issue_first_tiles();
             asm volatile("griddepcontrol.wait;" ::: "memory");
             while (next_piece<T_COLS>(P, blockIdx.x, gridDim.x, cursor, pc)) {
                 const int row0 = pc.rb * T_ROWS;
@@ -724,6 +809,7 @@ struct EpiParams {
     unsigned long long *peer_flag[16];
     unsigned long long seq;
     const unsigned long long *abort_marker; // flag word 16 of this rank (null: single GPU)
+    unsigned int *stop_state;               // device converge: {stopped, passes} (the streaming kernel decided), else null
 };
 
 template <int K>
@@ -731,6 +817,7 @@ __global__ void __launch_bounds__(256) k_gather_epilogue(EpiParams P) {
     __shared__ double s_sum[8][K];
     __shared__ bool s_last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (P.stop_state && *reinterpret_cast<volatile unsigned int *>(P.stop_state) != 0u) return;
     double loc[K];
 #pragma unroll
     for (int k = 0; k < K; k++) loc[k] = 0.0;
@@ -785,7 +872,10 @@ __global__ void __launch_bounds__(256) k_gather_epilogue(EpiParams P) {
             if (P.npeers > 0) { for (int g = 0; g < P.npeers; g++) P.peer_sums[g][tid] = v; }
             else P.block_sums[tid] = v;
         }
-        if (tid == 0) *P.done = 0;
+        if (tid == 0) {
+            *P.done = 0;
+            if (P.stop_state) P.stop_state[1]++; // device converge: this pass ran
+        }
         if (P.npeers > 0) {
             __threadfence_system();
             __syncthreads();
@@ -801,9 +891,12 @@ __global__ void __launch_bounds__(256) k_gather_epilogue(EpiParams P) {
 // waits until every rank's block of pass `seq` has arrived in this rank's buffer (flag[g] >= seq for all g).  A peer that does
 // not show up within timeout_ns turns into an error instead of a hung GPU: the abort markers are set (flag word 16 and the
 // host-mapped word), the kernels of later passes return at once and nothing more is published to the peers.
-__global__ void k_wait_flags(unsigned long long *flags, int G, unsigned long long seq, unsigned long long timeout_ns, unsigned long long *host_abort) {
+// stopped != null (device converge): a launch behind the pass that found convergence waits for nothing, since no flag follows
+__global__ void k_wait_flags(unsigned long long *flags, int G, unsigned long long seq, unsigned long long timeout_ns, unsigned long long *host_abort,
+                             const unsigned int *stopped = nullptr) {
     const int g = threadIdx.x;
     if (g >= G) return;
+    if (stopped && *reinterpret_cast<const volatile unsigned int *>(stopped) != 0u) return;
     unsigned long long t0;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0));
     while (true) {
@@ -839,11 +932,12 @@ static int launch_partial(daisy_solver *s, const GatherParams &P) {
 
 // wait_seq != 0 (fused exchange): the blocks of pass wait_seq must have arrived before the residual is read.  The fused TMA
 // kernel waits by itself, block by block; the other kernels get a k_wait_flags launch in front.
+// stop != null: a pass of a device converge (state, rule and threshold set by the caller; the tails are filled in here)
 template <int K>
-static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
+static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const DevStop *stop) {
     daisy_ctx *c = s->ctx;
     if (wait_seq != 0ull && !s->fused_epi) {
-        k_wait_flags<<<1, 32, 0, c->stream>>>(s->d_flags, s->G, wait_seq, s->timeout_ns, s->d_abort_host);
+        k_wait_flags<<<1, 32, 0, c->stream>>>(s->d_flags, s->G, wait_seq, s->timeout_ns, s->d_abort_host, stop ? stop->state : nullptr);
         DZ_CUDA(cudaGetLastError());
     }
     GatherParams P;
@@ -852,6 +946,13 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
     P.nsplit = s->nsplit; P.colw = s->colw; P.nrb = (s->nloc + G_WARPS * s->R - 1) / (G_WARPS * s->R);
     P.sk = 0; P.sk_S = P.sk_L = P.sk_total = 0; P.pin16 = 0;
     P.sk_list = P.sk_off = nullptr;
+    memset(&P.stop, 0, sizeof(P.stop));
+    if (stop) {
+        P.stop = *stop;
+        P.stop.tails = reinterpret_cast<const double *>(s->d_res[s->cur] + s->sums_off);
+        P.stop.tstride = s->bstride / 2; // bstride is a multiple of 4 floats
+        P.stop.G = s->G; P.stop.K = s->K;
+    }
     int rc;
     if (s->use_mma && (K == 16 || K == 32)) {
         if constexpr (K == 16 || K == 32) {
@@ -861,7 +962,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
                 DZ_CUDA(cudaFuncSetAttribute(k_gather_mma<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
                 attr_done[c->device & 63] = true;
             }
-            k_split_residual<K><<<(s->ncolsP + 255) / 256, 256, 0, c->stream>>>(s->d_res[s->cur], s->bstride, s->n, s->G * s->n, s->ncolsP, s->d_split);
+            k_split_residual<K><<<(s->ncolsP + 255) / 256, 256, 0, c->stream>>>(s->d_res[s->cur], s->bstride, s->n, s->G * s->n, s->ncolsP, s->d_split, P.stop);
             DZ_CUDA(cudaGetLastError());
             P.nrb = (s->nloc + MM_ROWS - 1) / MM_ROWS;
             k_gather_mma<K><<<s->grid, MM_THREADS, smem, c->stream>>>(P, s->tmFmma, s->tmSplit);
@@ -904,14 +1005,15 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
         {
             // chained single-GPU passes: programmatic dependent launch lets this grid move onto SMs as the previous pass leaves
             // them and stream its first F tiles meanwhile (the kernel waits for the previous grid before it touches anything
-            // a pass writes).  Multi-GPU passes keep plain stream order (their abort marker is read at kernel start).
+            // a pass writes).  Multi-GPU passes keep plain stream order (their abort marker is read at kernel start).  A device
+            // converge always chains on one GPU.
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((TmaCfg<K>::NCW + 3) * 32); cfg.dynamicSmemBytes = smem; cfg.stream = c->stream;
             cudaLaunchAttribute at[1];
             at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             at[0].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = at;
-            cfg.numAttrs = (s->fused_epi && s->chained && s->G == 1) ? 1 : 0;
+            cfg.numAttrs = (s->fused_epi && (s->chained || stop) && s->G == 1) ? 1 : 0;
             DZ_CUDA(cudaLaunchKernelEx(&cfg, k_gather_tma<K>, P, s->tmF, s->tmRes[s->cur], F));
         }
         DZ_CUDA(cudaGetLastError());
@@ -929,6 +1031,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
     E.M = s->d_M; E.mat = s->d_mat; E.res_out_block = next; E.B = s->d_B;
     E.cta_sums = s->d_cta_sums; E.block_sums = reinterpret_cast<double *>(next + s->sums_off); E.done = s->d_done;
     E.npeers = 0; E.seq = s->seq; E.abort_marker = s->fused ? s->d_flags + 16 : nullptr;
+    E.stop_state = P.stop.state;
     if (s->fused) {
         E.npeers = s->G;
         for (int g = 0; g < s->G; g++) {
@@ -948,17 +1051,17 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq) {
 
 static int scan_and_plan(daisy_solver *s);
 
-static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull) {
+static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull, const DevStop *stop = nullptr) {
     if (s->skip && s->scanned_version != s->ctx->F_version) { // F was written since the last scan (a host integer compare per pass)
         int rc = scan_and_plan(s);
         if (rc) return rc;
     }
     switch (s->Kp) {
-    case 1: return launch_pass_K<1>(s, wait_seq);
-    case 3: return launch_pass_K<3>(s, wait_seq);
-    case 9: return launch_pass_K<9>(s, wait_seq);
-    case 16: return launch_pass_K<16>(s, wait_seq);
-    case 32: return launch_pass_K<32>(s, wait_seq);
+    case 1: return launch_pass_K<1>(s, wait_seq, stop);
+    case 3: return launch_pass_K<3>(s, wait_seq, stop);
+    case 9: return launch_pass_K<9>(s, wait_seq, stop);
+    case 16: return launch_pass_K<16>(s, wait_seq, stop);
+    case 32: return launch_pass_K<32>(s, wait_seq, stop);
     }
     daisy_set_error("unsupported padded band count %d", s->Kp);
     return DAISY_E_INVALID;
@@ -1216,6 +1319,8 @@ static void free_solver(daisy_solver *s) {
     cudaFree(s->d_partial); cudaFree(s->d_cta_sums); cudaFree(s->d_done); cudaFree(s->d_split);
     cudaFree(s->d_rb_arrive); cudaFree(s->d_rb_sums);
     cudaFree(s->d_sk_list); cudaFree(s->d_sk_off);
+    cudaFree(s->d_stop);
+    if (s->h_stop) cudaFreeHost(s->h_stop);
     if (s->h_abort) cudaFreeHost(s->h_abort);
     if (s->e0) cudaEventDestroy(s->e0);
     if (s->e1) cudaEventDestroy(s->e1);
@@ -1589,6 +1694,133 @@ extern "C" int daisy_solver_converge(daisy_solver *s, double threshold, int per_
         if (rc) return rc;
         done++;
     }
+    if (passes_out) *passes_out = s->numpasses;
+    return DAISY_OK;
+}
+
+// ---- converge with the stop rule on the device ------------------------------------------------------------------------------
+// The passes of a call are launched back to back in batches; every pass but the first tests the band sums the previous pass left
+// (DevStop) and the pass that finds the residual converged stops the launches behind it.  Between batches the host reads
+// {stopped, passes} and the band sums of the last pass through one pinned copy and sizes the next batch so that it most likely
+// holds the deciding pass: the criterion (largest band total for per_band, total over bands otherwise) is extrapolated
+// geometrically from its ratio over the last batch, plus two launches -- the one that decides and one of margin, since a launch
+// that finds `stopped` costs a few microseconds and another batch a host round trip.  The first batch is 4 launches, a batch
+// without a contraction to extrapolate doubles, and no batch exceeds 64.
+static int ensure_stop_buffers(daisy_solver *s) {
+    if (s->d_stop) return DAISY_OK;
+    DZ_CUDA(cudaMalloc(&s->d_stop, 2 * sizeof(unsigned int)));
+    DZ_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&s->h_stop), sizeof(double) * (1 + (size_t)s->G * s->Kp), cudaHostAllocDefault));
+    return DAISY_OK;
+}
+
+static double stop_metric(const double *v, int K, int per_band) {
+    double m = per_band ? v[0] : 0.0;
+    for (int k = 0; k < K; k++) m = per_band ? (v[k] > m ? v[k] : m) : m + v[k];
+    return m;
+}
+
+static int abort_error(const daisy_solver *s) {
+    daisy_set_error("fused exchange: a peer's block of pass %llu did not arrive within %.1f s; the solver is stopped until daisy_solver_reset",
+                    *s->h_abort, (double)s->timeout_ns * 1e-9);
+    return DAISY_E_STATE;
+}
+
+// ss[0 .. n): one solver, or every device's solver of a group (fused exchange), all issued from this thread.  The first pass is
+// decided on the host from ss[0]'s sums, as the host loop does.
+int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per_band, int max_passes) {
+    daisy_solver *s0 = ss[0];
+    for (int i = 0; i < n; i++) {
+        daisy_solver *s = ss[i];
+        DZ_CUDA(cudaSetDevice(s->ctx->device));
+        if (s->fused && s->h_abort && *reinterpret_cast<volatile unsigned long long *>(s->h_abort) != 0ull) return abort_error(s);
+        int rc = ensure_stop_buffers(s);
+        if (rc) return rc;
+    }
+    DZ_CUDA(cudaSetDevice(s0->ctx->device));
+    if (!s0->sums_valid) { int rc = fetch_sums(s0); if (rc) return rc; }
+    if (!unconverged(s0, threshold, per_band)) return DAISY_OK; // nothing launched
+    std::vector<int> cur0((size_t)n);
+    std::vector<unsigned long long> seq0((size_t)n);
+    for (int i = 0; i < n; i++) {
+        daisy_solver *s = ss[i];
+        DZ_CUDA(cudaSetDevice(s->ctx->device));
+        DZ_CUDA(cudaMemsetAsync(s->d_stop, 0, 2 * sizeof(unsigned int), s->ctx->stream));
+        cur0[(size_t)i] = s->cur; seq0[(size_t)i] = s->seq;
+    }
+    const long long budget = max_passes > 0 ? max_passes : (1ll << 62);
+    long long issued = 0;
+    int batch = 4;
+    double m_prev = stop_metric(s0->sums.data(), s0->K, per_band);
+    std::vector<double> tot((size_t)s0->K);
+    while (true) {
+        const int nb = (int)std::min<long long>(batch, budget - issued);
+        for (int i = 0; i < n; i++) {
+            daisy_solver *s = ss[i];
+            cudaStream_t st = s->ctx->stream;
+            DZ_CUDA(cudaSetDevice(s->ctx->device));
+            for (int j = 0; j < nb; j++) {
+                DevStop ds;
+                memset(&ds, 0, sizeof(ds));
+                ds.state = s->d_stop; ds.rule = (issued + j == 0) ? -1 : (per_band ? 1 : 0); ds.threshold = threshold;
+                const unsigned long long wait_seq = s->fused ? s->seq : 0ull;
+                if (s->fused) s->seq++;
+                int rc = launch_pass(s, wait_seq, &ds);
+                if (rc) return rc;
+                s->cur ^= 1;
+            }
+            DZ_CUDA(cudaMemcpyAsync(s->h_stop, s->d_stop, 2 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+            if (i == 0) // band sums of the last pass (meaningful only if every pass of the batch ran): the next batch's size
+                for (int g = 0; g < s->G; g++)
+                    DZ_CUDA(cudaMemcpyAsync(reinterpret_cast<double *>(s->h_stop) + 1 + (size_t)g * s->Kp, s->d_res[s->cur] + (size_t)g * s->bstride + s->sums_off,
+                                            sizeof(double) * s->Kp, cudaMemcpyDeviceToHost, st));
+        }
+        issued += nb;
+        for (int i = 0; i < n; i++) {
+            DZ_CUDA(cudaSetDevice(ss[i]->ctx->device));
+            DZ_CUDA(cudaStreamSynchronize(ss[i]->ctx->stream));
+        }
+        for (int i = 0; i < n; i++)
+            if (ss[i]->fused && *reinterpret_cast<volatile unsigned long long *>(ss[i]->h_abort) != 0ull) return abort_error(ss[i]);
+        const unsigned int *state = reinterpret_cast<const unsigned int *>(s0->h_stop);
+        if (state[0] || issued >= budget) break;
+        const double *tails = reinterpret_cast<const double *>(s0->h_stop) + 1;
+        for (int k = 0; k < s0->K; k++) {
+            double v = 0.0;
+            for (int g = 0; g < s0->G; g++) v += tails[(size_t)g * s0->Kp + k];
+            tot[(size_t)k] = v;
+        }
+        const double m = stop_metric(tot.data(), s0->K, per_band);
+        const double r = pow(m / m_prev, 1.0 / nb); // contraction per pass over the last batch
+        double est = -1.0;
+        if (m > threshold && r > 0.0 && r < 1.0 && std::isfinite(r)) est = ceil(log(threshold / m) / log(r));
+        batch = (est >= 0.0 && est < 64.0) ? (int)est + 2 : (est >= 64.0 ? 64 : std::min(2 * nb, 64));
+        m_prev = m;
+    }
+    std::vector<unsigned int> passes((size_t)n);
+    for (int i = 0; i < n; i++) passes[(size_t)i] = reinterpret_cast<const unsigned int *>(ss[i]->h_stop)[1];
+    for (int i = 0; i < n; i++) {
+        daisy_solver *s = ss[i];
+        const unsigned int p = passes[(size_t)i];
+        s->cur = cur0[(size_t)i] ^ (int)(p & 1u);
+        s->numpasses += (int)p;
+        if (s->fused) s->seq = seq0[(size_t)i] + p;
+        s->sums_valid = false;
+        s->events_recorded = false; // no per-pass events: daisy_solver_last_step_ms keeps its value
+    }
+    for (int i = 1; i < n; i++)
+        if (passes[(size_t)i] != passes[0]) {
+            daisy_set_error("device converge: device %d ran %u passes, device 0 ran %u", i, passes[(size_t)i], passes[0]);
+            return DAISY_E_STATE;
+        }
+    return DAISY_OK;
+}
+
+extern "C" int daisy_solver_converge_device(daisy_solver *s, double threshold, int per_band, int max_passes, int *passes_out) {
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_converge_device: null solver");
+    DZ_REQUIRE(s->G == 1 || s->fused, DAISY_E_STATE, "daisy_solver_converge_device: a partitioned solver needs the fused exchange (daisy_solver_set_peers)");
+    DzRange range_("daisy_solver_converge_device");
+    int rc = dz_converge_device(&s, 1, threshold, per_band, max_passes);
+    if (rc) return rc;
     if (passes_out) *passes_out = s->numpasses;
     return DAISY_OK;
 }

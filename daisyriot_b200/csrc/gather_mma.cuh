@@ -99,9 +99,17 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&r)[16]) {
 }
 
 // residual bands of the current exchange buffer -> [Rh (K rows); Rl (K rows)] x ncolsP, Rh = R rounded to TF32,
-// Rl = (R - Rh) rounded to TF32
+// Rl = (R - Rh) rounded to TF32.  Device converge (stop.state != null): the first kernel of the pass takes the stop decision;
+// every CTA reaches the same one, and k_gather_mma and the epilogue only read `stopped`.
 template <int K>
-__global__ void k_split_residual(const float *__restrict__ res, int64_t bstride, int n, int ncols, int ncolsP, float *__restrict__ split) {
+__global__ void k_split_residual(const float *__restrict__ res, int64_t bstride, int n, int ncols, int ncolsP, float *__restrict__ split,
+                                 DevStop stop) {
+    if (stop.state) {
+        __shared__ int s_stop;
+        if (threadIdx.x == 0) s_stop = stop_decide(stop);
+        __syncthreads();
+        if (s_stop) return;
+    }
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncolsP) return;
     const int g = c / n, jl = c - g * n;
@@ -144,6 +152,7 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(d_empty + MM_ND);
     static_assert(MM_NS == 4 && MM_NA == 2 && MM_ND == 4, "mma_done ring indexing below assumes these depths");
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (P.stop.state && stop_stopped(P.stop)) return; // device converge: before any TMEM is allocated
     if (tid == 0) {
         for (int i = 0; i < MM_NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 4); mbar_init(&mma_done[i], 1); }  // empty: 4 converter warps
         for (int i = 0; i < MM_NA; i++) mbar_init(&a_full[i], 4);

@@ -317,6 +317,18 @@ extern "C" int daisy_group_solver_converge(daisy_group_solver *gs, double thresh
     return rc;
 }
 
+// the device converge over every device: the first pass decided from device 0's sums, every device's batches issued from this
+// thread; every device takes the same decisions from the same band sums, which the pass counts confirm
+extern "C" int daisy_group_solver_converge_device(daisy_group_solver *gs, double threshold, int per_band, int max_passes, int *passes_out) {
+    DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_converge_device: null solver");
+    if (gs->g->ndev == 1) return daisy_solver_converge_device(gs->s[0], threshold, per_band, max_passes, passes_out);
+    nvtxRangePushA("daisy_group_solver_converge_device");
+    int rc = dz_converge_device(gs->s.data(), gs->g->ndev, threshold, per_band, max_passes);
+    if (!rc && passes_out) *passes_out = daisy_solver_numpasses(gs->s[0]);
+    nvtxRangePop();
+    return rc;
+}
+
 // lightningvalues and residualvector of the whole scene, K x N band-major, assembled from the devices' row blocks
 extern "C" int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *residual) {
     DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_read: null solver");

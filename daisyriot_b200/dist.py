@@ -155,7 +155,18 @@ class PartitionedSolver:
     def reset(self):
         _lib.check(_lib.lib().daisy_solver_reset(self._s))
 
-    def converge(self, threshold: float, per_band: bool, max_passes: int = 0) -> int:
+    def converge(self, threshold: float, per_band: bool, max_passes: int = 0, on_device: bool = False) -> int:
+        """Passes run by this call.  ``on_device=True`` (fused exchange, or a single rank): every rank calls
+        ``daisy_solver_converge_device`` with the same arguments; the pass kernels apply the stop rule themselves, all ranks
+        stop at the same pass, and no pass waits for the host."""
+        if on_device:
+            if self.nranks > 1 and not self.fused:
+                raise _lib.DaisyError("PartitionedSolver.converge(on_device=True) needs the fused exchange; this solver exchanges through NCCL")
+            L = _lib.lib()
+            before = int(L.daisy_solver_numpasses(self._s))
+            out = C.c_int()
+            _lib.check(L.daisy_solver_converge_device(self._s, float(threshold), int(per_band), int(max_passes), C.byref(out)), "solver_converge_device")
+            return out.value - before
         passes = 0
         sums = self.band_sums()
         crit = (lambda s: (s > threshold).any()) if per_band else (lambda s: s.sum() > threshold)

@@ -160,6 +160,12 @@ int daisy_solver_step(daisy_solver *s, double *band_sums);
 /* converge_lightning(): while (criterion(residual) > threshold) step.  per_band=0: sum over all bands > threshold
  * (spectral, threshold 200, :145-151); per_band=1: any band sum > threshold (RGB/BW, 1e-4, :336-340, :410-415). */
 int daisy_solver_converge(daisy_solver *s, double threshold, int per_band, int max_passes, int *passes_out);
+/* converge_lightning with the stop rule evaluated on the device: same arguments, pass count, B, residual and band sums (bit for
+ * bit) as daisy_solver_converge, but the host does not wait between passes.  Single GPU, or a partitioned solver with the fused
+ * exchange (every rank calls it with the same arguments); DAISY_E_STATE for a partition exchanged by the host.  The passes are
+ * launched back to back in batches (on one GPU with programmatic dependent launch, whatever daisy_solver_set_chained says);
+ * no per-pass events are recorded, so daisy_solver_last_step_ms keeps its value. */
+int daisy_solver_converge_device(daisy_solver *s, double threshold, int per_band, int max_passes, int *passes_out);
 int daisy_solver_numpasses(daisy_solver *s);
 /* per-band sums of the current residual (what the convergence test looks at), K doubles */
 int daisy_solver_band_sums(daisy_solver *s, double *band_sums);
@@ -251,6 +257,8 @@ void daisy_group_solver_destroy(daisy_group_solver *gs);
 int daisy_group_solver_reset(daisy_group_solver *gs);
 int daisy_group_solver_step(daisy_group_solver *gs, double *band_sums);       /* band_sums may be NULL: nothing waits */
 int daisy_group_solver_converge(daisy_group_solver *gs, double threshold, int per_band, int max_passes, int *passes_out);
+/* daisy_solver_converge_device over every device (DAISY_E_STATE if the devices ran different pass counts) */
+int daisy_group_solver_converge_device(daisy_group_solver *gs, double threshold, int per_band, int max_passes, int *passes_out);
 int daisy_group_solver_numpasses(daisy_group_solver *gs);
 int daisy_group_solver_band_sums(daisy_group_solver *gs, double *band_sums);
 int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *residual);   /* K x N band-major, whole scene */

@@ -19,6 +19,14 @@ public:
         numpasses = passes;
         fetch();
     }
+    // converge_lightning with the stop rule evaluated by the pass kernels: same passes and bit-identical values, without a host
+    // round trip per pass (daisy_group_solver_converge_device)
+    void converge_lightning_on_device() {
+        int passes = 0;
+        check(daisy_group_solver_converge_device(solver, threshold, per_band, 0, &passes));
+        numpasses = passes;
+        fetch();
+    }
     virtual void increment_lightpass() {
         check(daisy_group_solver_step(solver, nullptr));
         numpasses = daisy_group_solver_numpasses(solver);

@@ -4,6 +4,7 @@
 // Prints one line of results the parity test compares with the Python path.
 #include <chrono>
 #include <cstdio>
+#include <cstring>
 #include <vector>
 #define TINYOBJLOADER_IMPLEMENTATION
 #include <tiny_obj_loader.h>
@@ -96,6 +97,12 @@ int main(int argc, char **argv) {
     if (getenv("DAISY_DEMO_NO_REFILL")) optixP.refill_RadMat = false;
     const auto t0 = std::chrono::high_resolution_clock::now();
     Lightning *l = Lightning::get_lightning(method, mesh, optixP, emission, wavelengths, true, argc > 7 ? argv[7] : nullptr); // main.cpp:108 passes matfile
+    // DAISY_DEMO_CONVERGE=device: solve again from reset() with the stop rule on the device; the SOLVE line must not change
+    const char *conv = getenv("DAISY_DEMO_CONVERGE");
+    if (conv && strcmp(conv, "device") == 0) {
+        l->reset();
+        l->converge_lightning_on_device();
+    }
     const double solve_s = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
     double sum = 0;
     for (auto &band : l->lightningvalues) for (float v : band) sum += v;

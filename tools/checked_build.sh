@@ -8,3 +8,4 @@ for t in ff gather9 gather32; do
   timeout 600 python tools/sanitize_target.py $t 2>&1 | tail -2
 done
 timeout 1800 python -m pytest tests/test_gpu_parity.py tests/test_gpu_gather_shapes.py -x -q -m gpu -k "(radmat or fixture_scene_rows or sample_counts or edge_heavy or irregular or empty_and_single or gather or closest or trace_screen or face_grids or perforated or chained) and not fused_exchange" 2>&1 | tail -4
+timeout 1800 python -m pytest tests/test_gpu_converge_device.py -x -q -m gpu -k "not group and not two_process and not shim" 2>&1 | tail -4
