@@ -316,10 +316,22 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
             const float *p = vertices + 3 * (size_t)tri_idx[6 * (size_t)i + k];
             for (int d = 0; d < 3; d++) { c->scene_lo[d] = fminf(c->scene_lo[d], p[d]); c->scene_hi[d] = fmaxf(c->scene_hi[d], p[d]); }
         }
-    float ext = 0.f;
-    for (int d = 0; d < 3; d++) if (ntri) ext = fmaxf(ext, c->scene_hi[d] - c->scene_lo[d]);
+    float ext = 0.f, mag = 0.f;
+    for (int d = 0; d < 3; d++)
+        if (ntri) {
+            ext = fmaxf(ext, c->scene_hi[d] - c->scene_lo[d]);
+            mag = fmaxf(mag, fmaxf(fabsf(c->scene_lo[d]), fabsf(c->scene_hi[d])));
+        }
     c->ext = ext;
-    c->pad = 1e-4f * ext; // conservative box padding; results never depend on it (tests compare with brute force)
+    // Conservative box padding; results never depend on it (tests compare with brute force).  1e-4 x the extent, but never
+    // below 16 ulp of the largest coordinate: far from the origin a smaller pad rounds away (lo - pad == lo), a ray lying in
+    // a box's face plane then reads 0 * inf = NaN there and the slab test drops a box that holds its hit.
+    const float ulp = nextafterf(mag, INFINITY) - mag;
+    c->pad = fmaxf(1e-4f * ext, 16.0f * ulp);
+    // The face grids and coplanar skipping rest on margins that are fractions of the extent too, and on ray origins that
+    // round by far less than those margins.  When the coordinates round at more than 1/256 of 1e-4 x the extent (a scene
+    // many times its own size away from the origin), neither is used: every plane id stays 0, so nothing is skipped.
+    const bool far_from_origin = 1e-4f * ext < 256.0f * ulp;
 #define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_ctx(c); return DAISY_E_CUDA; } } while (0)
     CC(cudaMalloc(&c->d_vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
     CC(cudaMalloc(&c->d_normals, sizeof(float) * 3 * (size_t)(nn > 0 ? nn : 1)));
@@ -332,7 +344,8 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
     if (ntri) CC(cudaMemcpy(c->d_tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
     {
         std::vector<int> pid;
-        assign_plane_ids(vertices, tri_idx, ntri, ext, pid);
+        if (far_from_origin) pid.assign((size_t)(ntri > 0 ? ntri : 1), 0);
+        else assign_plane_ids(vertices, tri_idx, ntri, ext, pid);
         { const int rc_ = dz_build_faces(c, vertices, tri_idx, ntri, pid); if (rc_) { free_ctx(c); return rc_; } } // renumbers pid: face f = id f + 1
         CC(cudaMalloc(&c->d_pid, sizeof(int) * pid.size()));
         CC(cudaMemcpy(c->d_pid, pid.data(), sizeof(int) * pid.size(), cudaMemcpyHostToDevice));

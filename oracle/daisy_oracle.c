@@ -283,9 +283,15 @@ orc_bvh *orc_bvh_build(const orc_mesh *m) {
         }
         bv->order[k] = k;
     }
-    float ext = 0.0f;
-    for (int d = 0; d < 3; d++) ext = fmaxf(ext, shi[d] - slo[d]);
-    bv->pad = 1e-4f * ext; /* generous conservative padding; results never depend on it (checked vs brute force) */
+    float ext = 0.0f, mag = 0.0f;
+    for (int d = 0; d < 3; d++) {
+        ext = fmaxf(ext, shi[d] - slo[d]);
+        if (N > 0) mag = fmaxf(mag, fmaxf(fabsf(slo[d]), fabsf(shi[d])));
+    }
+    /* generous conservative padding; results never depend on it (checked vs brute force).  Never below 16 ulp of the largest
+     * coordinate: far from the origin 1e-4 x extent rounds away (lo - pad == lo), and a ray lying in a box's face plane then
+     * reads 0 * inf = NaN there, which the slab test turns into a miss of a box that holds the hit. */
+    bv->pad = fmaxf(1e-4f * ext, 16.0f * (nextafterf(mag, INFINITY) - mag));
     if (N > 0) build_rec(bv, m, cent, 0, N);
     free(cent);
     return bv;

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from conftest import assert_rel, two_triangle_scene
+from geometry_scenes import irregular_walls, perforated_plate
 
 pytestmark = pytest.mark.gpu
 
@@ -518,50 +519,7 @@ def test_irregular_walls_vs_bruteforce(dz, uv50, seed):
     """Adversarial input for coplanar skipping: two facing walls and a tilted occluder triangulated irregularly (jittered grids,
     random diagonals, slivers, triangles 20x larger than their neighbours), vertex heights perturbed by rounding-sized noise
     on part of each wall, arbitrary wall orientation.  Masks and matrix must equal the brute-force oracle bit for bit."""
-    from daisyriot_b200.scenes import Scene
-    rng = np.random.RandomState(seed)
-
-    def rot(axis, ang):
-        axis = axis / np.linalg.norm(axis)
-        K = np.array([[0, -axis[2], axis[1]], [axis[2], 0, -axis[0]], [-axis[1], axis[0], 0]])
-        return np.eye(3) + np.sin(ang) * K + (1 - np.cos(ang)) * K @ K
-
-    R = rot(rng.normal(size=3), rng.uniform(0, 3))
-    V, T, VN = [], [], []
-
-    def wall(origin, eu, ev, n, nu, nv, flip):
-        base = len(V)
-        us = np.sort(np.concatenate([[0, 1], rng.uniform(0, 1, nu - 1)]))
-        vs = np.sort(np.concatenate([[0, 1], rng.uniform(0, 1, nv - 1)]))
-        if seed == 2:
-            us[1] = us[0] + 1e-3  # a column of slivers
-        for j in range(nv + 1):
-            for i in range(nu + 1):
-                p = origin + us[i] * eu + vs[j] * ev
-                if rng.uniform() < 0.3:
-                    p = p + n * rng.uniform(-2e-7, 2e-7) * 6.0
-                V.append(p)
-        ni = len(VN)
-        VN.append(n)
-        for j in range(nv):
-            for i in range(nu):
-                a, b, c, d = base + j * (nu + 1) + i, base + j * (nu + 1) + i + 1, base + (j + 1) * (nu + 1) + i, base + (j + 1) * (nu + 1) + i + 1
-                tris = [(a, b, d), (a, d, c)] if rng.uniform() < 0.5 else [(a, b, c), (b, d, c)]
-                for t in tris:
-                    T.append([*(t[::-1] if flip else t), ni, ni, ni])
-
-    ex, ey, ez = np.eye(3)
-    wall(np.zeros(3), 6 * ex, 6 * ez, ey, 9, 8, True)                       # floor, facing +y
-    wall(np.array([0, 4.0, 0]), 6 * ex, 6 * ez, -ey, 7, 9, False)           # ceiling, facing -y
-    wall(np.array([1.5, 1.7, 1.0]), 2.5 * ex + 0.4 * ey, 3 * ez, np.cross(2.5 * ex + 0.4 * ey, 3 * ez) / np.linalg.norm(np.cross(2.5 * ex + 0.4 * ey, 3 * ez)), 4, 5, False)
-    big = len(V)                                                            # one triangle much larger than its neighbours
-    V += [np.array([6.0, 0, 0]), np.array([9.0, 0, 0]), np.array([6.0, 0, 6.0])]
-    T.append([big, big + 2, big + 1, 0, 0, 0])
-    V = (np.asarray(V) @ R.T).astype(np.float32)
-    VN = (np.asarray(VN) @ R.T).astype(np.float32)
-    T = np.asarray(T, np.int32)
-    mats = [{"name": "w", "Kd": np.ones(3, np.float32), "Ke": np.zeros(3, np.float32), "Ks": np.zeros(3, np.float32)}]
-    sc = Scene(V, VN, T, np.zeros(len(T), np.int32), mats, f"irregular{seed}")
+    sc = irregular_walls(seed)
     p = _ctx(dz, sc, uv50)
     F = p.cudaCalculateRadiosityMatrix().rows()
     masks = p.visibilityMasks()
@@ -598,64 +556,7 @@ def test_perforated_faces_vs_bruteforce(dz, uv50, seed):
     and skim the floor); the sample pattern holds samples exactly on triangle edges and vertices.  Everything is rotated
     arbitrarily.  Covered / mixed / empty cells, flat stretches and end-point margins all come into play; masks and matrix
     must equal the brute-force oracle (every ray against every triangle) bit for bit."""
-    from daisyriot_b200.scenes import Scene
-    rng = np.random.RandomState(100 + seed)
-
-    def rot(axis, ang):
-        axis = axis / np.linalg.norm(axis)
-        K = np.array([[0, -axis[2], axis[1]], [axis[2], 0, -axis[0]], [-axis[1], axis[0], 0]])
-        return np.eye(3) + np.sin(ang) * K + (1 - np.cos(ang)) * K @ K
-
-    R = rot(rng.normal(size=3), rng.uniform(0, 3)) if seed == 2 else np.eye(3)
-    V, T, VN = [], [], []
-
-    def sheet(origin, eu, ev, n, nu, nv, flip, keep=None, split=None):
-        """nu x nv cells; keep(i, j) False = hole; split(i, j) True = the cell is cut into four sub-cells (T-junctions)."""
-        ni = len(VN)
-        VN.append(n)
-
-        def vid(s, t):
-            V.append(origin + s * eu + t * ev)
-            return len(V) - 1
-
-        grid = [[vid(i / nu, j / nv) for i in range(nu + 1)] for j in range(nv + 1)]
-
-        def quad(a, b, c, d):  # a b / c d
-            tris = [(a, b, d), (a, d, c)] if rng.uniform() < 0.5 else [(a, b, c), (b, d, c)]
-            for t in tris:
-                T.append([*(t[::-1] if flip else t), ni, ni, ni])
-
-        for j in range(nv):
-            for i in range(nu):
-                if keep is not None and not keep(i, j):
-                    continue
-                a, b, c, d = grid[j][i], grid[j][i + 1], grid[j + 1][i], grid[j + 1][i + 1]
-                if split is not None and split(i, j):
-                    m = [[a, vid((i + .5) / nu, j / nv), b], [vid(i / nu, (j + .5) / nv), vid((i + .5) / nu, (j + .5) / nv), vid((i + 1) / nu, (j + .5) / nv)],
-                         [c, vid((i + .5) / nu, (j + 1) / nv), d]]
-                    for jj in range(2):
-                        for ii in range(2):
-                            quad(m[jj][ii], m[jj][ii + 1], m[jj + 1][ii], m[jj + 1][ii + 1])
-                else:
-                    quad(a, b, c, d)
-
-    ex, ey, ez = np.eye(3)
-    sheet(np.zeros(3), 6 * ex, 6 * ez, ey, 7, 6, True)                       # floor, facing +y
-    sheet(np.array([0, 4.0, 0]), 6 * ex, 6 * ez, -ey, 6, 7, False)           # ceiling, facing -y
-    holes = rng.uniform(size=(9, 9)) < 0.25
-    splits = rng.uniform(size=(9, 9)) < 0.2
-    pu, pv = 4.2 * ex + 0.5 * ey, 4.0 * ez + 0.3 * ey
-    pn = np.cross(pu, pv) / np.linalg.norm(np.cross(pu, pv))
-    sheet(np.array([0.8, 1.8, 0.9]), pu, pv, pn, 9, 9, False, keep=lambda i, j: not holes[j, i] and not (i > 5 and j > 6), split=lambda i, j: splits[j, i])
-    # a second sheet in the same plane, overlapping part of the first (its vertices are points of the first sheet's plane)
-    sheet(np.array([0.8, 1.8, 0.9]) + 0.31 * pu + 0.27 * pv, 0.45 * pu, 0.4 * pv, pn, 4, 4, False)
-    # a fin standing on the floor: its lower edge lies in the floor's plane
-    sheet(np.array([1.0, 0.0, 5.2]), 4.0 * ex + 0.3 * ez, 0.9 * ey, np.cross(4.0 * ex + 0.3 * ez, 0.9 * ey) / np.linalg.norm(np.cross(4.0 * ex + 0.3 * ez, 0.9 * ey)), 8, 2, False)
-    V = (np.asarray(V) @ R.T).astype(np.float32)
-    VN = (np.asarray(VN) @ R.T).astype(np.float32)
-    T = np.asarray(T, np.int32)
-    mats = [{"name": "w", "Kd": np.ones(3, np.float32), "Ke": np.zeros(3, np.float32), "Ks": np.zeros(3, np.float32)}]
-    sc = Scene(V, VN, T, np.zeros(len(T), np.int32), mats, f"perforated{seed}")
+    sc = perforated_plate(seed)
     # the usual pattern with eight samples moved onto edges and vertices
     uv = uv50.copy()
     uv[:8] = np.array([[0, 0], [1, 0], [0, 1], [0.5, 0], [0, 0.5], [0.5, 0.5], [0.25, 0.75], [1e-4, 0.3]], np.float32)
