@@ -179,6 +179,25 @@ class OptixPrimeFunctionality:
         _lib.check(_lib.lib().daisy_formfactors_build(self._ctx, _lib.FF_HOST), "formfactors_build")
         return RadMat(self)
 
+    def updateGeometry(self, vertices=None, normals=None) -> None:
+        """Move the mesh: new vertex positions and/or normals (same counts, same triangles; ``None`` keeps an array).  The
+        hierarchy and every derived record are rebuilt, so queries answer for the new geometry at once; the matrix changes
+        only at :meth:`updateRadiosityMatrix`.  ``self.mesh`` takes the new arrays."""
+        v, n = _geometry_arrays(self.mesh, vertices, normals)
+        _lib.check(_lib.lib().daisy_ctx_update_geometry(self._ctx, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0]), "ctx_update_geometry")
+        self.mesh.vertices, self.mesh.normals = v, n
+
+    def updateRadiosityMatrix(self, variant=_lib.FF_DEVICE) -> RadMat:
+        """Bring the matrix to the current geometry, bit-identical to a fresh build, re-tracing only the pairs a change can
+        reach (everything when the matrix was loaded, built with another variant or other samples, or not built yet)."""
+        _lib.check(_lib.lib().daisy_formfactors_update(self._ctx, variant), "formfactors_update")
+        return RadMat(self)
+
+    def update_stats(self):
+        t, k, p, ms = C.c_int64(), C.c_int64(), C.c_int64(), C.c_double()
+        _lib.check(_lib.lib().daisy_formfactors_update_stats(self._ctx, C.byref(t), C.byref(k), C.byref(p), C.byref(ms)))
+        return {"tris_changed": t.value, "tiles_retraced": k.value, "pairs_retraced": p.value, "classify_ms": ms.value}
+
     def loadRadiosityMatrix(self, dense_rows: np.ndarray, row0: int = 0) -> RadMat:
         """The reference's matrix-cache path (``Lightning.h:84-96``): load instead of build."""
         a = np.ascontiguousarray(dense_rows, np.float32)
@@ -335,6 +354,16 @@ class DeviceGroup:
         _lib.check(_lib.lib().daisy_group_formfactors_build(self._g, _lib.FF_HOST), "group_formfactors_build")
         return self
 
+    def update_geometry(self, vertices=None, normals=None) -> None:
+        """:meth:`OptixPrimeFunctionality.updateGeometry` on every device."""
+        v, n = _geometry_arrays(self.mesh, vertices, normals)
+        _lib.check(_lib.lib().daisy_group_update_geometry(self._g, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0]), "group_update_geometry")
+        self.mesh.vertices, self.mesh.normals = v, n
+
+    def updateRadiosityMatrix(self, variant=_lib.FF_DEVICE):
+        _lib.check(_lib.lib().daisy_group_formfactors_update(self._g, variant), "group_formfactors_update")
+        return self
+
     def rows(self, row0=0, nrows=None) -> np.ndarray:
         nrows = self.N - row0 if nrows is None else nrows
         out = np.empty((nrows, self.N), np.float32)
@@ -403,6 +432,15 @@ class GroupSolver:
         B = np.ascontiguousarray(B, np.float32)
         R = np.ascontiguousarray(R, np.float32)
         _lib.check(_lib.lib().daisy_group_solver_write(self._s, _lib.fptr(B), _lib.fptr(R)), "group_solver_write")
+
+
+def _geometry_arrays(mesh: MeshS, vertices, normals):
+    """The arrays of an update: the mesh's own where ``None``, float32 copies of the same shape otherwise."""
+    v = np.array(mesh.vertices if vertices is None else vertices, np.float32, copy=True).reshape(-1, 3)
+    n = np.array(mesh.normals if normals is None else normals, np.float32, copy=True).reshape(-1, 3)
+    if v.shape != np.shape(mesh.vertices) or n.shape != np.shape(mesh.normals):
+        raise ValueError("updateGeometry: the vertex and normal counts stay those of the mesh")
+    return v, n
 
 
 def row_digest_host(F_rows: np.ndarray):

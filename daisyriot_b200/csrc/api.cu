@@ -6,6 +6,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <math.h>
+#include <algorithm>
 #include <unordered_map>
 #include <vector>
 
@@ -287,6 +288,8 @@ static void set_partition(daisy_ctx *c, int rank, int nranks) {
     c->ldF = ((ncols + 31) / 32) * 32;
 }
 
+static int build_geometry(daisy_ctx *c);
+
 extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
                                 int device, daisy_ctx **out) {
     DZ_REQUIRE(out, DAISY_E_INVALID, "daisy_ctx_create: null out pointer");
@@ -309,7 +312,48 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
     DZ_CUDA(cudaGetDeviceProperties(&prop, device));
     c->num_sms = prop.multiProcessorCount;
     set_partition(c, 0, 1);
-    // scene bounds over the vertices the triangles use (host: the inputs are host arrays anyway)
+    // (with no triangles the arrays may be null; nothing reads them then)
+    if (vertices) c->h_vertices.assign(vertices, vertices + 3 * (size_t)nv); else c->h_vertices.assign(3 * (size_t)nv, 0.f);
+    if (normals) c->h_normals.assign(normals, normals + 3 * (size_t)nn); else c->h_normals.assign(3 * (size_t)nn, 0.f);
+    if (ntri) c->h_tri.assign(tri_idx, tri_idx + 6 * (size_t)ntri);
+#define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_ctx(c); return DAISY_E_CUDA; } } while (0)
+    CC(cudaMalloc(&c->d_vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
+    CC(cudaMalloc(&c->d_normals, sizeof(float) * 3 * (size_t)(nn > 0 ? nn : 1)));
+    CC(cudaMalloc(&c->d_tri, sizeof(int) * 6 * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&c->d_geom, sizeof(PatchGeom) * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&c->d_plane, sizeof(float4) * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&c->d_nbr, sizeof(int) * 32 * (size_t)(ntri > 0 ? ntri : 1)));
+    if (ntri) CC(cudaMemcpy(c->d_tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
+    {
+        // MeshS::trianglesPerVertex (MeshS.cpp:107-109) as CSR, lists in ascending triangle order: Drawer::interpolate sums
+        // the patch colours of a vertex in exactly that order
+        std::vector<int> off((size_t)nv + 1, 0), adj((size_t)3 * (ntri > 0 ? ntri : 1), 0);
+        for (int i = 0; i < ntri; i++)
+            for (int k = 0; k < 3; k++) off[(size_t)tri_idx[6 * (size_t)i + k] + 1]++;
+        for (int v = 0; v < nv; v++) off[(size_t)v + 1] += off[v];
+        std::vector<int> fill(off.begin(), off.end() - 1);
+        for (int i = 0; i < ntri; i++)
+            for (int k = 0; k < 3; k++) adj[(size_t)fill[tri_idx[6 * (size_t)i + k]]++] = i;
+        CC(cudaMalloc(&c->d_vadj_off, sizeof(int) * off.size()));
+        CC(cudaMalloc(&c->d_vadj, sizeof(int) * adj.size()));
+        CC(cudaMemcpy(c->d_vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice));
+        CC(cudaMemcpy(c->d_vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice));
+    }
+#undef CC
+    const int rc = build_geometry(c);
+    if (rc) { free_ctx(c); return rc; }
+    *out = c;
+    return DAISY_OK;
+}
+
+// Everything derived from the vertex positions and normals (c->h_vertices, c->h_normals): scene bounds, extent, box padding,
+// plane ids, face grids, LBVH, tile order, patch and plane records, neighbour lists.  daisy_ctx_create and
+// daisy_ctx_update_geometry both run it; the device arrays sized by the triangle count exist already.
+static int build_geometry(daisy_ctx *c) {
+    const float *vertices = c->h_vertices.data(), *normals = c->h_normals.data();
+    const int32_t *tri_idx = c->h_tri.data();
+    const int ntri = c->N, nv = c->nv, nn = c->nn;
+    // scene bounds over the vertices the triangles use
     for (int d = 0; d < 3; d++) { c->scene_lo[d] = INFINITY; c->scene_hi[d] = -INFINITY; }
     for (int i = 0; i < ntri; i++)
         for (int k = 0; k < 3; k++) {
@@ -332,46 +376,34 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
     // round by far less than those margins.  When the coordinates round at more than 1/256 of 1e-4 x the extent (a scene
     // many times its own size away from the origin), neither is used: every plane id stays 0, so nothing is skipped.
     const bool far_from_origin = 1e-4f * ext < 256.0f * ulp;
-#define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_ctx(c); return DAISY_E_CUDA; } } while (0)
-    CC(cudaMalloc(&c->d_vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
-    CC(cudaMalloc(&c->d_normals, sizeof(float) * 3 * (size_t)(nn > 0 ? nn : 1)));
-    CC(cudaMalloc(&c->d_tri, sizeof(int) * 6 * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_geom, sizeof(PatchGeom) * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_plane, sizeof(float4) * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_nbr, sizeof(int) * 32 * (size_t)(ntri > 0 ? ntri : 1)));
-    if (nv) CC(cudaMemcpy(c->d_vertices, vertices, sizeof(float) * 3 * (size_t)nv, cudaMemcpyHostToDevice));
-    if (nn) CC(cudaMemcpy(c->d_normals, normals, sizeof(float) * 3 * (size_t)nn, cudaMemcpyHostToDevice));
-    if (ntri) CC(cudaMemcpy(c->d_tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
+    if (nv) DZ_CUDA(cudaMemcpy(c->d_vertices, vertices, sizeof(float) * 3 * (size_t)nv, cudaMemcpyHostToDevice));
+    if (nn) DZ_CUDA(cudaMemcpy(c->d_normals, normals, sizeof(float) * 3 * (size_t)nn, cudaMemcpyHostToDevice));
     {
         std::vector<int> pid;
         if (far_from_origin) pid.assign((size_t)(ntri > 0 ? ntri : 1), 0);
         else assign_plane_ids(vertices, tri_idx, ntri, ext, pid);
-        { const int rc_ = dz_build_faces(c, vertices, tri_idx, ntri, pid); if (rc_) { free_ctx(c); return rc_; } } // renumbers pid: face f = id f + 1
-        CC(cudaMalloc(&c->d_pid, sizeof(int) * pid.size()));
-        CC(cudaMemcpy(c->d_pid, pid.data(), sizeof(int) * pid.size(), cudaMemcpyHostToDevice));
+        dz_free_faces(c);
+        { const int rc_ = dz_build_faces(c, vertices, tri_idx, ntri, pid); if (rc_) return rc_; } // renumbers pid: face f = id f + 1
+        cudaFree(c->d_pid);
+        c->d_pid = nullptr;
+        DZ_CUDA(cudaMalloc(&c->d_pid, sizeof(int) * pid.size()));
+        DZ_CUDA(cudaMemcpy(c->d_pid, pid.data(), sizeof(int) * pid.size(), cudaMemcpyHostToDevice));
     }
-    {
-        // MeshS::trianglesPerVertex (MeshS.cpp:107-109) as CSR, lists in ascending triangle order: Drawer::interpolate sums
-        // the patch colours of a vertex in exactly that order
-        std::vector<int> off((size_t)nv + 1, 0), adj((size_t)3 * (ntri > 0 ? ntri : 1), 0);
-        for (int i = 0; i < ntri; i++)
-            for (int k = 0; k < 3; k++) off[(size_t)tri_idx[6 * (size_t)i + k] + 1]++;
-        for (int v = 0; v < nv; v++) off[(size_t)v + 1] += off[v];
-        std::vector<int> fill(off.begin(), off.end() - 1);
-        for (int i = 0; i < ntri; i++)
-            for (int k = 0; k < 3; k++) adj[(size_t)fill[tri_idx[6 * (size_t)i + k]]++] = i;
-        CC(cudaMalloc(&c->d_vadj_off, sizeof(int) * off.size()));
-        CC(cudaMalloc(&c->d_vadj, sizeof(int) * adj.size()));
-        CC(cudaMemcpy(c->d_vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice));
-        CC(cudaMemcpy(c->d_vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice));
-    }
-#undef CC
     int rc = dz_build_lbvh(c);
     if (!rc) rc = dz_precompute_geom(c);
-    if (!rc && cudaStreamSynchronize(c->stream) != cudaSuccess) { daisy_set_error("daisy_ctx_create: %s", cudaGetErrorString(cudaGetLastError())); rc = DAISY_E_CUDA; }
-    if (rc) { free_ctx(c); return rc; }
-    *out = c;
-    return DAISY_OK;
+    if (!rc && cudaStreamSynchronize(c->stream) != cudaSuccess) { daisy_set_error("geometry build: %s", cudaGetErrorString(cudaGetLastError())); rc = DAISY_E_CUDA; }
+    return rc;
+}
+
+extern "C" int daisy_ctx_update_geometry(daisy_ctx *ctx, const float *vertices, int nv, const float *normals, int nn) {
+    DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_ctx_update_geometry: null context");
+    DZ_REQUIRE(nv == ctx->nv && nn == ctx->nn, DAISY_E_INVALID, "daisy_ctx_update_geometry: nv and nn must match daisy_ctx_create (the topology does not change)");
+    DzRange range_("daisy_ctx_update_geometry: plane ids, face grids, LBVH, patch records");
+    DZ_CUDA(cudaSetDevice(ctx->device));
+    DZ_CUDA(cudaStreamSynchronize(ctx->stream)); // nothing enqueued may still read the arrays the rebuild replaces
+    if (vertices) ctx->h_vertices.assign(vertices, vertices + 3 * (size_t)nv);
+    if (normals) ctx->h_normals.assign(normals, normals + 3 * (size_t)nn);
+    return build_geometry(ctx);
 }
 
 extern "C" void daisy_ctx_destroy(daisy_ctx *ctx) {
@@ -479,6 +511,17 @@ static int ensure_F(daisy_ctx *ctx) {
     return DAISY_OK;
 }
 
+// what F now holds: the matrix of the current geometry, samples and this variant
+static void set_record(daisy_ctx *ctx, int variant) {
+    ctx->rec.valid = true;
+    ctx->rec.variant = variant;
+    ctx->rec.S = ctx->S;
+    memcpy(ctx->rec.uv, ctx->h_uv, sizeof(ctx->rec.uv));
+    ctx->rec.vertices = ctx->h_vertices;
+    ctx->rec.normals = ctx->h_normals;
+    ctx->rec.pad = ctx->pad;
+}
+
 extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_formfactors_build: null context");
     DZ_REQUIRE(variant == DAISY_FF_DEVICE || variant == DAISY_FF_HOST, DAISY_E_INVALID, "daisy_formfactors_build: bad variant");
@@ -498,6 +541,119 @@ extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     if (timing) fprintf(stderr, "daisy_formfactors_build: tile list + kernel + clean-up %.3f s (kernel %.3f s)\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t1).count(), ctx->ff_ms * 1e-3);
     ctx->have_F = true;
     ctx->F_version++;
+    set_record(ctx, variant);
+    return DAISY_OK;
+}
+
+// padded box of triangle t as k_refit (bvh.cu) computes it: the same IEEE operations, so the same floats
+static void tri_box(const float *V, const int *tri, int t, float pad, float4 *out2) {
+    const float *a = V + 3 * (size_t)tri[6 * (size_t)t], *b = V + 3 * (size_t)tri[6 * (size_t)t + 1], *c = V + 3 * (size_t)tri[6 * (size_t)t + 2];
+    out2[0] = make_float4(fminf(a[0], fminf(b[0], c[0])) - pad, fminf(a[1], fminf(b[1], c[1])) - pad, fminf(a[2], fminf(b[2], c[2])) - pad, 0.f);
+    out2[1] = make_float4(fmaxf(a[0], fmaxf(b[0], c[0])) + pad, fmaxf(a[1], fmaxf(b[1], c[1])) + pad, fmaxf(a[2], fmaxf(b[2], c[2])) + pad, 0.f);
+}
+
+#define UPD_CLUSTER 32 // dirty boxes per cluster (consecutive in Morton order)
+extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
+    DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_formfactors_update: null context");
+    DZ_REQUIRE(variant == DAISY_FF_DEVICE || variant == DAISY_FF_HOST, DAISY_E_INVALID, "daisy_formfactors_update: bad variant");
+    DZ_REQUIRE(ctx->S >= 1, DAISY_E_STATE, "daisy_formfactors_update: call daisy_ctx_set_samples first");
+    DzRange range_("daisy_formfactors_update: dirty set, tile classification, partial k_ff_tiles");
+    DZ_CUDA(cudaSetDevice(ctx->device));
+    int rc = ensure_F(ctx);
+    if (rc) return rc;
+    rc = dz_set_samples_const(ctx);
+    if (rc) return rc;
+    const int N = ctx->N;
+    ctx->upd_classify_ms = 0.0;
+    // F can be reused only if it holds this variant's matrix for these samples, and the samples keep every ray in its pair's shaft
+    const bool reuse = ctx->have_F && ctx->rec.valid && ctx->rec.variant == variant && ctx->rec.S == ctx->S &&
+                       memcmp(ctx->rec.uv, ctx->h_uv, sizeof(float) * 2 * (size_t)ctx->S) == 0 && !dz_samples_outside(ctx);
+    if (!reuse) {
+        rc = dz_build_formfactors(ctx, variant, nullptr, 0, 0, true);
+        if (rc) return rc;
+        ctx->upd_tris_changed = N;
+    } else {
+        // changed: a position or a normal differs bitwise from the record; moved: a position does (only those can occlude
+        // differently)
+        const float *V0 = ctx->rec.vertices.data(), *V1 = ctx->h_vertices.data(), *N0 = ctx->rec.normals.data(), *N1 = ctx->h_normals.data();
+        const int *tri = ctx->h_tri.data();
+        std::vector<unsigned char> changed((size_t)(N > 0 ? N : 1), 0);
+        std::vector<char> moved((size_t)(N > 0 ? N : 1), 0);
+        int64_t nchanged = 0;
+        for (int t = 0; t < N; t++) {
+            bool pos = false, nrm = false;
+            for (int k = 0; k < 3; k++) pos |= memcmp(V0 + 3 * (size_t)tri[6 * (size_t)t + k], V1 + 3 * (size_t)tri[6 * (size_t)t + k], 12) != 0;
+            for (int k = 3; k < 6; k++) nrm |= memcmp(N0 + 3 * (size_t)tri[6 * (size_t)t + k], N1 + 3 * (size_t)tri[6 * (size_t)t + k], 12) != 0;
+            changed[(size_t)t] = pos || nrm;
+            moved[(size_t)t] = pos;
+            nchanged += pos || nrm;
+        }
+        ctx->upd_tris_changed = nchanged;
+        if (nchanged == 0) { // F already is the matrix of this geometry
+            ctx->upd_tiles = 0; ctx->pairs_traced = 0; ctx->pairs_owned = 0; ctx->pairs_heavy = 0; ctx->ff_ms = 0.0;
+            ctx->upd_pairs = 0;
+            return DAISY_OK;
+        }
+        // dirty boxes: the moved triangles in Morton order (tile slots of the current hierarchy), clusters of UPD_CLUSTER
+        // consecutive ones, once with their recorded boxes and once with their current ones
+        std::vector<int> order;
+        for (int p = 0; p < ctx->nslots; p++) {
+            const int t = ctx->h_order[p];
+            if (t >= 0 && moved[(size_t)t]) order.push_back(t);
+        }
+        std::vector<float4> leaf, cbox;
+        std::vector<int2> crange;
+        for (int geom = 0; geom < 2; geom++) {
+            const float *V = geom ? V1 : V0;
+            const float pad = geom ? ctx->pad : ctx->rec.pad;
+            for (size_t i = 0; i < order.size(); i += UPD_CLUSTER) {
+                const size_t e = std::min(order.size(), i + UPD_CLUSTER);
+                float4 u0 = make_float4(INFINITY, INFINITY, INFINITY, 0.f), u1 = make_float4(-INFINITY, -INFINITY, -INFINITY, 0.f);
+                crange.push_back(make_int2((int)(leaf.size() / 2), (int)(leaf.size() / 2 + (e - i))));
+                for (size_t j = i; j < e; j++) {
+                    float4 b[2];
+                    tri_box(V, tri, order[j], pad, b);
+                    leaf.push_back(b[0]); leaf.push_back(b[1]);
+                    u0 = make_float4(fminf(u0.x, b[0].x), fminf(u0.y, b[0].y), fminf(u0.z, b[0].z), 0.f);
+                    u1 = make_float4(fmaxf(u1.x, b[1].x), fmaxf(u1.y, b[1].y), fmaxf(u1.z, b[1].z), 0.f);
+                }
+                cbox.push_back(u0); cbox.push_back(u1);
+            }
+        }
+        unsigned char *d_changed = nullptr;
+        float4 *d_leaf = nullptr, *d_cbox = nullptr;
+        int2 *d_crange = nullptr;
+        cudaError_t e = cudaMalloc(&d_changed, changed.size());
+        if (e == cudaSuccess) e = cudaMalloc(&d_leaf, sizeof(float4) * (leaf.empty() ? 1 : leaf.size()));
+        if (e == cudaSuccess) e = cudaMalloc(&d_cbox, sizeof(float4) * (cbox.empty() ? 1 : cbox.size()));
+        if (e == cudaSuccess) e = cudaMalloc(&d_crange, sizeof(int2) * (crange.empty() ? 1 : crange.size()));
+        if (e == cudaSuccess) e = cudaMemcpy(d_changed, changed.data(), changed.size(), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess && !leaf.empty()) e = cudaMemcpy(d_leaf, leaf.data(), sizeof(float4) * leaf.size(), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess && !cbox.empty()) e = cudaMemcpy(d_cbox, cbox.data(), sizeof(float4) * cbox.size(), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess && !crange.empty()) e = cudaMemcpy(d_crange, crange.data(), sizeof(int2) * crange.size(), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) {
+            DzUpdate upd;
+            upd.changed = d_changed; upd.leaf = d_leaf; upd.cbox = d_cbox; upd.crange = d_crange; upd.nclusters = (int)crange.size();
+            rc = dz_build_formfactors(ctx, variant, nullptr, 0, 0, true, &upd);
+        }
+        cudaFree(d_changed); cudaFree(d_leaf); cudaFree(d_cbox); cudaFree(d_crange);
+        if (e != cudaSuccess) { daisy_set_error("daisy_formfactors_update: %s", cudaGetErrorString(e)); return DAISY_E_CUDA; }
+        if (rc) return rc;
+    }
+    ctx->upd_pairs = ctx->pairs_traced;
+    ctx->have_F = true;
+    // also when this rank stored nothing: with peers, other ranks may have stored into its rows
+    ctx->F_version++;
+    set_record(ctx, variant);
+    return DAISY_OK;
+}
+
+extern "C" int daisy_formfactors_update_stats(daisy_ctx *ctx, int64_t *tris_changed, int64_t *tiles_retraced, int64_t *pairs_retraced, double *classify_ms) {
+    DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_formfactors_update_stats: null context");
+    if (tris_changed) *tris_changed = ctx->upd_tris_changed;
+    if (tiles_retraced) *tiles_retraced = ctx->upd_tiles;
+    if (pairs_retraced) *pairs_retraced = ctx->upd_pairs;
+    if (classify_ms) *classify_ms = ctx->upd_classify_ms;
     return DAISY_OK;
 }
 
@@ -580,6 +736,7 @@ extern "C" int daisy_formfactors_write_rows(daisy_ctx *ctx, int row0, int nrows,
     DZ_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->have_F = true;
     ctx->F_version++;
+    ctx->rec.valid = false; // F no longer is a matrix this library computed
     return DAISY_OK;
 }
 

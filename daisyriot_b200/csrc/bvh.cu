@@ -204,6 +204,9 @@ int dz_build_lbvh(daisy_ctx *ctx) {
     cudaEvent_t e0, e1;
     DZ_CUDA(cudaEventCreate(&e0));
     DZ_CUDA(cudaEventCreate(&e1));
+    // a rebuild (daisy_ctx_update_geometry) replaces the previous hierarchy
+    cudaFree(ctx->d_triverts); cudaFree(ctx->d_nodes); cudaFree(ctx->d_tribox); cudaFree(ctx->d_order); free(ctx->h_order);
+    ctx->d_triverts = nullptr; ctx->d_nodes = nullptr; ctx->d_tribox = nullptr; ctx->d_order = nullptr; ctx->h_order = nullptr;
     DZ_CUDA(cudaEventRecord(e0, st));
     DZ_CUDA(cudaMalloc(&ctx->d_triverts, sizeof(TriVerts) * (size_t)(N > 0 ? N : 1)));
     DZ_CUDA(cudaMalloc(&ctx->d_nodes, sizeof(BvhNode) * (size_t)(N > 1 ? N - 1 : 1)));

@@ -324,6 +324,32 @@ struct daisy_ctx {
     // cudaMalloc / cudaFree pair per buffer per call (dz_scratch, api.cu)
     void *scratch[6] = { nullptr, nullptr, nullptr, nullptr, nullptr, nullptr };
     size_t scratch_bytes[6] = { 0, 0, 0, 0, 0, 0 };
+    // host copies of the mesh: the current geometry (daisy_ctx_create / daisy_ctx_update_geometry) and the triangle list
+    std::vector<float> h_vertices, h_normals;
+    std::vector<int> h_tri;
+    // what F holds (daisy_formfactors_build / _update): the variant, sample pattern and geometry it was computed for, and the
+    // box padding of that geometry.  Cleared by daisy_formfactors_write_rows.
+    struct {
+        bool valid = false;
+        int variant = 0, S = 0;
+        float uv[2 * DAISY_MAX_SAMPLES];
+        std::vector<float> vertices, normals;
+        float pad = 0.f;
+    } rec;
+    // last daisy_formfactors_update
+    int64_t upd_tris_changed = 0, upd_tiles = 0, upd_pairs = 0;
+    double upd_classify_ms = 0.0;
+};
+
+// The part of F an update has to recompute (formfactor.cu, daisy_formfactors_update): per-triangle changed flags and the
+// dirty boxes -- the padded boxes of the moved triangles in the recorded and in the current geometry, as leaves grouped into
+// clusters of consecutive Morton order.  Device pointers.
+struct DzUpdate {
+    const unsigned char *changed; // N flags: a position or a normal of the triangle differs from the record
+    const float4 *leaf;           // 2 float4 per dirty box
+    const float4 *cbox;           // 2 float4 per cluster: union of its leaves
+    const int2 *crange;           // leaves [x, y) of each cluster
+    int nclusters;
 };
 cudaError_t dz_scratch(daisy_ctx *ctx, int slot, size_t bytes, void **out); // api.cu
 
@@ -341,4 +367,7 @@ int dz_solver_get_buffers(daisy_solver *s, float **res0, float **res1, unsigned 
 int dz_solver_set_peer_pointers(daisy_solver *s, float *const *res0, float *const *res1, unsigned long long *const *flags, int nranks); // gather.cu
 // converge with the stop rule on the device over n solvers issued from one thread (one GPU, or a group's devices)   // gather.cu
 int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per_band, int max_passes);
-int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F); // formfactor.cu
+// upd != null: only the pairs the update can reach are traced and stored (ctx->upd_tiles, upd_classify_ms report it)
+int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F,
+                         const DzUpdate *upd = nullptr);                                                    // formfactor.cu
+bool dz_samples_outside(const daisy_ctx *ctx);                                                              // formfactor.cu

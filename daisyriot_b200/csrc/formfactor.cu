@@ -14,6 +14,7 @@
 #include <math.h>
 #include <chrono>
 #include <stdlib.h>
+#include <algorithm>
 #include <vector>
 
 #define TILE 64
@@ -819,6 +820,131 @@ __device__ __forceinline__ uint64_t pair_mask_warp(const TriVerts *__restrict__ 
     return (uint64_t)mask_lo | ((uint64_t)mask_hi << 32);
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// Matrix updates after a geometry change (daisy_formfactors_update; DESIGN "Updating the matrix after a geometry change").
+// A pair whose two patches did not change keeps its entry unless a ray of the pair can be accepted by a moved triangle in the
+// recorded or in the current geometry; by the premise of the shaft culling above that needs the triangle's padded box in that
+// geometry to meet the pair's shaft.  The dirty boxes are those padded boxes, grouped into clusters.
+#define UPD_CAP 16 // dirty clusters listed per tile; a tile whose shaft meets more treats every pair as dirty
+
+// does the pair's shaft meet one of the dirty boxes listed for its tile?  (list: UPD_CAP + 1 ints, see FFParams::tile_dirty)
+__device__ __noinline__ bool pair_meets_dirty(const int *__restrict__ list, const TriVerts *__restrict__ tv, const float4 *__restrict__ cbox,
+                                              const int2 *__restrict__ crange, const float4 *__restrict__ leaf, int lo, int hi) {
+    const int n = __ldg(list);
+    if (n < 0) return true;
+    const Shaft sh = make_shaft(tv[lo], tv[hi]);
+    for (int i = 0; i < n; i++) {
+        const int k = __ldg(list + 1 + i);
+        const float4 b0 = __ldg(cbox + 2 * k), b1 = __ldg(cbox + 2 * k + 1);
+        if (!shaft_box(sh, b0.x, b0.y, b0.z, b1.x, b1.y, b1.z)) continue;
+        const int2 r = __ldg(crange + k);
+        for (int j = r.x; j < r.y; j++) {
+            const float4 l0 = __ldg(leaf + 2 * j), l1 = __ldg(leaf + 2 * j + 1);
+            if (shaft_box(sh, l0.x, l0.y, l0.z, l1.x, l1.y, l1.z)) return true;
+        }
+    }
+    return false;
+}
+
+// warp + block reduction of 6 values over the 128 threads of k_ff_classify (op 0 = min, 1 = max, 2 = sum per value)
+__device__ __forceinline__ void block_reduce6(float v[6], const int op[6], float (*s_red)[6]) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+#pragma unroll
+    for (int q = 0; q < 6; q++)
+        for (int o = 16; o > 0; o >>= 1) {
+            const float x = __shfl_xor_sync(0xffffffffu, v[q], o);
+            v[q] = op[q] == 0 ? fminf(v[q], x) : (op[q] == 1 ? fmaxf(v[q], x) : v[q] + x);
+        }
+    __syncthreads(); // s_red free for reuse
+    if (lane == 0)
+        for (int q = 0; q < 6; q++) s_red[w][q] = v[q];
+    __syncthreads();
+#pragma unroll
+    for (int q = 0; q < 6; q++) {
+        float a = s_red[0][q];
+        for (int j = 1; j < 4; j++) a = op[q] == 0 ? fminf(a, s_red[j][q]) : (op[q] == 1 ? fmaxf(a, s_red[j][q]) : a + s_red[j][q]);
+        v[q] = a;
+    }
+}
+
+// One CTA of 128 threads per job (the two slot groups of the tile, one slot per thread).  A tile is kept if a slot holds a
+// changed triangle or if the shaft of the whole tile -- the convex hull of all the vertices of both groups, tested like a
+// pair's shaft with D = the difference of the two groups' mean vertices -- meets a dirty cluster.  Kept jobs are appended
+// (in no particular order: the tile kernel schedules them dynamically anyway) with the clusters their shaft meets.
+__global__ void __launch_bounds__(128) k_ff_classify(const int2 *__restrict__ jobs, int njobs, const int *__restrict__ order,
+                                                     const TriVerts *__restrict__ tv, const unsigned char *__restrict__ changed,
+                                                     const float4 *__restrict__ cbox, int nclusters, int2 *__restrict__ kept_jobs,
+                                                     int *__restrict__ kept_lists, int *__restrict__ kept_count) {
+    __shared__ float s_red[4][6];
+    __shared__ int s_n, s_any, s_slot;
+    __shared__ int s_list[UPD_CAP];
+    const int tid = threadIdx.x;
+    for (int job = blockIdx.x; job < njobs; job += gridDim.x) {
+        const int2 jt = jobs[job];
+        if (tid == 0) { s_n = 0; s_any = 0; }
+        __syncthreads();
+        const int t = order[(tid < TILE ? jt.x * TILE : jt.y * TILE - TILE) + tid];
+        TriVerts T = {};
+        if (t >= 0) T = tv[t];
+        if (t >= 0 && changed[t]) s_any = 1; // benign race: every writer stores 1
+        const float4 p[3] = { T.a, T.b, T.c };
+        float v[6];
+        const int mnmx[6] = { 0, 0, 0, 1, 1, 1 }, sums[6] = { 2, 2, 2, 2, 2, 2 };
+        v[0] = v[1] = v[2] = INFINITY; v[3] = v[4] = v[5] = -INFINITY;
+        if (t >= 0)
+            for (int i = 0; i < 3; i++) {
+                v[0] = fminf(v[0], p[i].x); v[1] = fminf(v[1], p[i].y); v[2] = fminf(v[2], p[i].z);
+                v[3] = fmaxf(v[3], p[i].x); v[4] = fmaxf(v[4], p[i].y); v[5] = fmaxf(v[5], p[i].z);
+            }
+        block_reduce6(v, mnmx, s_red);
+        Shaft sh;
+        sh.lox = v[0]; sh.loy = v[1]; sh.loz = v[2]; sh.hix = v[3]; sh.hiy = v[4]; sh.hiz = v[5];
+        // group means: sums of vertices (row group in 0..2, column group in 3..5) and counts
+        float m[6] = { 0.f, 0.f, 0.f, 0.f, 0.f, 0.f };
+        if (t >= 0) {
+            const int o = tid < TILE ? 0 : 3;
+            m[o] = p[0].x + p[1].x + p[2].x; m[o + 1] = p[0].y + p[1].y + p[2].y; m[o + 2] = p[0].z + p[1].z + p[2].z;
+        }
+        block_reduce6(m, sums, s_red);
+        float cnt[6] = { (t >= 0 && tid < TILE) ? 3.f : 0.f, (t >= 0 && tid >= TILE) ? 3.f : 0.f, 0.f, 0.f, 0.f, 0.f };
+        block_reduce6(cnt, sums, s_red);
+        // any direction D gives a valid separating axis for the hull; the one between the groups' means separates best
+        sh.Dx = cnt[0] > 0.f && cnt[1] > 0.f ? m[3] / cnt[1] - m[0] / cnt[0] : 0.f;
+        sh.Dy = cnt[0] > 0.f && cnt[1] > 0.f ? m[4] / cnt[1] - m[1] / cnt[0] : 0.f;
+        sh.Dz = cnt[0] > 0.f && cnt[1] > 0.f ? m[5] / cnt[1] - m[2] / cnt[0] : 0.f;
+        float c[6] = { INFINITY, INFINITY, INFINITY, -INFINITY, -INFINITY, -INFINITY };
+        const int cmm[6] = { 0, 0, 0, 1, 1, 1 };
+        if (t >= 0)
+            for (int i = 0; i < 3; i++) {
+                const float q0 = p[i].y * sh.Dz - p[i].z * sh.Dy, q1 = p[i].z * sh.Dx - p[i].x * sh.Dz, q2 = p[i].x * sh.Dy - p[i].y * sh.Dx;
+                c[0] = fminf(c[0], q0); c[1] = fminf(c[1], q1); c[2] = fminf(c[2], q2);
+                c[3] = fmaxf(c[3], q0); c[4] = fmaxf(c[4], q1); c[5] = fmaxf(c[5], q2);
+            }
+        block_reduce6(c, cmm, s_red);
+        sh.c0min = c[0]; sh.c1min = c[1]; sh.c2min = c[2]; sh.c0max = c[3]; sh.c1max = c[4]; sh.c2max = c[5];
+        for (int i = tid; i < nclusters; i += blockDim.x) {
+            const float4 b0 = __ldg(cbox + 2 * i), b1 = __ldg(cbox + 2 * i + 1);
+            if (shaft_box(sh, b0.x, b0.y, b0.z, b1.x, b1.y, b1.z)) {
+                const int k = atomicAdd(&s_n, 1);
+                if (k < UPD_CAP) s_list[k] = i;
+            }
+        }
+        __syncthreads();
+        const int n = s_n;
+        if (tid == 0 && (s_any || n > 0)) {
+            s_slot = atomicAdd(kept_count, 1);
+            kept_jobs[s_slot] = jt;
+        }
+        __syncthreads();
+        if (s_any || n > 0) {
+            int *L = kept_lists + (size_t)s_slot * (UPD_CAP + 1);
+            if (tid == 0) L[0] = n > UPD_CAP ? -1 : n;
+            if (tid < n && tid < UPD_CAP) L[1 + tid] = s_list[tid];
+        }
+        __syncthreads();
+    }
+}
+
 struct FFParams {
     const PatchGeom *geom;
     const TriVerts *tv;
@@ -852,6 +978,9 @@ struct FFParams {
     unsigned long long *pair_counter; // [0] pairs traced by this context, [1] of those, pairs whose lower index it owns, [2] pairs that fell back to per-ray LBVH walks
     int njobs;
     const int2 *jobs;    // (row tile, col tile), col tile >= row tile
+    // update runs (PARTIAL, see dz_build_formfactors): the dirty set and, per job, the dirty clusters its tile's shaft meets
+    DzUpdate upd;
+    const int *tile_dirty; // (UPD_CAP + 1) ints per job: count (-1 = more than UPD_CAP: every pair of the tile is dirty), cluster ids
 };
 
 // Tile slots: [0, 64) = the row-tile's patches, [64, 128) = the column-tile's patches.  A listed pair is (rl, cl) plus a
@@ -893,7 +1022,10 @@ struct FFSmem {
 #define FF_CLK(slot) do { } while (0)
 #endif
 
-template <int VARIANT>
+// PARTIAL: an update run -- only the dirty pairs of a tile are traced and stored (pairs with a changed patch, and facing pairs
+// whose shaft meets a dirty box listed for the tile); every other entry of F is left as it is.
+#define UPD_KEEP 0x7fa5a5a5 // bit pattern of a tile entry an update does not store (a NaN no computation produces)
+template <int VARIANT, bool PARTIAL>
 __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams P) {
     extern __shared__ __align__(16) unsigned char ff_smem_raw[];
     FFSmem &sm = *reinterpret_cast<FFSmem *>(ff_smem_raw);
@@ -958,6 +1090,12 @@ __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams 
                 // after the fact (:335-336) -- same matrix, since a zero unoccluded factor gives a zero entry either way
                 trace = (r < c ? f_rc : f_cr) > 0.0f;
                 if (!trace) { f_rc = 0.0f; f_cr = 0.0f; }
+            }
+            if (PARTIAL) {
+                bool dirty = valid && (P.upd.changed[r] || P.upd.changed[c]);
+                if (valid && !dirty && trace)
+                    dirty = pair_meets_dirty(P.tile_dirty + (size_t)job * (UPD_CAP + 1), P.tv, P.upd.cbox, P.upd.crange, P.upd.leaf, min(r, c), max(r, c));
+                if (!dirty) { trace = false; f_rc = __int_as_float(UPD_KEEP); f_cr = f_rc; }
             }
             s_rc[rl][cl] = f_rc;
             s_cr[cl][rl] = f_cr;
@@ -1144,8 +1282,8 @@ __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams 
                 const int a = idx >> 6, b = idx & 63;
                 {
                     const int r = sm.id[a], c = sm.id[TILE + b];
-                    if (r >= 0 && c >= 0) {
-                        const float v = diag ? ((a < b) ? s_rc[a][b] : ((a > b) ? s_cr[a][b] : 0.0f)) : s_rc[a][b];
+                    const float v = diag ? ((a < b) ? s_rc[a][b] : ((a > b) ? s_cr[a][b] : (PARTIAL ? __int_as_float(UPD_KEEP) : 0.0f))) : s_rc[a][b];
+                    if (r >= 0 && c >= 0 && !(PARTIAL && __float_as_int(v) == UPD_KEEP)) {
                         if (P.peer_mode) {
                             const int g = r / P.n_per_rank;
                             DZ_ASSERT(g >= 0 && g < 16 && P.Fpeer[g] != nullptr && c < P.N);
@@ -1155,8 +1293,8 @@ __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams 
                 }
                 if (!diag) { // mirrored tile: row = column patch
                     const int r = sm.id[TILE + a], c = sm.id[b];
-                    if (r >= 0 && c >= 0) {
-                        const float v = s_cr[a][b];
+                    const float v = s_cr[a][b];
+                    if (r >= 0 && c >= 0 && !(PARTIAL && __float_as_int(v) == UPD_KEEP)) {
                         if (P.peer_mode) {
                             const int g = r / P.n_per_rank;
                             P.Fpeer[g][(size_t)(r - g * P.n_per_rank) * P.ldF + c] = v;
@@ -1170,7 +1308,15 @@ __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams 
     }
 }
 
-int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F) {
+bool dz_samples_outside(const daisy_ctx *ctx) {
+    for (int i = 0; i < ctx->S; i++) {
+        const float u = ctx->h_uv[2 * i], v = ctx->h_uv[2 * i + 1];
+        if (!(u >= 0.f && v >= 0.f && u + v <= 1.0f + 1e-6f)) return true;
+    }
+    return false;
+}
+
+int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F, const DzUpdate *upd) {
     const int N = ctx->N;
     if (N == 0) return DAISY_OK;
     cudaStream_t st = ctx->stream;
@@ -1230,27 +1376,56 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
     P.face_ncells = ctx->face_cells; P.face_nlist = ctx->face_list_ints;
 
     { const char *e = getenv("DAISY_FF_RING"); P.ring_on = !(e && e[0] == '0'); }
-    P.all_heavy = 0;
-    for (int i = 0; i < ctx->S; i++) {
-        const float u = ctx->h_uv[2 * i], v = ctx->h_uv[2 * i + 1];
-        if (!(u >= 0.f && v >= 0.f && u + v <= 1.0f + 1e-6f)) P.all_heavy = 1;
-    }
+    P.all_heavy = dz_samples_outside(ctx) ? 1 : 0;
     if (P.all_heavy) P.ring_on = 0;
     P.row0 = r0; P.row1 = r1;
     P.F = write_F ? ctx->d_F : nullptr; P.ldF = ctx->ldF;
     P.peer_mode = peer ? 1 : 0; P.n_per_rank = ctx->rows_per_rank;
     for (int g = 0; g < 16; g++) P.Fpeer[g] = (peer && g < ctx->nranks) ? ctx->peerF[g] : nullptr;
     P.masks = d_masks; P.mrow0 = mrow0; P.mrow1 = mrow1;
+    P.upd = DzUpdate{};
     P.ntiles = ntiles; P.job_counter = d_counter; P.pair_counter = d_pairs; P.njobs = (int)njobs; P.jobs = d_jobs;
     cudaEvent_t e0, e1;
     DZ_CUDA(cudaEventCreate(&e0));
     DZ_CUDA(cudaEventCreate(&e1));
+    // update run: classify the jobs on the device, keep the tiles the update can reach, each with its dirty clusters
+    int2 *d_kept = nullptr;
+    int *d_lists = nullptr;
+    P.tile_dirty = nullptr;
+    if (upd) {
+        P.upd = *upd;
+        int *d_count = nullptr;
+        DZ_CUDA(cudaMalloc(&d_kept, sizeof(int2) * (njobs ? njobs : 1)));
+        DZ_CUDA(cudaMalloc(&d_lists, sizeof(int) * (UPD_CAP + 1) * (njobs ? njobs : 1)));
+        DZ_CUDA(cudaMalloc(&d_count, sizeof(int)));
+        DZ_CUDA(cudaMemsetAsync(d_count, 0, sizeof(int), st));
+        DZ_CUDA(cudaEventRecord(e0, st));
+        if (njobs)
+            k_ff_classify<<<(int)std::min<size_t>(njobs, (size_t)ctx->num_sms * 16), 128, 0, st>>>(d_jobs, (int)njobs, ctx->d_order, ctx->d_triverts, upd->changed,
+                                                                                                  upd->cbox, upd->nclusters, d_kept, d_lists, d_count);
+        DZ_CUDA(cudaGetLastError());
+        DZ_CUDA(cudaEventRecord(e1, st));
+        int kept = 0;
+        DZ_CUDA(cudaMemcpyAsync(&kept, d_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        DZ_CUDA(cudaStreamSynchronize(st));
+        float cms = 0.f;
+        DZ_CUDA(cudaEventElapsedTime(&cms, e0, e1));
+        cudaFree(d_count);
+        ctx->upd_classify_ms = cms;
+        njobs = (size_t)kept;
+        P.njobs = kept; P.jobs = d_kept; P.tile_dirty = d_lists;
+        lap("classification");
+    }
+    if (write_F) ctx->upd_tiles = (int64_t)njobs;
     int blocks_per_sm = 0;
     const size_t smem = sizeof(FFSmem);
-    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_DEVICE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_HOST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (variant == DAISY_FF_DEVICE) DZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_ff_tiles<DAISY_FF_DEVICE>, FF_THREADS, smem));
-    else DZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_ff_tiles<DAISY_FF_HOST>, FF_THREADS, smem));
+    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_DEVICE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_HOST, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_DEVICE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DZ_CUDA(cudaFuncSetAttribute(k_ff_tiles<DAISY_FF_HOST, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kernel = variant == DAISY_FF_DEVICE ? (upd ? k_ff_tiles<DAISY_FF_DEVICE, true> : k_ff_tiles<DAISY_FF_DEVICE, false>)
+                                             : (upd ? k_ff_tiles<DAISY_FF_HOST, true> : k_ff_tiles<DAISY_FF_HOST, false>);
+    DZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, kernel, FF_THREADS, smem));
     if (blocks_per_sm < 1) blocks_per_sm = 1;
     int grid = ctx->num_sms * blocks_per_sm; // persistent CTAs, a multiple of the SM count
     if ((size_t)grid > njobs) grid = (int)njobs;
@@ -1259,10 +1434,7 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
     P.scratch = d_scratch;
     lap("allocations, uploads");
     DZ_CUDA(cudaEventRecord(e0, st));
-    if (grid > 0) {
-        if (variant == DAISY_FF_DEVICE) k_ff_tiles<DAISY_FF_DEVICE><<<grid, FF_THREADS, smem, st>>>(P);
-        else k_ff_tiles<DAISY_FF_HOST><<<grid, FF_THREADS, smem, st>>>(P);
-    }
+    if (grid > 0) kernel<<<grid, FF_THREADS, smem, st>>>(P);
     DZ_CUDA(cudaGetLastError());
     DZ_CUDA(cudaEventRecord(e1, st));
     unsigned long long pairs[3] = { 0, 0, 0 };
@@ -1297,7 +1469,7 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
 #endif
     if (write_F) { ctx->ff_ms = ms; ctx->pairs_traced = (int64_t)pairs[0]; ctx->pairs_owned = (int64_t)pairs[1]; ctx->pairs_heavy = (int64_t)pairs[2]; }
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    cudaFree(d_jobs); cudaFree(d_counter); cudaFree(d_pairs); cudaFree(d_scratch);
+    cudaFree(d_jobs); cudaFree(d_counter); cudaFree(d_pairs); cudaFree(d_scratch); cudaFree(d_kept); cudaFree(d_lists);
     free(h_jobs);
     lap("clean-up");
     return DAISY_OK;

@@ -139,6 +139,31 @@ extern "C" int daisy_group_formfactors_build(daisy_group *g, int variant) {
     return rc;
 }
 
+extern "C" int daisy_group_update_geometry(daisy_group *g, const float *vertices, int nv, const float *normals, int nn) {
+    DZ_REQUIRE(g, DAISY_E_INVALID, "daisy_group_update_geometry: null group");
+    return for_each_device(g, "daisy_group_update_geometry", [&](int i) { return daisy_ctx_update_geometry(g->ctx[(size_t)i], vertices, nv, normals, nn); });
+}
+
+extern "C" int daisy_group_formfactors_update(daisy_group *g, int variant) {
+    DZ_REQUIRE(g, DAISY_E_INVALID, "daisy_group_formfactors_update: null group");
+    nvtxRangePushA("daisy_group_formfactors_update");
+    // the peers are wired by the first build; an update without one traces everything and needs them just the same
+    int rc = DAISY_OK;
+    if (g->ndev > 1 && !g->ctx[0]->peers_set) {
+        rc = for_each_device(g, "daisy_group_formfactors_update (alloc)", [&](int i) { return daisy_formfactors_alloc(g->ctx[(size_t)i]); });
+        if (!rc) {
+            float *F[16] = { nullptr };
+            for (int i = 0; i < g->ndev; i++) F[i] = g->ctx[(size_t)i]->d_F;
+            for (int i = 0; i < g->ndev && !rc; i++) rc = dz_ctx_set_peer_pointers(g->ctx[(size_t)i], F, g->ndev);
+        }
+    }
+    if (!rc) rc = for_each_device(g, "daisy_group_formfactors_update", [&](int i) { return daisy_formfactors_update(g->ctx[(size_t)i], variant); });
+    // devices store into each other's rows: every matrix may have changed after the join
+    for (int i = 0; i < g->ndev; i++) g->ctx[(size_t)i]->F_version++;
+    nvtxRangePop();
+    return rc;
+}
+
 static int owner_of(daisy_group *g, int row) {
     const int n = g->ctx[0]->rows_per_rank;
     int o = n > 0 ? row / n : 0;

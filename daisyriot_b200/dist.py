@@ -81,6 +81,18 @@ def build_formfactors_sharded(optixP, variant: int = _lib.FF_DEVICE, group=None,
         tdist.barrier(group=group)  # peers have finished writing into this rank's rows
 
 
+def update_formfactors_sharded(optixP, variant: int = _lib.FF_DEVICE, group=None):
+    """Row-sharded matrix update after ``optixP.updateGeometry`` (called with identical arrays on every rank): each rank
+    re-traces its share of the tiles the change can reach -- with the peer mappings of an earlier
+    :func:`build_formfactors_sharded`, each such tile on exactly one rank -- then all ranks barrier as after the build."""
+    import torch
+    import torch.distributed as tdist
+    _lib.check(_lib.lib().daisy_formfactors_update(optixP._ctx, variant), "formfactors_update")
+    if optixP.nranks > 1:
+        torch.cuda.synchronize()
+        tdist.barrier(group=group)  # peers have finished writing into this rank's rows
+
+
 class _DevMem:
     """Exposes a raw device pointer through __cuda_array_interface__ so torch can alias it without a copy."""
 

@@ -231,6 +231,30 @@ def cornell_box(n_patches: int, n_fluorescent: int = 2, seed: int = 0x5EED) -> S
     return sc
 
 
+CORNELL_LAMP, CORNELL_SHORT_BLOCK, CORNELL_TALL_BLOCK = [15], [5, 6, 7, 8, 9], [10, 11, 12, 13, 14]  # quads of cornell_box
+
+
+def cornell_moved(scene: Scene, quads, offset=(0.0, 0.0, 0.0), angle_y: float = 0.0):
+    """(vertices, normals) of a :func:`cornell_box` scene with the given quads rotated by ``angle_y`` radians about the
+    vertical axis through their centre, then translated by ``offset``.  Quad q holds triangles [q*2*nu*nv, (q+1)*2*nu*nv) and
+    its own vertices and normal, so nothing else moves."""
+    per = scene.numtriangles // 16
+    tri = np.concatenate([scene.tri[q * per:(q + 1) * per] for q in quads])
+    vi, ni = np.unique(tri[:, :3]), np.unique(tri[:, 3:])
+    V = np.array(scene.vertices, np.float64)
+    VN = np.array(scene.normals, np.float64)
+    c, s_ = np.cos(angle_y), np.sin(angle_y)
+    R = np.array([[c, 0, s_], [0, 1, 0], [-s_, 0, c]])
+    centre = V[vi].mean(axis=0)
+    V[vi] = (V[vi] - centre) @ R.T + centre + np.asarray(offset, np.float64)
+    VN[ni] = VN[ni] @ R.T
+    V32, VN32 = np.array(scene.vertices, np.float32), np.array(scene.normals, np.float32)
+    V32[vi] = V[vi].astype(np.float32)
+    if angle_y:
+        VN32[ni] = VN[ni].astype(np.float32)
+    return V32, VN32
+
+
 def write_obj(scene: Scene, directory: str, stem: str | None = None):
     """Write ``scene`` as OBJ + MTL (the inverse of :func:`load_obj`; float32 values survive the round trip).
     Lets the reference's own loader (``MeshS::loadFromFile``) read the synthetic scenes."""

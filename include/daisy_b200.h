@@ -133,6 +133,26 @@ int daisy_ctx_face_count(daisy_ctx *ctx);
 int daisy_formfactors_stats(daisy_ctx *ctx, int64_t *pairs_traced, int64_t *pairs_owned, int64_t *rays, double *lbvh_ms,
                             double *ff_ms);
 
+/* ---- geometry updates ---------------------------------------------------------------------------------------
+ * daisy_ctx_update_geometry: new vertex positions (nv x 3) and/or normals (nn x 3) for the mesh given to daisy_ctx_create;
+ * the triangle list stays, nv and nn must be the create-time counts (DAISY_E_INVALID otherwise), NULL keeps that array.
+ * Everything derived from the geometry is rebuilt as daisy_ctx_create builds it (bounds, plane ids, face grids, LBVH,
+ * patch records), so closest hit, daisy_trace_screen, daisy_visibility_masks and daisy_unoccluded_rows answer for the new
+ * geometry at once.  F is left as it is until daisy_formfactors_update.
+ * daisy_formfactors_update: F becomes, bit for bit, what daisy_formfactors_build(ctx, variant) gives on a fresh context with
+ * the current geometry, samples and partition, but only the entries that can differ from the matrix F holds are traced and
+ * stored: pairs with a changed patch (a position or normal differs bitwise), and pairs whose shaft meets a moved triangle in
+ * its recorded or its current position.  The context records the variant, samples and geometry of its last build or update;
+ * everything is traced when F holds no such matrix (no build yet, daisy_formfactors_write_rows since, another variant, other
+ * samples) or the sample pattern has points outside the triangle.  Solvers on the context stay valid and rescan F (their B and
+ * residual are untouched: reset them).  daisy_formfactors_stats describes the update's kernel run and the rebuild's LBVH.
+ * Several processes (CUDA-IPC peers): every rank calls both with identical arrays, then the host barriers, as for the build.
+ * daisy_formfactors_update_stats: the last update's triangles changed, tiles and facing pairs this context re-traced, and
+ * device milliseconds of the tile classification. */
+int daisy_ctx_update_geometry(daisy_ctx *ctx, const float *vertices, int nv, const float *normals, int nn);
+int daisy_formfactors_update(daisy_ctx *ctx, int variant);
+int daisy_formfactors_update_stats(daisy_ctx *ctx, int64_t *tris_changed, int64_t *tiles_retraced, int64_t *pairs_retraced, double *classify_ms);
+
 /* multi-GPU build without redundant tracing: allocate (and zero) this rank's rows, publish a 64-byte CUDA IPC handle,
  * receive every rank's handle (nranks x 64 bytes, rank order), then daisy_formfactors_build computes each
  * upper-triangle tile on exactly one rank and stores the tile / its mirror straight into the owning ranks' matrices
@@ -251,6 +271,9 @@ int daisy_group_formfactors_write_rows(daisy_group *g, int row0, int nrows, cons
 int daisy_group_formfactors_to_csc(daisy_group *g, int64_t *nnz, float *values, int32_t *inner_idx, int32_t *outer_ptr);
 /* unique mutually facing pairs of the whole matrix, rays cast, slowest device's LBVH / form-factor kernel milliseconds */
 int daisy_group_formfactors_stats(daisy_group *g, int64_t *pairs, int64_t *rays, double *lbvh_ms, double *ff_ms);
+/* daisy_ctx_update_geometry / daisy_formfactors_update on every device (each traces its share of the tiles the update reaches) */
+int daisy_group_update_geometry(daisy_group *g, const float *vertices, int nv, const float *normals, int nn);
+int daisy_group_formfactors_update(daisy_group *g, int variant);
 int daisy_group_solver_create(daisy_group *g, int K, const float *E, const float *M, int nmat, const int32_t *mat_idx,
                               daisy_group_solver **out);
 void daisy_group_solver_destroy(daisy_group_solver *gs);

@@ -10,3 +10,4 @@ done
 timeout 1800 python -m pytest tests/test_gpu_parity.py tests/test_gpu_gather_shapes.py -x -q -m gpu -k "(radmat or fixture_scene_rows or sample_counts or edge_heavy or irregular or empty_and_single or gather or closest or trace_screen or face_grids or perforated or chained) and not fused_exchange" 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_far_geometry.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_converge_device.py -x -q -m gpu -k "not group and not two_process and not shim" 2>&1 | tail -4
+timeout 1800 python -m pytest tests/test_gpu_geometry_update.py -x -q -m gpu -k "not group" 2>&1 | tail -4
