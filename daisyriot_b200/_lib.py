@@ -54,6 +54,8 @@ SYMBOLS = {
     "daisy_formfactors_read_rows": (_i, [_vp, _i, _i, _fp]),
     "daisy_formfactors_to_csc": (_i, [_vp, _i64p, _fp, _ip, _ip]),
     "daisy_formfactors_write_rows": (_i, [_vp, _i, _i, _fp]),
+    "daisy_formfactors_write_csc": (_i, [_vp, C.c_int64, _fp, _ip, _ip]),
+    "daisy_formfactors_csc_uploads": (_i, [_vp]),
     "daisy_visibility_masks": (_i, [_vp, _i, _i, _i, C.POINTER(C.c_uint64)]),
     "daisy_formfactors_row_digest": (_i, [_vp, _i, _i, C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
     "daisy_formfactors_stats": (_i, [_vp, _i64p, _i64p, _i64p, _dp, _dp]),
@@ -89,6 +91,7 @@ SYMBOLS = {
     "daisy_group_formfactors_read_rows": (_i, [_vp, _i, _i, _fp]),
     "daisy_group_formfactors_write_rows": (_i, [_vp, _i, _i, _fp]),
     "daisy_group_formfactors_to_csc": (_i, [_vp, _i64p, _fp, _ip, _ip]),
+    "daisy_group_formfactors_write_csc": (_i, [_vp, C.c_int64, _fp, _ip, _ip]),
     "daisy_group_formfactors_stats": (_i, [_vp, _i64p, _i64p, _dp, _dp]),
     "daisy_group_update_geometry": (_i, [_vp, _fp, _i, _fp, _i]),
     "daisy_group_formfactors_update": (_i, [_vp, _i]),

@@ -204,6 +204,14 @@ class OptixPrimeFunctionality:
         _lib.check(_lib.lib().daisy_formfactors_write_rows(self._ctx, row0, a.shape[0], _lib.fptr(a)), "formfactors_write_rows")
         return RadMat(self)
 
+    def loadRadiosityMatrixCSC(self, values, inner, outer) -> RadMat:
+        """The matrix-cache path from the CSC arrays themselves (``DeserializeMat``'s ``SpMat``, :func:`deserialize_csc`):
+        validated and scattered on the device, no dense matrix on the host.  ``outer`` holds N + 1 column starts.  Entries
+        not listed become +0.0; partitioned contexts keep the rows of their range."""
+        v, i, o = _csc_arrays(values, inner, outer, self.N)
+        _lib.check(_lib.lib().daisy_formfactors_write_csc(self._ctx, v.size, _lib.fptr(v), _lib.iptr(i), _lib.iptr(o)), "formfactors_write_csc")
+        return RadMat(self)
+
     def visibilityMasks(self, row0=0, nrows=None, variant=_lib.FF_DEVICE) -> np.ndarray:
         nrows = self.N - row0 if nrows is None else nrows
         out = np.empty((nrows, self.N), np.uint64)
@@ -370,6 +378,25 @@ class DeviceGroup:
         _lib.check(_lib.lib().daisy_group_formfactors_read_rows(self._g, row0, nrows, _lib.fptr(out)), "group_formfactors_read_rows")
         return out
 
+    def to_csc(self):
+        """(values, innerIndices, outerStarts) of the whole matrix, as :meth:`RadMat.to_csc` gives them on one GPU."""
+        L = _lib.lib()
+        nnz = C.c_int64()
+        _lib.check(L.daisy_group_formfactors_to_csc(self._g, C.byref(nnz), None, None, None), "group_formfactors_to_csc")
+        vals = np.empty(nnz.value, np.float32)
+        inner = np.empty(nnz.value, np.int32)
+        outer = np.empty(self.N + 1, np.int32)
+        _lib.check(L.daisy_group_formfactors_to_csc(self._g, C.byref(nnz), _lib.fptr(vals), _lib.iptr(inner), _lib.iptr(outer)),
+                   "group_formfactors_to_csc")
+        return vals, inner, outer
+
+    def loadRadiosityMatrixCSC(self, values, inner, outer):
+        """:meth:`OptixPrimeFunctionality.loadRadiosityMatrixCSC` over the group: every device validates, then keeps its rows."""
+        v, i, o = _csc_arrays(values, inner, outer, self.N)
+        _lib.check(_lib.lib().daisy_group_formfactors_write_csc(self._g, v.size, _lib.fptr(v), _lib.iptr(i), _lib.iptr(o)),
+                   "group_formfactors_write_csc")
+        return self
+
     def stats(self):
         p, r, a, b = C.c_int64(), C.c_int64(), C.c_double(), C.c_double()
         _lib.check(_lib.lib().daisy_group_formfactors_stats(self._g, C.byref(p), C.byref(r), C.byref(a), C.byref(b)))
@@ -432,6 +459,16 @@ class GroupSolver:
         B = np.ascontiguousarray(B, np.float32)
         R = np.ascontiguousarray(R, np.float32)
         _lib.check(_lib.lib().daisy_group_solver_write(self._s, _lib.fptr(B), _lib.fptr(R)), "group_solver_write")
+
+
+def _csc_arrays(values, inner, outer, n: int):
+    """Contiguous float32 / int32 copies of CSC arrays, checked for their lengths (the values themselves the library checks)."""
+    v = np.ascontiguousarray(values, np.float32).reshape(-1)
+    i = np.ascontiguousarray(inner, np.int32).reshape(-1)
+    o = np.ascontiguousarray(outer, np.int32).reshape(-1)
+    if o.size != n + 1 or i.size != v.size:
+        raise ValueError("CSC arrays: outer needs N + 1 entries and inner as many as values")
+    return v, i, o
 
 
 def _geometry_arrays(mesh: MeshS, vertices, normals):
@@ -509,6 +546,19 @@ def deserialize_mat(path: str):
     return dense
 
 
+def deserialize_csc(path: str):
+    """``Lightning::DeserializeMat`` (``Lightning.h:51-74``) -> (values, innerIndices, outerStarts) as the file holds them,
+    with the closing sentinel ``outer[N] = nnz`` appended (the file stores outerSize entries); no dense matrix is built."""
+    with open(path, "rb") as f:
+        rows, cols, nnz, a, b = struct.unpack("<5i", f.read(20))
+        vals = np.frombuffer(f.read(4 * nnz), np.float32)
+        outer = np.frombuffer(f.read(4 * a), np.int32)
+        inner = np.frombuffer(f.read(4 * nnz), np.int32)
+    if vals.size != nnz or outer.size != a or inner.size != nnz:
+        raise ValueError("%s: truncated matrix file" % path)
+    return vals, inner, np.append(outer, np.int32(nnz)).astype(np.int32)
+
+
 class Lightning:
     """Reference ``Lightning`` base (``Lightning.h:7-97``): owns ``RadMat``; ``get_lightning`` is the factory."""
 
@@ -554,7 +604,7 @@ class Lightning:
 
     def initMatFromFile(self, mesh, optixP, matfile):  # Lightning.h:84-96
         if os.path.exists(matfile):
-            self.RadMat = optixP.loadRadiosityMatrix(deserialize_mat(matfile))
+            self.RadMat = optixP.loadRadiosityMatrixCSC(*deserialize_csc(matfile))
         else:
             self.initMat(mesh, optixP)
             serialize_mat(matfile, *self.RadMat.to_csc(), mesh.numtriangles)

@@ -502,7 +502,7 @@ extern "C" int daisy_unoccluded_rows(daisy_ctx *ctx, int variant, int row0, int 
     return rc;
 }
 
-static int ensure_F(daisy_ctx *ctx) {
+int dz_ensure_F(daisy_ctx *ctx) {
     if (ctx->d_F) return DAISY_OK;
     size_t rows = (size_t)(ctx->row1 - ctx->row0);
     size_t bytes = sizeof(float) * (rows ? rows : 1) * (size_t)ctx->ldF;
@@ -530,7 +530,7 @@ extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     DZ_CUDA(cudaSetDevice(ctx->device));
     const bool timing = getenv("DAISY_TIMING") != nullptr; // stderr: where the wall time of the call goes
     const auto t0 = std::chrono::steady_clock::now();
-    int rc = ensure_F(ctx);
+    int rc = dz_ensure_F(ctx);
     if (rc) return rc;
     if (timing) { cudaStreamSynchronize(ctx->stream); fprintf(stderr, "daisy_formfactors_build: matrix allocation + zero fill %.3f s\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count()); }
     rc = dz_set_samples_const(ctx);
@@ -559,7 +559,7 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
     DZ_REQUIRE(ctx->S >= 1, DAISY_E_STATE, "daisy_formfactors_update: call daisy_ctx_set_samples first");
     DzRange range_("daisy_formfactors_update: dirty set, tile classification, partial k_ff_tiles");
     DZ_CUDA(cudaSetDevice(ctx->device));
-    int rc = ensure_F(ctx);
+    int rc = dz_ensure_F(ctx);
     if (rc) return rc;
     rc = dz_set_samples_const(ctx);
     if (rc) return rc;
@@ -661,7 +661,7 @@ extern "C" int daisy_formfactors_update_stats(daisy_ctx *ctx, int64_t *tris_chan
 extern "C" int daisy_formfactors_alloc(daisy_ctx *ctx) {
     DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_formfactors_alloc: null context");
     DZ_CUDA(cudaSetDevice(ctx->device));
-    int rc = ensure_F(ctx);
+    int rc = dz_ensure_F(ctx);
     if (rc) return rc;
     DZ_CUDA(cudaStreamSynchronize(ctx->stream)); // the zero fill must be complete before any peer may write
     return DAISY_OK;
@@ -728,7 +728,7 @@ extern "C" int daisy_formfactors_write_rows(daisy_ctx *ctx, int row0, int nrows,
     DZ_REQUIRE(ctx && (nrows == 0 || in), DAISY_E_INVALID, "daisy_formfactors_write_rows: null argument");
     DZ_REQUIRE(nrows >= 0 && row0 >= ctx->row0 && row0 + nrows <= ctx->row1, DAISY_E_INVALID, "daisy_formfactors_write_rows: rows outside this context's range");
     DZ_CUDA(cudaSetDevice(ctx->device));
-    int rc = ensure_F(ctx);
+    int rc = dz_ensure_F(ctx);
     if (rc) return rc;
     if (nrows)
         DZ_CUDA(cudaMemcpy2DAsync(ctx->d_F + (size_t)(row0 - ctx->row0) * ctx->ldF, sizeof(float) * (size_t)ctx->ldF, in, sizeof(float) * (size_t)ctx->N,
@@ -745,8 +745,9 @@ extern "C" int daisy_formfactors_to_csc(daisy_ctx *ctx, int64_t *nnz, float *val
     DZ_REQUIRE(ctx->have_F, DAISY_E_STATE, "daisy_formfactors_to_csc: no form factors yet");
     DZ_REQUIRE(ctx->nranks == 1, DAISY_E_STATE, "daisy_formfactors_to_csc: single-GPU contexts only");
     DZ_CUDA(cudaSetDevice(ctx->device));
+    if (!dz_csc_host()) return dz_csc_export(&ctx, 1, nnz, values, inner_idx, outer_ptr, "daisy_formfactors_to_csc");
     const int N = ctx->N;
-    // host-side conversion in row chunks (this is the hand-back path for callers that still want an Eigen SpMat)
+    // DAISY_CSC_HOST=1: host-side conversion of dense row read-backs in row chunks
     std::vector<int64_t> colcount((size_t)N + 1, 0);
     const int chunk = (int)fmax(1.0, fmin((double)N, (double)(128u << 20) / (4.0 * (N ? N : 1))));
     std::vector<float> rows((size_t)chunk * (N ? N : 1));

@@ -274,6 +274,14 @@ struct __align__(16) DzFace {
 
 __device__ __forceinline__ f3 xyz(float4 v) { return mk3(v.x, v.y, v.z); }
 
+// streaming load of 4 floats that are read once: no L1 allocation (F in the gather passes, the tile scan, the CSC count)
+__device__ __forceinline__ float4 ldg_stream(const float *p) {
+    float4 r;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::128B.v4.f32 {%0,%1,%2,%3}, [%4];"
+                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
+    return r;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 struct daisy_ctx {
     int device = 0;
@@ -339,6 +347,9 @@ struct daisy_ctx {
     // last daisy_formfactors_update
     int64_t upd_tris_changed = 0, upd_tiles = 0, upd_pairs = 0;
     double upd_classify_ms = 0.0;
+    // last daisy_formfactors_write_csc: uploads of the CSC arrays (1: kept resident while validated and scattered, 2: chunks
+    // uploaded for the validation, rows only, and again for the scatter)
+    int csc_uploads = 0;
 };
 
 // The part of F an update has to recompute (formfactor.cu, daisy_formfactors_update): per-triangle changed flags and the
@@ -371,3 +382,8 @@ int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per
 int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F,
                          const DzUpdate *upd = nullptr);                                                    // formfactor.cu
 bool dz_samples_outside(const daisy_ctx *ctx);                                                              // formfactor.cu
+int dz_ensure_F(daisy_ctx *ctx); // allocate F (zero-filled) if it does not exist yet                          // api.cu
+// the matrix cache on the device (csc.cu): ctx[0..n) hold rows [row0, row1) each, in ascending order, together all N rows
+bool dz_csc_host(); // DAISY_CSC_HOST=1: hand F back through the host conversion of dense row read-backs instead
+int dz_csc_export(daisy_ctx *const *ctx, int n, int64_t *nnz, float *values, int32_t *inner_idx, int32_t *outer_ptr, const char *what);
+int dz_csc_import(daisy_ctx *const *ctx, int n, int64_t nnz, const float *values, const int32_t *inner_idx, const int32_t *outer_ptr, const char *what);

@@ -126,12 +126,6 @@ __device__ __forceinline__ void tma_load_3d(void *dst, const CUtensorMap *tm, in
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
                  ::"r"(smem_u32(dst)), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ float4 ldg_stream(const float *p) {
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.L2::128B.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-}
 
 // Device converge (daisy_solver_converge_device, DESIGN 3.3): the passes of one call are launched back to back and every pass
 // but the first applies converge_lightning's stop rule to the band sums the previous pass left in the tails of the buffer it

@@ -211,6 +211,11 @@ extern "C" int daisy_group_formfactors_write_rows(daisy_group *g, int row0, int 
 extern "C" int daisy_group_formfactors_to_csc(daisy_group *g, int64_t *nnz, float *values, int32_t *inner_idx, int32_t *outer_ptr) {
     DZ_REQUIRE(g && nnz, DAISY_E_INVALID, "daisy_group_formfactors_to_csc: null argument");
     if (g->ndev == 1) return daisy_formfactors_to_csc(g->ctx[0], nnz, values, inner_idx, outer_ptr);
+    if (!dz_csc_host()) {
+        for (daisy_ctx *c : g->ctx) DZ_REQUIRE(c->have_F, DAISY_E_STATE, "daisy_group_formfactors_to_csc: no form factors yet");
+        return dz_csc_export(g->ctx.data(), g->ndev, nnz, values, inner_idx, outer_ptr, "daisy_group_formfactors_to_csc");
+    }
+    // DAISY_CSC_HOST=1: host-side conversion of dense row read-backs
     const int N = g->N;
     std::vector<int64_t> colcount((size_t)N + 1, 0);
     int chunk = (int)((128u << 20) / (4.0 * (N ? N : 1)));
@@ -243,6 +248,14 @@ extern "C" int daisy_group_formfactors_to_csc(daisy_group *g, int64_t *nnz, floa
             }
     }
     return DAISY_OK;
+}
+
+// every device validates the whole matrix before any device stores; each keeps the rows of its block, and a device that owns
+// no rows gets have_F as daisy_group_formfactors_write_rows gives it
+extern "C" int daisy_group_formfactors_write_csc(daisy_group *g, int64_t nnz, const float *values, const int32_t *inner_idx, const int32_t *outer_ptr) {
+    DZ_REQUIRE(g, DAISY_E_INVALID, "daisy_group_formfactors_write_csc: null group");
+    DzRange range_("daisy_group_formfactors_write_csc");
+    return dz_csc_import(g->ctx.data(), g->ndev, nnz, values, inner_idx, outer_ptr, "daisy_group_formfactors_write_csc");
 }
 
 extern "C" int daisy_group_formfactors_stats(daisy_group *g, int64_t *pairs, int64_t *rays, double *lbvh_ms, double *ff_ms) {

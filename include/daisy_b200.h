@@ -114,10 +114,24 @@ int daisy_formfactors_ld(daisy_ctx *ctx, int64_t *ld_out);
 /* copy rows to host: out[(r-row0)*N + c], rows must lie inside the context's row range */
 int daisy_formfactors_read_rows(daisy_ctx *ctx, int row0, int nrows, float *out);
 /* refill an Eigen::SparseMatrix<float> (column-major CSC, sorted inner indices, as setFromTriplets leaves it,
- * VS/OptixPrimeFunctionality.cpp:25).  Call with values==NULL to get nnz first.  Single-GPU contexts only. */
+ * VS/OptixPrimeFunctionality.cpp:25).  Call with values==NULL to get nnz first.  Single-GPU contexts only.
+ * Entry (r, c), c < N, is listed exactly when F[r][c] != 0.0f (+-0 are not, NaN, +-inf and denormals are), values bit for bit.
+ * The conversion runs on the device and only the CSC arrays cross PCIe; DAISY_CSC_HOST=1 converts dense row read-backs on the
+ * host instead (same arrays).  DAISY_E_INVALID when nnz > 2^31 - 1 (the count-only call still returns nnz). */
 int daisy_formfactors_to_csc(daisy_ctx *ctx, int64_t *nnz, float *values, int32_t *inner_idx, int32_t *outer_ptr);
 /* load a dense matrix instead of building it (the reference's on-disk cache path, VS/Lightning.h:84-96) */
 int daisy_formfactors_write_rows(daisy_ctx *ctx, int row0, int nrows, const float *in);
+/* load F from a CSC matrix (Eigen::SparseMatrix<float> compressed, column-major, as DeserializeMat leaves it, VS/Lightning.h:51-74):
+ * outer_ptr = N+1 column starts (outer_ptr[N] == nnz), inner_idx = row of each value, strictly ascending within a column.  Every
+ * entry not listed becomes +0.0; listed values are stored bit for bit (explicit zeros and -0.0 included).  Partitioned contexts
+ * take the whole matrix and keep the rows of their range.  Same effect on the context as daisy_formfactors_write_rows (F_version
+ * moves, the build record is cleared, solvers rescan).  Invalid input: DAISY_E_INVALID and F unchanged.  Only the CSC arrays
+ * cross PCIe; they stay resident on the device while validated and scattered when they fit in half its free memory, else they
+ * go up in chunks twice (validation, then the scatter). */
+int daisy_formfactors_write_csc(daisy_ctx *ctx, int64_t nnz, const float *values, const int32_t *inner_idx, const int32_t *outer_ptr);
+/* how the last daisy_formfactors_write_csc on this context staged the arrays: 1 = one upload kept resident, 2 = column chunks
+ * uploaded twice (row indices for the validation, then values and rows for the scatter), 0 = none yet */
+int daisy_formfactors_csc_uploads(daisy_ctx *ctx);
 /* parity aid: visibility hit masks of rows [row0,row0+nrows): out[(r-row0)*N + c], bit i = sample i of the pair
  * (min(r,c) -> max(r,c)) saw its destination (the test at VS/OptixPrimeFunctionality.cpp:208); 0 if not traced. */
 int daisy_visibility_masks(daisy_ctx *ctx, int variant, int row0, int nrows, uint64_t *out);
@@ -269,6 +283,8 @@ int daisy_group_formfactors_build(daisy_group *g, int variant);
 int daisy_group_formfactors_read_rows(daisy_group *g, int row0, int nrows, float *out);
 int daisy_group_formfactors_write_rows(daisy_group *g, int row0, int nrows, const float *in);      /* the matrix-cache path, rows routed to their owners */
 int daisy_group_formfactors_to_csc(daisy_group *g, int64_t *nnz, float *values, int32_t *inner_idx, int32_t *outer_ptr);
+/* daisy_formfactors_write_csc for the whole group: every device validates before any stores, each keeps its row block */
+int daisy_group_formfactors_write_csc(daisy_group *g, int64_t nnz, const float *values, const int32_t *inner_idx, const int32_t *outer_ptr);
 /* unique mutually facing pairs of the whole matrix, rays cast, slowest device's LBVH / form-factor kernel milliseconds */
 int daisy_group_formfactors_stats(daisy_group *g, int64_t *pairs, int64_t *rays, double *lbvh_ms, double *ff_ms);
 /* daisy_ctx_update_geometry / daisy_formfactors_update on every device (each traces its share of the tiles the update reaches) */

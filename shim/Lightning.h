@@ -89,24 +89,20 @@ protected:
         std::copy(op.begin(), op.end(), m.outerIndexPtr());
         return true;
     }
-    // dense rows of the cached matrix go to the GPU in chunks (daisy_formfactors_write_rows = the cache path of the C-ABI)
-    void upload(SpMat &m, OptixPrimeFunctionality &optixP) {
-        const int n = (int)m.rows();
-        Eigen::SparseMatrix<float, Eigen::RowMajor> R = m;
-        const int chunk = std::max(1, std::min(n, (int)((64u << 20) / (4u * (unsigned)std::max(n, 1)))));
-        std::vector<float> rows((size_t)chunk * n);
-        for (int r0 = 0; r0 < n; r0 += chunk) {
-            const int nr = std::min(chunk, n - r0);
-            std::fill(rows.begin(), rows.begin() + (size_t)nr * n, 0.f);
-            for (int r = 0; r < nr; r++)
-                for (Eigen::SparseMatrix<float, Eigen::RowMajor>::InnerIterator it(R, r0 + r); it; ++it) rows[(size_t)r * n + it.col()] = it.value();
-            if (!check(daisy_group_formfactors_write_rows(optixP.group, r0, nr, rows.data()))) return;
+    // the cached matrix goes to the GPUs as it is, CSC arrays only: validated there, then scattered into every device's rows
+    // (entries not listed become +0.0, as in a dense load of the same matrix)
+    void upload(SpMat &m, OptixPrimeFunctionality &optixP, int n) {
+        if (m.rows() != n || m.cols() != n) { // write_csc reads n + 1 column starts: a cache of another mesh is refused here
+            std::cerr << "Cached matrix is " << m.rows() << " x " << m.cols() << ", the mesh has " << n << " patches: not loaded" << std::endl;
+            return;
         }
+        m.makeCompressed();
+        check(daisy_group_formfactors_write_csc(optixP.group, (int64_t)m.nonZeros(), m.valuePtr(), m.innerIndexPtr(), m.outerIndexPtr()));
     }
     void initMatFromFile(MeshS &mesh, OptixPrimeFunctionality &optixP, char *matfile) { // Lightning.h:84-96
         RadMat = SpMat(mesh.numtriangles, mesh.numtriangles);
         if (DeserializeMat(RadMat, matfile)) {
-            upload(RadMat, optixP);
+            upload(RadMat, optixP, mesh.numtriangles);
             std::cout << "Deserialized matrix" << std::endl;
         } else {
             initMat(mesh, optixP);
