@@ -10,7 +10,8 @@
 // with work items (row block) x (column range):
 //   k_gather_tma<K>      K <= 9: a producer warp fills a 6-stage shared-memory ring with tiled TMA loads (F tile +
 //                        residual band slices), 8 consumer warps do K FMAs per F element; the default
-//   k_gather_mma<K>      K = 16 / 32: tcgen05 3xTF32 tensor-core kernel with the F operand staged in TMEM (gather_mma.cuh)
+//   k_gather_mma<K>      K = 16 / 32 / 64: tcgen05 3xTF32 tensor-core kernel with the F operand staged in TMEM (gather_mma.cuh);
+//                        the only kernel for K > 32
 //   k_gather_partial<K>  the first-generation register-prefetch kernel, kept selectable (DAISY_GATHER=ldg) as a reference point
 // k_gather_epilogue sums the column-range partials, applies the per-material KxK matrix, accumulates B, writes the new
 // residual into this rank's exchange block -- or, with the fused exchange, into every rank's buffer over NVLink -- and
@@ -63,7 +64,7 @@ struct daisy_solver {
     int64_t occupied = 0;
     double scan_ms = 0.0;
     bool use_tma = true;
-    bool use_mma = false;               // K = 16 / 32: tcgen05 3xTF32 path (gather_mma.cuh)
+    bool use_mma = false;               // K = 16 / 32 / 64: tcgen05 3xTF32 path (gather_mma.cuh)
     bool fused_epi = false;             // k_gather_tma does the epilogue (and the exchange wait) itself: one launch per pass
     float *d_split = nullptr;           // [Rh; Rl]: 2*Kp x ncolsP, rewritten at the start of every pass
     int ncolsP = 0;
@@ -948,8 +949,8 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
         P.stop.G = s->G; P.stop.K = s->K;
     }
     int rc;
-    if (s->use_mma && (K == 16 || K == 32)) {
-        if constexpr (K == 16 || K == 32) {
+    if (s->use_mma && (K == 16 || K == 32 || K == 64)) {
+        if constexpr (K == 16 || K == 32 || K == 64) {
             constexpr size_t smem = mm_smem_bytes<K>();
             static bool attr_done[64] = { false }; // per device
             if (!attr_done[c->device & 63]) {
@@ -963,6 +964,9 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
             DZ_CUDA(cudaGetLastError());
         }
         rc = DAISY_OK;
+    } else if constexpr (K > 32) {
+        daisy_set_error("%d bands run only on the tensor-core kernel", K); // daisy_solver_create refuses the other paths
+        return DAISY_E_INVALID;
     } else if (s->use_tma) {
         constexpr int NST = tma_nstage<K>();
         size_t smem = (size_t)NST * tma_stage_bytes<K>() + 2 * NST * sizeof(uint64_t) + tma_epi_bytes<K>();
@@ -1056,6 +1060,7 @@ static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull, cons
     case 9: return launch_pass_K<9>(s, wait_seq, stop);
     case 16: return launch_pass_K<16>(s, wait_seq, stop);
     case 32: return launch_pass_K<32>(s, wait_seq, stop);
+    case 64: return launch_pass_K<64>(s, wait_seq, stop);
     }
     daisy_set_error("unsupported padded band count %d", s->Kp);
     return DAISY_E_INVALID;
@@ -1143,7 +1148,8 @@ static void plan(daisy_solver *s) {
     s->grid = sms;
     const char *env = getenv("DAISY_GATHER");
     s->use_tma = !(env && strcmp(env, "ldg") == 0);
-    // wide band counts run on the tensor cores unless DAISY_GATHER=fp32 (or ldg) asks for the CUDA-core kernels
+    // wide band counts run on the tensor cores unless DAISY_GATHER=fp32 (or ldg) asks for the CUDA-core kernels (K <= 32 only:
+    // daisy_solver_create refuses those for more bands)
     s->use_mma = s->use_tma && s->Kp >= 16 && !(env && strcmp(env, "fp32") == 0);
     {
         const char *e2 = getenv("DAISY_GATHER_EPI"); // "split": keep the separate epilogue kernel (A/B switch)
@@ -1297,7 +1303,7 @@ static int scan_and_plan(daisy_solver *s) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-static int padded_K(int K) { return K <= 1 ? 1 : K <= 3 ? 3 : K <= 9 ? 9 : K <= 16 ? 16 : 32; }
+static int padded_K(int K) { return K <= 1 ? 1 : K <= 3 ? 3 : K <= 9 ? 9 : K <= 16 ? 16 : K <= 32 ? 32 : 64; }
 
 static void free_solver(daisy_solver *s) {
     if (!s) return;
@@ -1352,7 +1358,13 @@ static int compute_sums_from_host(daisy_solver *s, const float *res /* K x N */)
 extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const float *M, int nmat, const int32_t *mat_idx,
                                    daisy_solver **out) {
     DZ_REQUIRE(ctx && out && E && M && mat_idx, DAISY_E_INVALID, "daisy_solver_create: null argument");
-    DZ_REQUIRE(K >= 1 && K <= DAISY_MAX_BANDS, DAISY_E_INVALID, "daisy_solver_create: K must be in [1,32]");
+    DZ_REQUIRE(K >= 1 && K <= DAISY_MAX_BANDS, DAISY_E_INVALID,
+               "daisy_solver_create: K must be in [1,64] (kernels for 1, 3, 9, 16, 32 and 64 bands, K padded up to the next)");
+    {
+        const char *env = getenv("DAISY_GATHER");
+        DZ_REQUIRE(K <= 32 || !(env && (strcmp(env, "fp32") == 0 || strcmp(env, "ldg") == 0)), DAISY_E_INVALID,
+                   "daisy_solver_create: K > 32 runs only on the tensor-core kernel; DAISY_GATHER=fp32 / ldg has no kernel for it");
+    }
     DZ_REQUIRE(nmat >= 1, DAISY_E_INVALID, "daisy_solver_create: need at least one material");
     DZ_REQUIRE(ctx->have_F, DAISY_E_STATE, "daisy_solver_create: build or load the form factors first");
     DZ_REQUIRE(ctx->N > 0, DAISY_E_INVALID, "daisy_solver_create: empty mesh");

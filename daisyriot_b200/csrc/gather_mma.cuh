@@ -1,4 +1,4 @@
-// gather_mma.cuh -- the gather pass for wide band counts (K = 16 / 32) on the 5th-generation tensor cores.
+// gather_mma.cuh -- the gather pass for wide band counts (K = 16 / 32 / 64) on the 5th-generation tensor cores.
 //
 // With K bands every F element feeds K FMAs; at K = 32 that is 16 flop per HBM byte, beyond what the FP32 pipe can
 // sustain at HBM speed (128 FMA/clk/SM against 5.8 F elements/clk/SM x 32).  The contraction
@@ -8,30 +8,33 @@
 // (3xTF32):  F = Fh + Fl,  R = Rh + Rl,  F*R ~= Fh*Rh + Fh*Rl + Fl*Rh, every term rounded to nearest (cvt.rna), so the
 // split error is unbiased and < 2^-21 relative.  The tensor core adds into its FP32 accumulator with truncation; over
 // thousands of k-steps that is a systematic bias (measured 4.5e-6 after 2048 columns), so the TMEM accumulator only
-// ever holds ONE 64-column stage (16 MMAs) and the stage sums are added up in FP32 round-to-nearest by the epilogue
+// ever holds ONE 64-column stage (16 MMAs, 24 at K = 64) and the stage sums are added up in FP32 round-to-nearest by the epilogue
 // warps (tcgen05.ld moves 64 B/clk, which is why the accumulator is not drained more often than that).
 //
 // Per CTA (one per SM, persistent over (128-row block) x (column range) items):
 //   warp 0      TMA producer: per stage two F sub-tiles 128 x 32 (SWIZZLE_128B) + two band sub-tiles [Rh;Rl] 2K x 32,
-//               4-stage ring
+//               4-stage ring (3 stages at K = 64)
 //   warps 4-11  converters (two sets alternating stages): LDS their row of the F tile, Fh = tf32(F) (round to nearest),
 //               Fl = F - Fh, tcgen05.st both into a TMEM operand ring -- the A operand is read from TMEM, so the F
 //               bytes cross shared memory exactly once on the way in and once to registers
 //   warp 1      MMA issuer (one elected lane): per 8-column k-step  D[:, 0:2K] += Fh x [Rh;Rl]^T  and  D[:, 0:K] += Fl x Rh^T,
+//               at K = 64 D[:, 0:K] += Fh x Rh^T, Fh x Rl^T and Fl x Rh^T (three MMAs of N = 64 into the same columns),
 //               one tcgen05.commit per stage on the mma_done ring (frees the smem slot and the operand slot, signals the
 //               epilogue); this thread is the kernel's critical path
-//   warps 12-15 epilogue: per stage tcgen05.ld the 2K accumulator columns, acc[k] += D[:, k] + D[:, K+k]; at the end
+//   warps 12-15 epilogue: per stage tcgen05.ld the 2K accumulator columns, acc[k] += D[:, k] + D[:, K+k] (K = 64: the K
+//               columns, acc[k] += D[:, k], in two 32-column chunks); at the end
 //               of the item the column-range partials go to global memory
 //   warp 2      TMEM allocation
-// TMEM: 4 accumulator buffers (2K columns each) + 2 operand stages (128 columns each) = 512 columns for K = 32.
+// TMEM: 4 accumulator buffers (2K columns each) + 2 operand stages (128 columns each) = 512 columns for K = 32; K = 64:
+// 3 accumulator buffers of 64 columns, the operand stages at columns 256-511 (MmaCfg).
 #pragma once
 
 #define MM_ROWS 128
 #define MM_SUB 32   // columns per SWIZZLE_128B sub-tile (128 bytes)
 #define MM_COLS 64  // columns per stage: two sub-tiles, i.e. 256 contiguous bytes of every F row per stage
-#define MM_NS 4     // shared-memory stages
+#define MM_NS 4     // shared-memory stages (K = 16 / 32)
 #define MM_NA 2     // TMEM operand stages (128 columns each: 64 of Fh, 64 of Fl)
-#define MM_ND 4     // TMEM accumulator buffers (one stage each)
+#define MM_ND 4     // TMEM accumulator buffers (one stage each; K = 16 / 32)
 #define MM_THREADS 512
 
 __device__ __forceinline__ bool elect_one() {
@@ -126,10 +129,21 @@ __global__ void k_split_residual(const float *__restrict__ res, int64_t bstride,
     }
 }
 
+// Ring depths and TMEM layout per band count.  K = 16 / 32: 4 shared-memory stages, 4 accumulator buffers of 2K columns
+// (Fh x Rh and Fh x Rl side by side, Fl x Rh added into the first K).  K = 64: a stage is 64 KB (32 KB of F + 32 KB of
+// [Rh;Rl]), so 3 stages fill the 227 KB; all three products go into the same K columns (24 MMAs of N = 64 per stage instead
+// of 16), which keeps the drain at 64 columns per stage (512 of the 1424-cycle HBM budget, as at K = 32) and lets 3
+// accumulator buffers of 64 columns sit below the operand ring at column 256.  ND <= NS and NA < NS: no mma_done slot can
+// complete a second phase before every role has observed the first (see k_gather_mma).
+template <int K> struct MmaCfg {
+    static constexpr int NS = MM_NS, ND = MM_ND, DCOLS = 2 * K, A_COL0 = MM_ND * 2 * K;
+};
+template <> struct MmaCfg<64> { static constexpr int NS = 3, ND = 3, DCOLS = 64, A_COL0 = 256; };
+
 template <int K>
 __host__ __device__ constexpr int mm_stage_bytes() { return 2 * (MM_ROWS * MM_SUB * 4 + 2 * K * MM_SUB * 4); }
 template <int K>
-__host__ __device__ constexpr int mm_smem_bytes() { return MM_NS * mm_stage_bytes<K>() + 1024 + 512; }
+__host__ __device__ constexpr int mm_smem_bytes() { return MmaCfg<K>::NS * mm_stage_bytes<K>() + 1024 + 512; }
 
 template <int K>
 __global__ void __launch_bounds__(MM_THREADS, 1)
@@ -138,25 +152,36 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
     constexpr int F_SUB = MM_ROWS * MM_SUB * 4;  // one F sub-tile
     constexpr int B_SUB = 2 * K * MM_SUB * 4;    // one band sub-tile
     constexpr int B_OFF = 2 * F_SUB;             // band sub-tiles follow the two F sub-tiles
-    constexpr int DCOLS = 2 * K;                 // accumulator columns per buffer
-    constexpr int A_COL0 = MM_ND * DCOLS;        // operand ring starts after the accumulator buffers
+    constexpr int NS = MmaCfg<K>::NS, ND = MmaCfg<K>::ND;
+    constexpr int DCOLS = MmaCfg<K>::DCOLS;      // accumulator columns per buffer
+    constexpr int A_COL0 = MmaCfg<K>::A_COL0;    // operand ring starts after the accumulator buffers
     constexpr int A_COLS = 2 * MM_COLS;          // Fh columns then Fl columns
     constexpr uint32_t IDESC_2K = tc_idesc_tf32(MM_ROWS, 2 * K), IDESC_K = tc_idesc_tf32(MM_ROWS, K);
-    static_assert(A_COL0 + MM_NA * A_COLS <= 512, "TMEM budget");
+    static_assert(ND * DCOLS <= A_COL0 && A_COL0 + MM_NA * A_COLS <= 512, "TMEM budget");
+    static_assert(NS * STAGE + 1024 + 512 <= 227 * 1024, "shared-memory budget");
     extern __shared__ unsigned char mm_smem_raw[];
     const uint32_t raw = smem_u32(mm_smem_raw);
     unsigned char *base = mm_smem_raw + (((raw + 1023u) & ~1023u) - raw); // SWIZZLE_128B tiles need 1024-byte alignment
-    uint64_t *bars = reinterpret_cast<uint64_t *>(base + (size_t)MM_NS * STAGE);
-    uint64_t *full = bars, *empty = bars + MM_NS, *a_full = bars + 2 * MM_NS;
-    uint64_t *mma_done = a_full + MM_NA, *d_empty = mma_done + MM_NS;
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(d_empty + MM_ND);
-    static_assert(MM_NS == 4 && MM_NA == 2 && MM_ND == 4, "mma_done ring indexing below assumes these depths");
+    uint64_t *bars = reinterpret_cast<uint64_t *>(base + (size_t)NS * STAGE);
+    // full barriers: the two converter sets take alternate stages, so with an odd ring depth a slot's consecutive stages
+    // belong to different sets, and the set of stage it + NS could wait for the slot's next phase before the current one has
+    // completed -- which a parity wait cannot tell from a completed phase.  NF = 2 NS barriers then give every barrier to one set.
+    constexpr int NF = (NS % 2 == 0) ? NS : 2 * NS;
+    uint64_t *full = bars, *empty = bars + NF, *a_full = bars + NF + NS;
+    static_assert((NF + 2 * NS + MM_NA + ND) * 8 + 4 <= 512, "barrier space");
+    uint64_t *mma_done = a_full + MM_NA, *d_empty = mma_done + NS;
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(d_empty + ND);
+    // mma_done[it % NS] completes once per stage, and every waiter must see a phase before the slot completes again: the
+    // epilogue releases stage it before the MMAs of stage it + NS may start (ND <= NS), and the converters wait on stage
+    // it - NA before they hand over stage it, which the MMAs of every later stage follow (NA < NS)
+    static_assert(MM_NA == 2 && ND <= NS && MM_NA < NS, "mma_done ring indexing below assumes these depths");
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (P.stop.state && stop_stopped(P.stop)) return; // device converge: before any TMEM is allocated
     if (tid == 0) {
-        for (int i = 0; i < MM_NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 4); mbar_init(&mma_done[i], 1); }  // empty: 4 converter warps
+        for (int i = 0; i < NS; i++) { mbar_init(&full[i], 1); mbar_init(&empty[i], 4); mbar_init(&mma_done[i], 1); }  // empty: 4 converter warps
+        for (int i = NS; i < NF; i++) mbar_init(&full[i], 1);
         for (int i = 0; i < MM_NA; i++) mbar_init(&a_full[i], 4);
-        for (int i = 0; i < MM_ND; i++) mbar_init(&d_empty[i], 4);
+        for (int i = 0; i < ND; i++) mbar_init(&d_empty[i], 4);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 2) {
@@ -180,17 +205,18 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
                 const int c_begin = split * P.colw, c_end = min(P.ncols, c_begin + P.colw);
                 const int nstep = (c_end - c_begin + MM_COLS - 1) / MM_COLS;
                 for (int s = 0; s < nstep; s++, it++) {
-                    const int st = it % MM_NS;
-                    mbar_wait(&empty[st], ((it / MM_NS) & 1) ^ 1);      // converters have read the F tiles of stage it-4
-                    mbar_wait(&mma_done[st], ((it / MM_NS) & 1) ^ 1);   // the MMAs of stage it-4 have read its band tiles
+                    const int st = it % NS;
+                    mbar_wait(&empty[st], ((it / NS) & 1) ^ 1);      // converters have read the F tiles of stage it-NS
+                    mbar_wait(&mma_done[st], ((it / NS) & 1) ^ 1);   // the MMAs of stage it-NS have read its band tiles
                     unsigned char *sf = base + (size_t)st * STAGE;
                     const int c0 = c_begin + s * MM_COLS;
-                    mbar_expect_tx(&full[st], (uint32_t)STAGE);
+                    uint64_t *fb = &full[it % NF];
+                    mbar_expect_tx(fb, (uint32_t)STAGE);
                     // F streams through L2 evict_first: it is read once per pass and must not push the split residual out
-                    tma_load_2d_hint(sf, &tmF, c0, rb * MM_ROWS, &full[st], pol_first);
-                    tma_load_2d_hint(sf + F_SUB, &tmF, c0 + MM_SUB, rb * MM_ROWS, &full[st], pol_first);
-                    tma_load_2d(sf + B_OFF, &tmR, c0, 0, &full[st]);
-                    tma_load_2d(sf + B_OFF + B_SUB, &tmR, c0 + MM_SUB, 0, &full[st]);
+                    tma_load_2d_hint(sf, &tmF, c0, rb * MM_ROWS, fb, pol_first);
+                    tma_load_2d_hint(sf + F_SUB, &tmF, c0 + MM_SUB, rb * MM_ROWS, fb, pol_first);
+                    tma_load_2d(sf + B_OFF, &tmR, c0, 0, fb);
+                    tma_load_2d(sf + B_OFF + B_SUB, &tmR, c0 + MM_SUB, 0, fb);
                 }
             }
         }
@@ -198,7 +224,7 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
         // ------------------------------- MMA issuer ---------------------------------
         // The whole warp runs the loop (uniform control flow keeps descriptors in uniform registers); one elected lane
         // issues.  The issuing thread is the critical path of this kernel (per-MMA issue ~40 clk plus the barrier
-        // round trips), so it waits on two barriers per stage and signals one: a_full[a] implies full[st] (the
+        // round trips), so it waits on two barriers per stage and signals one: a_full[a] implies the stage's full barrier (the
         // converters waited on it), and a single commit per stage serves the producer (smem slot), the converters
         // (operand slot) and the epilogue (accumulator ready).
         const bool leader = elect_one();
@@ -207,9 +233,9 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
             const int c_begin = split * P.colw, c_end = min(P.ncols, c_begin + P.colw);
             const int nstep = (c_end - c_begin + MM_COLS - 1) / MM_COLS;
             for (int s = 0; s < nstep; s++, it++) {
-                const int st = it % MM_NS, a = it % MM_NA, b = it % MM_ND;
+                const int st = it % NS, a = it % MM_NA, b = it % ND;
                 mbar_wait(&a_full[a], (it / MM_NA) & 1);
-                mbar_wait(&d_empty[b], ((it / MM_ND) & 1) ^ 1);
+                mbar_wait(&d_empty[b], ((it / ND) & 1) ^ 1);
                 tc_fence_after();
                 const uint32_t b_addr = smem_u32(base + (size_t)st * STAGE + B_OFF);
                 const uint32_t a_tmem = tmem + A_COL0 + a * A_COLS;
@@ -218,10 +244,17 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
 #pragma unroll
                     for (int k = 0; k < MM_COLS / 8; k++) {
                         const uint64_t bdesc = tc_smem_desc_sw128(b_addr + (k >> 2) * B_SUB + (k & 3) * 32);
-                        tc_mma_tf32_ts(d_tmem, a_tmem + k * 8, bdesc, IDESC_2K, k > 0 ? 1u : 0u);        // Fh x [Rh;Rl]
+                        if constexpr (K == 64) {
+                            // Rl starts K rows = 8 KB into the band sub-tile: a whole number of 1024-byte swizzle atoms
+                            const uint64_t bdesc_l = tc_smem_desc_sw128(b_addr + (k >> 2) * B_SUB + K * 128 + (k & 3) * 32);
+                            tc_mma_tf32_ts(d_tmem, a_tmem + k * 8, bdesc, IDESC_K, k > 0 ? 1u : 0u);     // Fh x Rh
+                            tc_mma_tf32_ts(d_tmem, a_tmem + k * 8, bdesc_l, IDESC_K, 1u);                // Fh x Rl
+                        } else {
+                            tc_mma_tf32_ts(d_tmem, a_tmem + k * 8, bdesc, IDESC_2K, k > 0 ? 1u : 0u);    // Fh x [Rh;Rl]
+                        }
                         tc_mma_tf32_ts(d_tmem, a_tmem + MM_COLS + k * 8, bdesc, IDESC_K, 1u);          // Fl x Rh
                     }
-                    tc_commit(&mma_done[it % MM_NS]);
+                    tc_commit(&mma_done[it % NS]);
                 }
                 __syncwarp();
             }
@@ -237,8 +270,8 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
             const int nstep = (c_end - c_begin + MM_COLS - 1) / MM_COLS;
             for (int s = 0; s < nstep; s++, it++) {
                 if ((it & 1) != set) continue;
-                const int st = it % MM_NS, a = it % MM_NA;
-                mbar_wait(&full[st], (it / MM_NS) & 1);
+                const int st = it % NS, a = it % MM_NA;
+                mbar_wait(&full[it % NF], (it / NF) & 1);
                 const uint32_t a_tmem = tmem + lane_off + A_COL0 + a * A_COLS;
 #pragma unroll
                 for (int sub = 0; sub < 2; sub++) {
@@ -262,7 +295,7 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
                         if (lane == 0) mbar_arrive(&empty[st]);     // both F sub-tiles are in registers
                     }
                     if (sub == 0) {
-                        if (it >= MM_NA) mbar_wait(&mma_done[(it - MM_NA) % MM_NS], ((it - MM_NA) / MM_NS) & 1); // MMAs of stage it-2 are done with this operand slot
+                        if (it >= MM_NA) mbar_wait(&mma_done[(it - MM_NA) % NS], ((it - MM_NA) / NS) & 1); // MMAs of stage it-2 are done with this operand slot
                         tc_fence_after();
                     }
                     tc_st32(a_tmem + sub * MM_SUB, hi);
@@ -286,10 +319,23 @@ k_gather_mma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
 #pragma unroll
             for (int k = 0; k < K; k++) out[k] = 0.0f;
             for (int s = 0; s < nstep; s++, it++) {
-                const int b = it % MM_ND;
-                mbar_wait(&mma_done[it % MM_NS], (it / MM_NS) & 1);
+                const int b = it % ND;
+                mbar_wait(&mma_done[it % NS], (it / NS) & 1);
                 tc_fence_after();
-                if constexpr (K == 32) {
+                if constexpr (K == 64) {
+                    // one 32-column chunk in registers at a time: out[64] and 64 loaded columns would not fit 128 registers
+                    uint32_t r[32];
+#pragma unroll
+                    for (int h = 0; h < 2; h++) {
+                        tc_ld32(tmem + lane_off + b * DCOLS + h * 32, r);
+                        tc_wait_ld();
+#pragma unroll
+                        for (int k = 0; k < 32; k++) out[h * 32 + k] += __uint_as_float(r[k]);
+                    }
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(&d_empty[b]);
+                } else if constexpr (K == 32) {
                     uint32_t r0[32], r1[32];
                     tc_ld32(tmem + lane_off + b * DCOLS, r0);
                     tc_ld32(tmem + lane_off + b * DCOLS + 32, r1);

@@ -31,7 +31,7 @@ def block_layout(K_padded: int, n: int):
 
 
 def padded_K(K: int) -> int:
-    return 1 if K <= 1 else 3 if K <= 3 else 9 if K <= 9 else 16 if K <= 16 else 32
+    return 1 if K <= 1 else 3 if K <= 3 else 9 if K <= 9 else 16 if K <= 16 else 32 if K <= 32 else 64
 
 
 def exchange_pass(step_local, next_buffer, rank: int, nranks: int, group=None):

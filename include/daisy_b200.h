@@ -29,7 +29,9 @@ extern "C" {
 #define DAISY_E_NOMEM (-4)
 
 #define DAISY_MAX_SAMPLES 64 /* visibility masks are 64-bit; the reference uses RAYS_PER_PATCH = 50 */
-#define DAISY_MAX_BANDS 32
+/* bands of a solver: kernels exist for 1, 3, 9, 16, 32 and 64 bands and K runs padded up to the next of these (inert zero
+ * bands); K > 32 runs only on the tensor-core kernel (DAISY_GATHER=fp32 / ldg: daisy_solver_create returns DAISY_E_INVALID) */
+#define DAISY_MAX_BANDS 64
 
 typedef struct daisy_ctx daisy_ctx;       /* ~ OptixPrimeFunctionality (+ the RadMat it fills) */
 typedef struct daisy_solver daisy_solver; /* ~ Lightning / SpectralLightning / RGBLightning / BWLightning */
@@ -183,7 +185,7 @@ int64_t daisy_formfactors_pairs_fallback(daisy_ctx *ctx);
  *   K=3, M=diag(rho_rgb)  : RGBLightning      (:298-384)
  *   K=#wavelengths, full M: SpectralLightning (:99-295, hot loop :196-226)
  * E: K x N band-major emission (already scaled by emission_value, as set_sampled_emission does, :263-273).
- * M: nmat x K x K column-major; mat_idx: N material ids (MeshS::materialIndexPerTriangle). */
+ * M: nmat x K x K column-major; mat_idx: N material ids (MeshS::materialIndexPerTriangle).  1 <= K <= DAISY_MAX_BANDS. */
 int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const float *M, int nmat, const int32_t *mat_idx,
                         daisy_solver **out);
 void daisy_solver_destroy(daisy_solver *s);
@@ -225,7 +227,8 @@ int daisy_solver_last_step_ms(daisy_solver *s, double *ms);
  * next pass's grid moves onto SMs as the previous pass leaves them and streams its first F tiles meanwhile.  Results are
  * unchanged (the kernel waits for the previous pass before it reads or writes anything a pass writes). */
 int daisy_solver_set_chained(daisy_solver *s, int on);
-/* kernels one pass launches in this solver's configuration: 1 for K <= 9 (streaming, epilogue and exchange wait in one kernel) */
+/* kernels one pass launches in this solver's configuration: 1 for K <= 9 (streaming, epilogue and exchange wait in one kernel),
+ * 3 on the tensor-core path (K = 10-64: residual split, streaming kernel, epilogue), plus 1 with the fused exchange */
 int daisy_solver_launches_per_pass(daisy_solver *s);
 /* Tile skipping (K <= 9; DAISY_GATHER_SKIP=0 streams the whole matrix instead): a pass streams only the 64-row x 256-column tiles
  * of F that hold an entry other than +-0.  The solver scans F for them at daisy_solver_create and again before the first pass

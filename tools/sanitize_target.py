@@ -1,5 +1,5 @@
 """Small-N runs of the three hot kernels for compute-sanitizer (tools/sanitize.sh): k_ff_tiles (form factors + masks),
-k_gather_tma<9> (fused epilogue, several column splits) and k_gather_mma<32> (tcgen05).  Results are checked against the
+k_gather_tma<9> (fused epilogue, several column splits), k_gather_mma<32> and k_gather_mma<64> (tcgen05).  Results are checked against the
 oracle so that a sanitizer run is also a parity run."""
 import ctypes as C
 import sys
@@ -24,7 +24,7 @@ if what == "ff":
     print("ff ok", p.stats())
     p.close()
 else:
-    K = 9 if what == "gather9" else 32
+    K = {"gather9": 9, "gather32": 32, "gather64": 64}[what]
     N = 4096 if K == 9 else 1024
     sc = scenes.cornell_box(N)
     p = dz.OptixPrimeFunctionality(dz.MeshS.from_scene(sc), rands=uv)
