@@ -1,5 +1,6 @@
-"""Scene builders shared by the geometry tests: the adversarial walls of test_gpu_parity.py, and translated / scaled copies of
-any scene for the far-from-origin tests (test_far_geometry_oracle.py, test_gpu_far_geometry.py)."""
+"""Scene builders shared by the geometry tests: the adversarial walls of test_gpu_parity.py, translated / scaled copies of
+any scene for the far-from-origin tests (test_far_geometry_oracle.py, test_gpu_far_geometry.py), and the scenes that push
+the form-factor kernel past its fixed capacities (test_ff_limits_scenes.py, test_gpu_ff_limits.py)."""
 import numpy as np
 
 from daisyriot_b200 import scenes
@@ -201,3 +202,193 @@ def closest_hit_rays(sc, seed, n_random=3000, n_axis=4000):
     p = a + u[:, None] * (b - a) + v[:, None] * (c - a)
     out.append(np.concatenate([p.astype(np.float32), unit(rng.normal(size=(len(tri), 3)))], 1))
     return np.ascontiguousarray(np.concatenate(out), np.float32)
+
+
+# ---- capacity limits of the form-factor kernel ----------------------------------------------------------------------------
+# formfactor.cu has three fixed capacities, and a scene past any of them takes another code path:
+# * SHAFT_CAP = 256 candidates per pair: a longer shaft list flags the pair heavy, and phase 2b traces its rays one LBVH walk each;
+# * DAISY_MAX_FACES = 64 face grids: further planes of 32 or more triangles stay ordinary candidates, with plane ids above nfaces;
+# * NBR_CAP = 32 ints of neighbour list (31 neighbours): a patch with more coplanar neighbours loses coplanar skipping.
+# The builders below put small scenes on both sides of each limit.  Their premises are checked in test_ff_limits_scenes.py.
+
+class _Builder:
+    """Triangles with one normal each (the normal array holds one entry per triangle)."""
+
+    def __init__(self):
+        self.V, self.VN, self.T = [], [], []
+
+    def tri(self, a, b, c, n):
+        base, ni = len(self.V), len(self.VN)
+        self.V += [np.asarray(a, np.float64), np.asarray(b, np.float64), np.asarray(c, np.float64)]
+        self.VN.append(np.asarray(n, np.float64) / np.linalg.norm(n))
+        self.T.append([base, base + 1, base + 2, ni, ni, ni])
+
+    def grid(self, origin, eu, ev, n, nu, nv):
+        """nu x nv quads of two triangles each; shared edges are bit-identical (one vertex array per grid)."""
+        base, ni = len(self.V), len(self.VN)
+        origin, eu, ev = (np.asarray(x, np.float64) for x in (origin, eu, ev))
+        for j in range(nv + 1):
+            for i in range(nu + 1):
+                self.V.append(origin + (i / nu) * eu + (j / nv) * ev)
+        self.VN.append(np.asarray(n, np.float64) / np.linalg.norm(n))
+        for j in range(nv):
+            for i in range(nu):
+                a, b = base + j * (nu + 1) + i, base + j * (nu + 1) + i + 1
+                c, d = a + nu + 1, b + nu + 1
+                self.T += [[a, b, d, ni, ni, ni], [a, d, c, ni, ni, ni]]
+
+    def scene(self, name):
+        V = np.asarray(self.V, np.float64).astype(np.float32)
+        VN = np.asarray(self.VN, np.float64).astype(np.float32)
+        T = np.asarray(self.T, np.int32).reshape(-1, 6)
+        return Scene(V, VN, T, np.zeros(len(T), np.int32), _one_material(), name)
+
+
+def _random_triangles(b, rng, centres, radius, tilt=(0.3, 2.8)):
+    """One equilateral triangle of circumradius `radius` around each centre, each in its own random orientation: the xy-plane
+    turned about a random axis by an angle drawn from `tilt` (radians)."""
+    ang = np.array([0.0, 2 * np.pi / 3, 4 * np.pi / 3])
+    flat = radius * np.stack([np.cos(ang), np.sin(ang), np.zeros(3)], 1)
+    for c in centres:
+        R = _rot(rng.normal(size=3), rng.uniform(*tilt))
+        p = flat @ R.T + c
+        b.tri(p[0], p[1], p[2], np.cross(p[1] - p[0], p[2] - p[0]))
+
+
+def lifted(sc, k, dz=1.5):
+    """The vertex array of sc with triangle k's three vertices raised by dz along z (the builders give every occluder
+    vertices of its own)."""
+    V = sc.vertices.copy()
+    V[sc.tri[k, :3], 2] += np.float32(dz)
+    return V
+
+
+def edge_pattern(uv):
+    """The pattern with its first eight samples moved onto triangle edges and vertices (u = 0, v = 0, u + v = 1)."""
+    uv = np.array(uv, np.float32)
+    uv[:8] = np.array([[0, 0], [1, 0], [0, 1], [0.5, 0], [0, 0.5], [0.5, 0.5], [0.25, 0.75], [1e-4, 0.3]], np.float32)
+    return uv
+
+
+def random_pattern(S, seed):
+    rng = np.random.RandomState(seed)
+    u = rng.uniform(0, 1, S)
+    v = rng.uniform(0, 1, S) * (1 - u)
+    return np.stack([u, v], 1).astype(np.float32)
+
+
+def shaft_cap_scene(n_occ, seed=0):
+    """Two single-triangle plates one unit apart, facing each other -- A (triangle 0) at z = 0 with normal +z, B (triangle 1) the
+    same triangle at z = 1 with normal -z -- and n_occ small triangles between them (triangles 2 ...), each in its own random
+    orientation (tilted 0.1-0.8 rad): centres with x, y in [1, 8], x + y < 8.5, z in [0.4, 0.6], vertices 0.35 from the centre.  Every occluder's
+    box lies inside the hull of A and B by at least 0.05, far above the 1e-3 box padding, so the pair (A, B) has exactly n_occ
+    shaft candidates; any other pair has fewer."""
+    rng = np.random.RandomState(1000 + seed)
+    b = _Builder()
+    b.tri((0, 0, 0), (10, 0, 0), (0, 10, 0), (0, 0, 1))
+    b.tri((0, 0, 1), (10, 0, 1), (0, 10, 1), (0, 0, -1))
+    centres = []
+    while len(centres) < n_occ:
+        x, y = rng.uniform(1.0, 8.0, 2)
+        if x + y < 8.5:
+            centres.append((x, y, rng.uniform(0.4, 0.6)))
+    _random_triangles(b, rng, centres, 0.35, tilt=(0.1, 0.8))  # nearly face-on: they hide part of A from B
+    return b.scene(f"shaft_cap{n_occ}")
+
+
+def occluded_walls(nu, nv, seed=0, n_occ=360):
+    """Two facing 10 x 10 walls, z = 0 (normal +z) and z = 1 (normal -z), each cut into nu x nv quads, and n_occ small occluders
+    (circumradius 0.12) clustered in x, y in [4.3, 5.7], z in [0.3, 0.7].  Hundreds of wall-to-wall pairs see more than 256
+    occluders in their shafts; the walls' own triangles are coplanar neighbours of every wall patch."""
+    rng = np.random.RandomState(2000 + seed)
+    b = _Builder()
+    b.grid((0, 0, 0), (10, 0, 0), (0, 10, 0), (0, 0, 1), nu, nv)
+    b.grid((0, 0, 1), (0, 10, 0), (10, 0, 0), (0, 0, -1), nv, nu)
+    centres = np.stack([rng.uniform(4.3, 5.7, n_occ), rng.uniform(4.3, 5.7, n_occ), rng.uniform(0.3, 0.7, n_occ)], 1)
+    _random_triangles(b, rng, centres, 0.12)
+    return b.scene(f"occluded_walls{nu}x{nv}")
+
+
+MANY_PLANES_KINDS = ("floor", "ceiling", "vertical")
+
+
+def many_planes(nplates, seed=0):
+    """nplates plates of 4 x 4 quads (32 triangles each), every plate in its own axis-aligned plane, in this order: plate q is
+    MANY_PLANES_KINDS[(q + 1) % 3] -- a floor plate at y = 1e-3 q, a ceiling plate at y = 4 - 1e-3 q (both 1 x 1, on a 5 x 5
+    layout of x, z cells), or a vertical plate in the plane x = 0.3 + 0.2 j (y in [1.5, 2.5], z over one cell) that blocks
+    rays between floor and ceiling.  Then 40 small tilted occluders between them.  All plates have the same size, so the
+    face grids go to the first 64 plates in order (face f = plate f), and vertical plates sit among faces 32-63 and among the
+    planes left without a grid."""
+    rng = np.random.RandomState(3000 + seed)
+    b = _Builder()
+    seen = {k: 0 for k in MANY_PLANES_KINDS}
+    for q in range(nplates):
+        kind = MANY_PLANES_KINDS[(q + 1) % 3]
+        j = seen[kind]
+        seen[kind] += 1
+        cx, cz = float(j % 5), float((j // 5) % 5)
+        if kind == "floor":
+            b.grid((cx, 1e-3 * q, cz), (0, 0, 1), (1, 0, 0), (0, 1, 0), 4, 4)
+        elif kind == "ceiling":
+            b.grid((cx, 4 - 1e-3 * q, cz), (1, 0, 0), (0, 0, 1), (0, -1, 0), 4, 4)
+        else:
+            x = 0.3 + 0.2 * j
+            b.grid((x, 1.5, float((3 * j) % 5)), (0, 1, 0), (0, 0, 1), (1 if j % 2 else -1, 0, 0), 4, 4)
+    centres = np.stack([rng.uniform(0.2, 4.8, 40), rng.uniform(0.8, 3.2, 40), rng.uniform(0.2, 4.8, 40)], 1)
+    _random_triangles(b, rng, centres, 0.3)
+    return b.scene(f"many_planes{nplates}")
+
+
+def fan_floor(n):
+    """A plate (triangles 0 and 1: a 2 x 2 square at y = 1.5, normal -y), a tilted occluder (triangle 2) and a floor at y = 0 made
+    of ONE fan of n triangles around a centre vertex (triangles 3 ...): a closed disk of radius 2, apex angle 360 / n degrees
+    (11.25 for n = 32, 9 for n = 40: all pass the sliver rule 8 h >= longest edge).  Every fan triangle contains the centre, so
+    each has n - 1 coplanar neighbours: n = 32 fills the neighbour list exactly, n = 33 is one past it."""
+    b = _Builder()
+    b.tri((-1, 1.5, -1), (1, 1.5, -1), (1, 1.5, 1), (0, -1, 0))
+    b.tri((-1, 1.5, -1), (1, 1.5, 1), (-1, 1.5, 1), (0, -1, 0))
+    p = np.array([[-0.4, 0.7, -0.3], [0.6, 0.8, 0.1], [-0.1, 0.9, 0.7]])
+    b.tri(p[0], p[1], p[2], np.cross(p[1] - p[0], p[2] - p[0]))
+    base = len(b.V)
+    b.V.append(np.zeros(3))
+    for i in range(n):
+        a = 2 * np.pi * i / n
+        b.V.append(np.array([2 * np.cos(a), 0.0, 2 * np.sin(a)]))
+    b.VN.append(np.array([0.0, 1.0, 0.0]))
+    ni = len(b.VN) - 1
+    for i in range(n):
+        b.T.append([base, base + 1 + (i + 1) % n, base + 1 + i, ni, ni, ni])
+    return b.scene(f"fan{n}")
+
+
+def padded_boxes(sc, tris, pad):
+    """float64 boxes (len(tris), 6) = (lo xyz, hi xyz) of the listed triangles, grown by pad on every side."""
+    P = sc.vertices[sc.tri[np.asarray(tris), :3]].astype(np.float64)  # (M, 3 vertices, 3)
+    return np.concatenate([P.min(1) - pad, P.max(1) + pad], 1)
+
+
+def shaft_meets(sc, pairs, boxes):
+    """float64 statement of formfactor.cu's shaft_box: (len(pairs), len(boxes)) bool, True where the box may meet the hull of
+    the pair's two triangles (six separating axes: x, y, z and D x {x, y, z}, D = centroid difference x 3, the kernel's slack)."""
+    pairs = np.asarray(pairs).reshape(-1, 2)
+    P = sc.vertices[sc.tri[pairs.reshape(-1), :3]].astype(np.float64).reshape(len(pairs), 6, 3)
+    lo, hi = P.min(1)[:, None, :], P.max(1)[:, None, :]
+    D = (P[:, 3:].sum(1) - P[:, :3].sum(1))[:, None, :]
+    blo, bhi = boxes[None, :, :3], boxes[None, :, 3:]
+    ok = ~((blo > hi) | (bhi < lo)).any(2)
+    c, h = 0.5 * (blo + bhi), 0.5 * (bhi - blo)
+    aD = np.abs(D)
+    for a, b in ((1, 2), (2, 0), (0, 1)):  # axis D x e: projection p = c_a D_b - c_b D_a, as q0 / q1 / q2 of make_shaft
+        q = P[:, :, a] * D[:, :, b] - P[:, :, b] * D[:, :, a]
+        p = c[..., a] * D[..., b] - c[..., b] * D[..., a]
+        r = h[..., a] * aD[..., b] + h[..., b] * aD[..., a]
+        r = r + 1e-5 * (np.abs(p) + r)
+        ok &= ~((p - r > q.max(1)[:, None]) | (p + r < q.min(1)[:, None]))
+    return ok
+
+
+def facing_pairs(orc):
+    """(lo, hi) pairs the kernel traces: the unoccluded factor from the lower to the higher triangle id is > 0."""
+    U = orc.unoccluded_rows(0, orc.N)
+    lo, hi = np.nonzero(np.triu(U > 0, 1))
+    return np.stack([lo, hi], 1)

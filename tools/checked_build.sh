@@ -13,3 +13,4 @@ timeout 1800 python -m pytest tests/test_gpu_converge_device.py -x -q -m gpu -k 
 timeout 1800 python -m pytest tests/test_gpu_geometry_update.py -x -q -m gpu -k "not group" 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_matrix_cache.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_wide_bands.py -x -q -m gpu 2>&1 | tail -4
+timeout 1800 python -m pytest tests/test_gpu_ff_limits.py -x -q -m gpu 2>&1 | tail -4
