@@ -65,6 +65,7 @@ SYMBOLS = {
     "daisy_formfactors_pairs_fallback": (C.c_int64, [_vp]),
     "daisy_ctx_update_geometry": (_i, [_vp, _fp, _i, _fp, _i]),
     "daisy_formfactors_update": (_i, [_vp, _i]),
+    "daisy_ctx_replace_mesh": (_i, [_vp, _fp, _i, _fp, _i, _ip, _i, _ip]),
     "daisy_formfactors_update_stats": (_i, [_vp, _i64p, _i64p, _i64p, _dp]),
     "daisy_solver_create": (_i, [_vp, _i, _fp, _fp, _i, _ip, C.POINTER(_vp)]),
     "daisy_solver_destroy": (None, [_vp]),
@@ -95,6 +96,7 @@ SYMBOLS = {
     "daisy_group_formfactors_stats": (_i, [_vp, _i64p, _i64p, _dp, _dp]),
     "daisy_group_update_geometry": (_i, [_vp, _fp, _i, _fp, _i]),
     "daisy_group_formfactors_update": (_i, [_vp, _i]),
+    "daisy_group_replace_mesh": (_i, [_vp, _fp, _i, _fp, _i, _ip, _i, _ip]),
     "daisy_group_solver_create": (_i, [_vp, _i, _fp, _fp, _i, _ip, C.POINTER(_vp)]),
     "daisy_group_solver_destroy": (None, [_vp]),
     "daisy_group_solver_reset": (_i, [_vp]),

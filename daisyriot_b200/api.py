@@ -187,6 +187,16 @@ class OptixPrimeFunctionality:
         _lib.check(_lib.lib().daisy_ctx_update_geometry(self._ctx, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0]), "ctx_update_geometry")
         self.mesh.vertices, self.mesh.normals = v, n
 
+    def replaceMesh(self, mesh: MeshS, previous) -> None:
+        """Replace the mesh (objects removed or added, vertices renumbered): ``previous[t]`` = index in the current mesh of the
+        triangle new triangle t continues, or -1 for a new one.  Queries answer for the new mesh at once; the matrix is remapped
+        at once (entries of new triangles +0.0) and traced where the edit reaches it at :meth:`updateRadiosityMatrix`.  Solvers
+        created before are stale: create new ones.  ``self.mesh`` and ``self.N`` follow."""
+        v, n, t, prev = _mesh_edit_arrays(mesh, previous)
+        _lib.check(_lib.lib().daisy_ctx_replace_mesh(self._ctx, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0], _lib.iptr(t), t.shape[0],
+                                                     _lib.iptr(prev)), "ctx_replace_mesh")
+        self.mesh, self.N = mesh, t.shape[0]
+
     def updateRadiosityMatrix(self, variant=_lib.FF_DEVICE) -> RadMat:
         """Bring the matrix to the current geometry, bit-identical to a fresh build, re-tracing only the pairs a change can
         reach (everything when the matrix was loaded, built with another variant or other samples, or not built yet)."""
@@ -368,6 +378,13 @@ class DeviceGroup:
         _lib.check(_lib.lib().daisy_group_update_geometry(self._g, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0]), "group_update_geometry")
         self.mesh.vertices, self.mesh.normals = v, n
 
+    def replace_mesh(self, mesh: MeshS, previous) -> None:
+        """:meth:`OptixPrimeFunctionality.replaceMesh` on every device (the row blocks follow the new N)."""
+        v, n, t, prev = _mesh_edit_arrays(mesh, previous)
+        _lib.check(_lib.lib().daisy_group_replace_mesh(self._g, _lib.fptr(v), v.shape[0], _lib.fptr(n), n.shape[0], _lib.iptr(t), t.shape[0],
+                                                       _lib.iptr(prev)), "group_replace_mesh")
+        self.mesh, self.N = mesh, t.shape[0]
+
     def updateRadiosityMatrix(self, variant=_lib.FF_DEVICE):
         _lib.check(_lib.lib().daisy_group_formfactors_update(self._g, variant), "group_formfactors_update")
         return self
@@ -478,6 +495,22 @@ def _geometry_arrays(mesh: MeshS, vertices, normals):
     if v.shape != np.shape(mesh.vertices) or n.shape != np.shape(mesh.normals):
         raise ValueError("updateGeometry: the vertex and normal counts stay those of the mesh")
     return v, n
+
+
+def _mesh_edit_arrays(mesh: MeshS, previous):
+    """The arrays of a mesh replacement: contiguous float32 / int32 copies, ``previous`` checked for its length (one entry per
+    new triangle) and for holding integers (the values themselves the library checks)."""
+    v = np.ascontiguousarray(mesh.vertices, np.float32).reshape(-1, 3)
+    n = np.ascontiguousarray(mesh.normals, np.float32).reshape(-1, 3)
+    t = np.ascontiguousarray(mesh.triangleIndices, np.int32).reshape(-1, 6)
+    p = np.asarray(previous)
+    if p.ndim != 1 or p.shape[0] != t.shape[0]:
+        raise ValueError("replaceMesh: previous needs one entry per triangle of the new mesh")
+    if p.size and not np.issubdtype(p.dtype, np.integer):
+        raise ValueError("replaceMesh: previous holds triangle indices (integers)")
+    if p.size and (p.min() < np.iinfo(np.int32).min or p.max() > np.iinfo(np.int32).max):
+        raise ValueError("replaceMesh: previous does not fit int32")
+    return v, n, t, np.ascontiguousarray(p, np.int32)
 
 
 def row_digest_host(F_rows: np.ndarray):

@@ -7,6 +7,8 @@
 #include <string.h>
 #include <math.h>
 #include <algorithm>
+#include <string>
+#include <thread>
 #include <unordered_map>
 #include <vector>
 
@@ -273,57 +275,66 @@ extern "C" int daisy_face_grid_dump(const float *vertices, int nv, const int32_t
     return dz_face_grid_dump(ext, vertices, tri_idx, ntri, pid, face, frame16, state, count, capacity);
 }
 
-static void set_partition(daisy_ctx *c, int rank, int nranks) {
-    c->rank = rank; c->nranks = nranks;
-    int n = (c->N + nranks - 1) / nranks;
+// the row layout of `nranks` blocks over N rows (daisy_ctx_set_partition documents it)
+struct RowLayout { int rows_per_rank, row0, row1; int64_t ldF; };
+static RowLayout row_layout(int N, int rank, int nranks) {
+    int n = (N + nranks - 1) / nranks;
     // single block: multiple of 4 (16-byte TMA alignment); several blocks: multiple of 256 so that a 256-column
     // TMA tile of the residual never straddles two ranks' blocks
     n = (nranks > 1) ? ((n + 255) / 256) * 256 : ((n + 3) / 4) * 4;
     if (n < 4) n = 4;
-    c->rows_per_rank = n;
-    c->row0 = (int)fmin((double)c->N, (double)rank * n);
-    c->row1 = (int)fmin((double)c->N, (double)(rank + 1) * n);
+    RowLayout l;
+    l.rows_per_rank = n;
+    l.row0 = (int)fmin((double)N, (double)rank * n);
+    l.row1 = (int)fmin((double)N, (double)(rank + 1) * n);
     int64_t ncols = (int64_t)nranks * n;
-    if (ncols < c->N) ncols = c->N;
-    c->ldF = ((ncols + 31) / 32) * 32;
+    if (ncols < N) ncols = N;
+    l.ldF = ((ncols + 31) / 32) * 32;
+    return l;
+}
+
+static void set_partition(daisy_ctx *c, int rank, int nranks) {
+    c->rank = rank; c->nranks = nranks;
+    const RowLayout l = row_layout(c->N, rank, nranks);
+    c->rows_per_rank = l.rows_per_rank; c->row0 = l.row0; c->row1 = l.row1; c->ldF = l.ldF;
 }
 
 static int build_geometry(daisy_ctx *c);
 
-extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
-                                int device, daisy_ctx **out) {
-    DZ_REQUIRE(out, DAISY_E_INVALID, "daisy_ctx_create: null out pointer");
-    *out = nullptr;
-    DzRange range_("daisy_ctx_create: mesh upload, plane ids, LBVH, patch records");
-    DZ_REQUIRE(nv >= 0 && nn >= 0 && ntri >= 0, DAISY_E_INVALID, "daisy_ctx_create: negative count");
-    DZ_REQUIRE(ntri == 0 || (vertices && normals && tri_idx), DAISY_E_INVALID, "daisy_ctx_create: null array");
+// the checks daisy_ctx_create and daisy_ctx_replace_mesh make on a mesh (host only, nothing changed on failure)
+static int check_mesh(const char *what, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri) {
+    if (!(nv >= 0 && nn >= 0 && ntri >= 0)) { daisy_set_error("%s: negative count", what); return DAISY_E_INVALID; }
+    if (!(ntri == 0 || (vertices && normals && tri_idx))) { daisy_set_error("%s: null array", what); return DAISY_E_INVALID; }
     for (int i = 0; i < ntri; i++)
         for (int k = 0; k < 6; k++) {
-            int v = tri_idx[6 * (size_t)i + k];
-            DZ_REQUIRE(v >= 0 && v < (k < 3 ? nv : nn), DAISY_E_INVALID, "daisy_ctx_create: triangle index out of range");
+            const int v = tri_idx[6 * (size_t)i + k];
+            if (!(v >= 0 && v < (k < 3 ? nv : nn))) { daisy_set_error("%s: triangle index out of range", what); return DAISY_E_INVALID; }
         }
-    int ndev = 0;
-    DZ_CUDA(cudaGetDeviceCount(&ndev));
-    DZ_REQUIRE(device >= 0 && device < ndev, DAISY_E_INVALID, "daisy_ctx_create: no such CUDA device");
-    DZ_CUDA(cudaSetDevice(device));
-    daisy_ctx *c = new daisy_ctx();
-    c->device = device; c->N = ntri; c->nv = nv; c->nn = nn;
-    cudaDeviceProp prop;
-    DZ_CUDA(cudaGetDeviceProperties(&prop, device));
-    c->num_sms = prop.multiProcessorCount;
-    set_partition(c, 0, 1);
-    // (with no triangles the arrays may be null; nothing reads them then)
-    if (vertices) c->h_vertices.assign(vertices, vertices + 3 * (size_t)nv); else c->h_vertices.assign(3 * (size_t)nv, 0.f);
-    if (normals) c->h_normals.assign(normals, normals + 3 * (size_t)nn); else c->h_normals.assign(3 * (size_t)nn, 0.f);
-    if (ntri) c->h_tri.assign(tri_idx, tri_idx + 6 * (size_t)ntri);
-#define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_ctx(c); return DAISY_E_CUDA; } } while (0)
-    CC(cudaMalloc(&c->d_vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
-    CC(cudaMalloc(&c->d_normals, sizeof(float) * 3 * (size_t)(nn > 0 ? nn : 1)));
-    CC(cudaMalloc(&c->d_tri, sizeof(int) * 6 * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_geom, sizeof(PatchGeom) * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_plane, sizeof(float4) * (size_t)(ntri > 0 ? ntri : 1)));
-    CC(cudaMalloc(&c->d_nbr, sizeof(int) * 32 * (size_t)(ntri > 0 ? ntri : 1)));
-    if (ntri) CC(cudaMemcpy(c->d_tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
+    return DAISY_OK;
+}
+
+// The device arrays sized by the mesh's counts: vertices, normals, triangle list (uploaded), patch / plane records, neighbour
+// lists and MeshS::trianglesPerVertex as CSR (uploaded).  All or nothing: on failure nothing stays allocated.
+struct MeshArrays {
+    float *vertices = nullptr, *normals = nullptr;
+    int *tri = nullptr, *nbr = nullptr, *vadj_off = nullptr, *vadj = nullptr;
+    PatchGeom *geom = nullptr;
+    float4 *plane = nullptr;
+};
+static void free_mesh_arrays(MeshArrays &m) {
+    cudaFree(m.vertices); cudaFree(m.normals); cudaFree(m.tri); cudaFree(m.geom); cudaFree(m.plane); cudaFree(m.nbr); cudaFree(m.vadj_off); cudaFree(m.vadj);
+    m = MeshArrays();
+}
+static int alloc_mesh_arrays(const int32_t *tri_idx, int nv, int nn, int ntri, MeshArrays &m) {
+    m = MeshArrays();
+#define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_mesh_arrays(m); return DAISY_E_CUDA; } } while (0)
+    CC(cudaMalloc(&m.vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
+    CC(cudaMalloc(&m.normals, sizeof(float) * 3 * (size_t)(nn > 0 ? nn : 1)));
+    CC(cudaMalloc(&m.tri, sizeof(int) * 6 * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&m.geom, sizeof(PatchGeom) * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&m.plane, sizeof(float4) * (size_t)(ntri > 0 ? ntri : 1)));
+    CC(cudaMalloc(&m.nbr, sizeof(int) * 32 * (size_t)(ntri > 0 ? ntri : 1)));
+    if (ntri) CC(cudaMemcpy(m.tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
     {
         // MeshS::trianglesPerVertex (MeshS.cpp:107-109) as CSR, lists in ascending triangle order: Drawer::interpolate sums
         // the patch colours of a vertex in exactly that order
@@ -334,13 +345,53 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
         std::vector<int> fill(off.begin(), off.end() - 1);
         for (int i = 0; i < ntri; i++)
             for (int k = 0; k < 3; k++) adj[(size_t)fill[tri_idx[6 * (size_t)i + k]]++] = i;
-        CC(cudaMalloc(&c->d_vadj_off, sizeof(int) * off.size()));
-        CC(cudaMalloc(&c->d_vadj, sizeof(int) * adj.size()));
-        CC(cudaMemcpy(c->d_vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice));
-        CC(cudaMemcpy(c->d_vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice));
+        CC(cudaMalloc(&m.vadj_off, sizeof(int) * off.size()));
+        CC(cudaMalloc(&m.vadj, sizeof(int) * adj.size()));
+        CC(cudaMemcpy(m.vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice));
+        CC(cudaMemcpy(m.vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice));
     }
 #undef CC
-    const int rc = build_geometry(c);
+    return DAISY_OK;
+}
+
+// the context takes the mesh (host copies and the arrays of alloc_mesh_arrays; its previous arrays are freed)
+static void install_mesh(daisy_ctx *c, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri, MeshArrays &m) {
+    MeshArrays old;
+    old.vertices = c->d_vertices; old.normals = c->d_normals; old.tri = c->d_tri; old.geom = c->d_geom; old.plane = c->d_plane; old.nbr = c->d_nbr;
+    old.vadj_off = c->d_vadj_off; old.vadj = c->d_vadj;
+    free_mesh_arrays(old);
+    c->d_vertices = m.vertices; c->d_normals = m.normals; c->d_tri = m.tri; c->d_geom = m.geom; c->d_plane = m.plane; c->d_nbr = m.nbr;
+    c->d_vadj_off = m.vadj_off; c->d_vadj = m.vadj;
+    m = MeshArrays();
+    c->N = ntri; c->nv = nv; c->nn = nn;
+    // (with no triangles the arrays may be null; nothing reads them then)
+    if (vertices) c->h_vertices.assign(vertices, vertices + 3 * (size_t)nv); else c->h_vertices.assign(3 * (size_t)nv, 0.f);
+    if (normals) c->h_normals.assign(normals, normals + 3 * (size_t)nn); else c->h_normals.assign(3 * (size_t)nn, 0.f);
+    if (ntri) c->h_tri.assign(tri_idx, tri_idx + 6 * (size_t)ntri); else c->h_tri.clear();
+}
+
+extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                                int device, daisy_ctx **out) {
+    DZ_REQUIRE(out, DAISY_E_INVALID, "daisy_ctx_create: null out pointer");
+    *out = nullptr;
+    DzRange range_("daisy_ctx_create: mesh upload, plane ids, LBVH, patch records");
+    int rc = check_mesh("daisy_ctx_create", vertices, nv, normals, nn, tri_idx, ntri);
+    if (rc) return rc;
+    int ndev = 0;
+    DZ_CUDA(cudaGetDeviceCount(&ndev));
+    DZ_REQUIRE(device >= 0 && device < ndev, DAISY_E_INVALID, "daisy_ctx_create: no such CUDA device");
+    DZ_CUDA(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    DZ_CUDA(cudaGetDeviceProperties(&prop, device));
+    MeshArrays m;
+    rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, m);
+    if (rc) return rc;
+    daisy_ctx *c = new daisy_ctx();
+    c->device = device;
+    c->num_sms = prop.multiProcessorCount;
+    install_mesh(c, vertices, nv, normals, nn, tri_idx, ntri, m);
+    set_partition(c, 0, 1);
+    rc = build_geometry(c);
     if (rc) { free_ctx(c); return rc; }
     *out = c;
     return DAISY_OK;
@@ -517,8 +568,16 @@ static void set_record(daisy_ctx *ctx, int variant) {
     ctx->rec.variant = variant;
     ctx->rec.S = ctx->S;
     memcpy(ctx->rec.uv, ctx->h_uv, sizeof(ctx->rec.uv));
-    ctx->rec.vertices = ctx->h_vertices;
-    ctx->rec.normals = ctx->h_normals;
+    const int N = ctx->N;
+    const int *tri = ctx->h_tri.data();
+    ctx->rec.tri.resize((size_t)18 * N);
+    for (int t = 0; t < N; t++)
+        for (int k = 0; k < 3; k++) {
+            memcpy(&ctx->rec.tri[18 * (size_t)t + 3 * k], &ctx->h_vertices[3 * (size_t)tri[6 * (size_t)t + k]], 12);
+            memcpy(&ctx->rec.tri[18 * (size_t)t + 9 + 3 * k], &ctx->h_normals[3 * (size_t)tri[6 * (size_t)t + 3 + k]], 12);
+        }
+    ctx->rec.has.assign((size_t)N, 1);
+    ctx->rec.ghost.clear();
     ctx->rec.pad = ctx->pad;
 }
 
@@ -545,9 +604,8 @@ extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     return DAISY_OK;
 }
 
-// padded box of triangle t as k_refit (bvh.cu) computes it: the same IEEE operations, so the same floats
-static void tri_box(const float *V, const int *tri, int t, float pad, float4 *out2) {
-    const float *a = V + 3 * (size_t)tri[6 * (size_t)t], *b = V + 3 * (size_t)tri[6 * (size_t)t + 1], *c = V + 3 * (size_t)tri[6 * (size_t)t + 2];
+// padded box of the triangle (a, b, c) as k_refit (bvh.cu) computes it: the same IEEE operations, so the same floats
+static void tri_box(const float *a, const float *b, const float *c, float pad, float4 *out2) {
     out2[0] = make_float4(fminf(a[0], fminf(b[0], c[0])) - pad, fminf(a[1], fminf(b[1], c[1])) - pad, fminf(a[2], fminf(b[2], c[2])) - pad, 0.f);
     out2[1] = make_float4(fmaxf(a[0], fmaxf(b[0], c[0])) + pad, fmaxf(a[1], fmaxf(b[1], c[1])) + pad, fmaxf(a[2], fmaxf(b[2], c[2])) + pad, 0.f);
 }
@@ -573,29 +631,34 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
         if (rc) return rc;
         ctx->upd_tris_changed = N;
     } else {
-        // changed: a position or a normal differs bitwise from the record; moved: a position does (only those can occlude
-        // differently)
-        const float *V0 = ctx->rec.vertices.data(), *V1 = ctx->h_vertices.data(), *N0 = ctx->rec.normals.data(), *N1 = ctx->h_normals.data();
+        // changed: no record (added since), or a position or a normal differs bitwise from the record; moved: a recorded
+        // position differs (only those, and added triangles, can occlude differently)
+        const float *R = ctx->rec.tri.data(), *V1 = ctx->h_vertices.data(), *N1 = ctx->h_normals.data();
+        const unsigned char *has = ctx->rec.has.data();
         const int *tri = ctx->h_tri.data();
         std::vector<unsigned char> changed((size_t)(N > 0 ? N : 1), 0);
-        std::vector<char> moved((size_t)(N > 0 ? N : 1), 0);
+        std::vector<char> moved((size_t)(N > 0 ? N : 1), 0); // 1: moved, 2: added
         int64_t nchanged = 0;
         for (int t = 0; t < N; t++) {
             bool pos = false, nrm = false;
-            for (int k = 0; k < 3; k++) pos |= memcmp(V0 + 3 * (size_t)tri[6 * (size_t)t + k], V1 + 3 * (size_t)tri[6 * (size_t)t + k], 12) != 0;
-            for (int k = 3; k < 6; k++) nrm |= memcmp(N0 + 3 * (size_t)tri[6 * (size_t)t + k], N1 + 3 * (size_t)tri[6 * (size_t)t + k], 12) != 0;
-            changed[(size_t)t] = pos || nrm;
-            moved[(size_t)t] = pos;
-            nchanged += pos || nrm;
+            if (has[t]) {
+                for (int k = 0; k < 3; k++) pos |= memcmp(R + 18 * (size_t)t + 3 * k, V1 + 3 * (size_t)tri[6 * (size_t)t + k], 12) != 0;
+                for (int k = 0; k < 3; k++) nrm |= memcmp(R + 18 * (size_t)t + 9 + 3 * k, N1 + 3 * (size_t)tri[6 * (size_t)t + 3 + k], 12) != 0;
+            }
+            changed[(size_t)t] = !has[t] || pos || nrm;
+            moved[(size_t)t] = !has[t] ? 2 : pos;
+            nchanged += changed[(size_t)t];
         }
         ctx->upd_tris_changed = nchanged;
-        if (nchanged == 0) { // F already is the matrix of this geometry
+        const std::vector<float4> &ghost = ctx->rec.ghost;
+        if (nchanged == 0 && ghost.empty()) { // F already is the matrix of this geometry
             ctx->upd_tiles = 0; ctx->pairs_traced = 0; ctx->pairs_owned = 0; ctx->pairs_heavy = 0; ctx->ff_ms = 0.0;
             ctx->upd_pairs = 0;
             return DAISY_OK;
         }
-        // dirty boxes: the moved triangles in Morton order (tile slots of the current hierarchy), clusters of UPD_CLUSTER
-        // consecutive ones, once with their recorded boxes and once with their current ones
+        // dirty boxes: the moved and added triangles in Morton order (tile slots of the current hierarchy), clusters of
+        // UPD_CLUSTER consecutive ones, the moved ones once with their recorded boxes, all of them with their current ones; then
+        // the boxes of the triangles removed since the record, in the order they were removed
         std::vector<int> order;
         for (int p = 0; p < ctx->nslots; p++) {
             const int t = ctx->h_order[p];
@@ -603,23 +666,34 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
         }
         std::vector<float4> leaf, cbox;
         std::vector<int2> crange;
-        for (int geom = 0; geom < 2; geom++) {
-            const float *V = geom ? V1 : V0;
-            const float pad = geom ? ctx->pad : ctx->rec.pad;
-            for (size_t i = 0; i < order.size(); i += UPD_CLUSTER) {
-                const size_t e = std::min(order.size(), i + UPD_CLUSTER);
+        auto add_clusters = [&](const std::vector<float4> &boxes) {
+            const size_t n = boxes.size() / 2;
+            for (size_t i = 0; i < n; i += UPD_CLUSTER) {
+                const size_t e = std::min(n, i + UPD_CLUSTER);
                 float4 u0 = make_float4(INFINITY, INFINITY, INFINITY, 0.f), u1 = make_float4(-INFINITY, -INFINITY, -INFINITY, 0.f);
                 crange.push_back(make_int2((int)(leaf.size() / 2), (int)(leaf.size() / 2 + (e - i))));
                 for (size_t j = i; j < e; j++) {
-                    float4 b[2];
-                    tri_box(V, tri, order[j], pad, b);
-                    leaf.push_back(b[0]); leaf.push_back(b[1]);
-                    u0 = make_float4(fminf(u0.x, b[0].x), fminf(u0.y, b[0].y), fminf(u0.z, b[0].z), 0.f);
-                    u1 = make_float4(fmaxf(u1.x, b[1].x), fmaxf(u1.y, b[1].y), fmaxf(u1.z, b[1].z), 0.f);
+                    const float4 b0 = boxes[2 * j], b1 = boxes[2 * j + 1];
+                    leaf.push_back(b0); leaf.push_back(b1);
+                    u0 = make_float4(fminf(u0.x, b0.x), fminf(u0.y, b0.y), fminf(u0.z, b0.z), 0.f);
+                    u1 = make_float4(fmaxf(u1.x, b1.x), fmaxf(u1.y, b1.y), fmaxf(u1.z, b1.z), 0.f);
                 }
                 cbox.push_back(u0); cbox.push_back(u1);
             }
+        };
+        std::vector<float4> boxes;
+        for (int geom = 0; geom < 2; geom++) {
+            boxes.clear();
+            for (const int t : order) {
+                float4 b[2];
+                if (geom == 0 && moved[(size_t)t] == 2) continue; // added: no recorded box
+                if (geom == 0) tri_box(R + 18 * (size_t)t, R + 18 * (size_t)t + 3, R + 18 * (size_t)t + 6, ctx->rec.pad, b);
+                else tri_box(V1 + 3 * (size_t)tri[6 * (size_t)t], V1 + 3 * (size_t)tri[6 * (size_t)t + 1], V1 + 3 * (size_t)tri[6 * (size_t)t + 2], ctx->pad, b);
+                boxes.push_back(b[0]); boxes.push_back(b[1]);
+            }
+            add_clusters(boxes);
         }
+        add_clusters(ghost);
         unsigned char *d_changed = nullptr;
         float4 *d_leaf = nullptr, *d_cbox = nullptr;
         int2 *d_crange = nullptr;
@@ -646,6 +720,209 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
     ctx->F_version++;
     set_record(ctx, variant);
     return DAISY_OK;
+}
+
+// ---- mesh replacement ------------------------------------------------------------------------------------------------
+// The matrix being replaced, as the remap reads it: old row p lives in block p / rows_per_rank, on that rank's device.
+struct RemapSrc {
+    const float *F[16];
+    int rows_per_rank, nranks, N;
+    int64_t ld;
+};
+
+// new row row0 + blockIdx.x = old row prev[r] gathered through prev[c]; +0.0 where a triangle is new, in the padding columns
+// and in the rows of the allocation past N
+__global__ void __launch_bounds__(256) k_remap_F(float *__restrict__ F, int64_t ld, int row0, int N, const int *__restrict__ prev, RemapSrc src) {
+    const int r = row0 + (int)blockIdx.x;
+    const int p = r < N ? prev[r] : -1;
+    const float *in = nullptr;
+    if (p >= 0) {
+        DZ_ASSERT(p < src.N);
+        const int g = min(p / src.rows_per_rank, src.nranks - 1);
+        DZ_ASSERT(g >= 0 && p - g * src.rows_per_rank < src.rows_per_rank);
+        in = src.F[g] + (size_t)(p - g * src.rows_per_rank) * src.ld;
+    }
+    float *out = F + (size_t)blockIdx.x * ld;
+    for (int64_t c = threadIdx.x; c < ld; c += blockDim.x) {
+        float v = 0.0f;
+        if (in && c < N) {
+            const int q = prev[c];
+            DZ_ASSERT(q >= -1 && q < src.N);
+            if (q >= 0) v = in[q];
+        }
+        out[c] = v;
+    }
+}
+
+// The build record follows the triangles: a continued triangle keeps its recorded vertices and normals, a new one has none, and
+// a recorded triangle nobody continues leaves its recorded box behind (in the Morton order of the hierarchy it leaves).  When
+// the survivors do not keep their relative order, the record is dropped: the visibility rays of a pair run from the lower to
+// the higher id and hits tie-break on (t, id), so a pair whose order flips may see other hits.
+static void carry_record(daisy_ctx *c, const int32_t *previous, int ntri, bool monotone) {
+    auto &rec = c->rec;
+    if (rec.valid && !monotone) rec.valid = false;
+    if (!rec.valid) { rec.tri.clear(); rec.has.clear(); rec.ghost.clear(); return; }
+    std::vector<char> kept((size_t)(c->N > 0 ? c->N : 1), 0);
+    for (int t = 0; t < ntri; t++)
+        if (previous[t] >= 0) kept[(size_t)previous[t]] = 1;
+    for (int p = 0; p < c->nslots; p++) {
+        const int t = c->h_order[p];
+        if (t < 0 || kept[(size_t)t] || !rec.has[(size_t)t]) continue;
+        const float *R = &rec.tri[18 * (size_t)t];
+        float4 b[2];
+        tri_box(R, R + 3, R + 6, rec.pad, b);
+        rec.ghost.push_back(b[0]); rec.ghost.push_back(b[1]);
+    }
+    std::vector<float> tri((size_t)18 * ntri);
+    std::vector<unsigned char> has((size_t)ntri, 0);
+    for (int t = 0; t < ntri; t++) {
+        const int p = previous[t];
+        if (p < 0 || !rec.has[(size_t)p]) continue;
+        memcpy(&tri[18 * (size_t)t], &rec.tri[18 * (size_t)p], 18 * sizeof(float));
+        has[(size_t)t] = 1;
+    }
+    rec.tri.swap(tri);
+    rec.has.swap(has);
+}
+
+int dz_replace_mesh(daisy_ctx *const *ctx, int n, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                    const int32_t *previous, const char *what) {
+    int rc = check_mesh(what, vertices, nv, normals, nn, tri_idx, ntri);
+    if (rc) return rc;
+    const int oldN = ctx[0]->N;
+    if (ntri > 0 && !previous) { daisy_set_error("%s: null previous", what); return DAISY_E_INVALID; }
+    bool monotone = true;
+    {
+        std::vector<char> seen((size_t)(oldN > 0 ? oldN : 1), 0);
+        int last = -1;
+        for (int t = 0; t < ntri; t++) {
+            const int p = previous[t];
+            if (p < -1 || p >= oldN) { daisy_set_error("%s: previous[%d] = %d is neither -1 nor a triangle of the current mesh (%d)", what, t, p, oldN); return DAISY_E_INVALID; }
+            if (p < 0) continue;
+            if (seen[(size_t)p]) { daisy_set_error("%s: triangle %d of the current mesh is continued twice (previous[%d])", what, p, t); return DAISY_E_INVALID; }
+            seen[(size_t)p] = 1;
+            monotone &= p > last;
+            last = p;
+        }
+    }
+    const bool remap = ctx[0]->d_F != nullptr; // a matrix exists: it is remapped so that its shape follows N
+    for (int i = 0; i < n; i++)
+        DZ_REQUIRE((ctx[i]->d_F != nullptr) == remap, DAISY_E_STATE, "replace mesh: some devices of the group hold a matrix and some do not");
+    const bool rewire = ctx[0]->peers_set;
+    const bool timing = getenv("DAISY_TIMING") != nullptr; // stderr: where the wall time of the call goes
+    const auto t0 = std::chrono::steady_clock::now();
+    // (1) everything new is allocated on every device before anything of a context changes
+    std::vector<MeshArrays> arr((size_t)n);
+    std::vector<float *> F((size_t)n, nullptr);
+    std::vector<int *> d_prev((size_t)n, nullptr);
+    std::vector<RowLayout> lay((size_t)n);
+    auto discard = [&]() {
+        for (int i = 0; i < n; i++) {
+            cudaSetDevice(ctx[i]->device);
+            free_mesh_arrays(arr[(size_t)i]);
+            cudaFree(F[(size_t)i]); cudaFree(d_prev[(size_t)i]);
+        }
+    };
+    auto cuda_fail = [&](cudaError_t e, const char *step) {
+        cudaGetLastError();
+        discard();
+        daisy_set_error("%s: %s: %s (the context is unchanged)", what, step, cudaGetErrorString(e));
+        return DAISY_E_CUDA;
+    };
+    for (int i = 0; i < n; i++) {
+        daisy_ctx *c = ctx[i];
+        cudaError_t e = cudaSetDevice(c->device);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream); // nothing enqueued may still read what is replaced
+        if (e != cudaSuccess) return cuda_fail(e, "device");
+        lay[(size_t)i] = row_layout(ntri, c->rank, c->nranks);
+        rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, arr[(size_t)i]);
+        if (rc) { discard(); return rc; }
+        if (!remap) continue;
+        const RowLayout &l = lay[(size_t)i];
+        const size_t bytes = sizeof(float) * (size_t)std::max(l.row1 - l.row0, 1) * (size_t)l.ldF;
+        e = cudaMalloc(&F[(size_t)i], bytes);
+        if (e == cudaErrorMemoryAllocation) {
+            cudaGetLastError();
+            discard();
+            daisy_set_error("%s: device %d: no room for the remapped matrix (%.2f GB) next to the current one; the context is unchanged", what, c->device, bytes * 1e-9);
+            return DAISY_E_NOMEM;
+        }
+        if (e == cudaSuccess) e = cudaMalloc(&d_prev[(size_t)i], sizeof(int) * (size_t)(ntri > 0 ? ntri : 1));
+        if (e == cudaSuccess && ntri) e = cudaMemcpy(d_prev[(size_t)i], previous, sizeof(int) * (size_t)ntri, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) return cuda_fail(e, "allocation");
+    }
+    // (2) remap on every device, reading the old rows where they live (a group's devices through peer access)
+    const auto t1 = std::chrono::steady_clock::now();
+    if (remap) {
+        RemapSrc src;
+        for (int g = 0; g < 16; g++) src.F[g] = g < n ? ctx[g]->d_F : nullptr;
+        src.rows_per_rank = ctx[0]->rows_per_rank; src.nranks = ctx[0]->nranks; src.N = oldN; src.ld = ctx[0]->ldF;
+        for (int i = 0; i < n; i++) {
+            const RowLayout &l = lay[(size_t)i];
+            cudaError_t e = cudaSetDevice(ctx[i]->device);
+            if (e == cudaSuccess) {
+                k_remap_F<<<std::max(l.row1 - l.row0, 1), 256, 0, ctx[i]->stream>>>(F[(size_t)i], l.ldF, l.row0, ntri, d_prev[(size_t)i], src);
+                e = cudaGetLastError();
+            }
+            if (e != cudaSuccess) return cuda_fail(e, "k_remap_F");
+        }
+        for (int i = 0; i < n; i++) {
+            cudaError_t e = cudaSetDevice(ctx[i]->device);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx[i]->stream);
+            if (e != cudaSuccess) return cuda_fail(e, "k_remap_F");
+        }
+    }
+    const auto t2 = std::chrono::steady_clock::now();
+    // (3) commit: the contexts take the new mesh, matrix and row layout
+    for (int i = 0; i < n; i++) {
+        daisy_ctx *c = ctx[i];
+        cudaSetDevice(c->device);
+        carry_record(c, previous, ntri, monotone);
+        install_mesh(c, vertices, nv, normals, nn, tri_idx, ntri, arr[(size_t)i]);
+        const RowLayout &l = lay[(size_t)i];
+        c->rows_per_rank = l.rows_per_rank; c->row0 = l.row0; c->row1 = l.row1; c->ldF = l.ldF;
+        if (remap) { cudaFree(c->d_F); c->d_F = F[(size_t)i]; cudaFree(d_prev[(size_t)i]); }
+        c->peers_set = false;
+        c->F_version++;
+        c->mesh_version++;
+    }
+    if (rewire) {
+        float *Fs[16] = { nullptr };
+        for (int i = 0; i < n; i++) Fs[i] = ctx[i]->d_F;
+        for (int i = 0; i < n; i++) {
+            rc = dz_ctx_set_peer_pointers(ctx[i], Fs, n);
+            if (rc) return rc;
+        }
+    }
+    // (4) everything derived from the mesh, rebuilt on every device at once
+    std::vector<int> rcs((size_t)n, DAISY_OK);
+    std::vector<std::string> errs((size_t)n);
+    auto rebuild = [&](int i) {
+        cudaSetDevice(ctx[i]->device);
+        rcs[(size_t)i] = build_geometry(ctx[i]);
+        if (rcs[(size_t)i]) errs[(size_t)i] = daisy_last_error();
+    };
+    if (n == 1) rebuild(0);
+    else {
+        std::vector<std::thread> th;
+        for (int i = 0; i < n; i++) th.emplace_back(rebuild, i);
+        for (auto &t : th) t.join();
+    }
+    for (int i = 0; i < n; i++)
+        if (rcs[(size_t)i]) { daisy_set_error("%s: device %d: %s", what, ctx[i]->device, errs[(size_t)i].c_str()); return rcs[(size_t)i]; }
+    if (timing)
+        fprintf(stderr, "%s: allocation %.3f s, k_remap_F %.3f s, host rebuild %.3f s\n", what, std::chrono::duration<double>(t1 - t0).count(),
+                std::chrono::duration<double>(t2 - t1).count(), std::chrono::duration<double>(std::chrono::steady_clock::now() - t2).count());
+    return DAISY_OK;
+}
+
+extern "C" int daisy_ctx_replace_mesh(daisy_ctx *ctx, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                                      const int32_t *previous) {
+    DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_ctx_replace_mesh: null context");
+    DZ_REQUIRE(ctx->nranks == 1, DAISY_E_STATE,
+               "daisy_ctx_replace_mesh: the context holds one block of a matrix partitioned across processes; the other rows live in the other processes (create new contexts instead)");
+    DzRange range_("daisy_ctx_replace_mesh: k_remap_F, plane ids, face grids, LBVH, patch records");
+    return dz_replace_mesh(&ctx, 1, vertices, nv, normals, nn, tri_idx, ntri, previous, "daisy_ctx_replace_mesh");
 }
 
 extern "C" int daisy_formfactors_update_stats(daisy_ctx *ctx, int64_t *tris_changed, int64_t *tiles_retraced, int64_t *pairs_retraced, double *classify_ms) {

@@ -332,16 +332,20 @@ struct daisy_ctx {
     // cudaMalloc / cudaFree pair per buffer per call (dz_scratch, api.cu)
     void *scratch[6] = { nullptr, nullptr, nullptr, nullptr, nullptr, nullptr };
     size_t scratch_bytes[6] = { 0, 0, 0, 0, 0, 0 };
-    // host copies of the mesh: the current geometry (daisy_ctx_create / daisy_ctx_update_geometry) and the triangle list
+    // host copies of the mesh: the current geometry (daisy_ctx_create / _update_geometry / _replace_mesh) and the triangle list
     std::vector<float> h_vertices, h_normals;
     std::vector<int> h_tri;
+    uint64_t mesh_version = 0; // bumped by daisy_ctx_replace_mesh: solvers created before it are stale (other N, other materials)
     // what F holds (daisy_formfactors_build / _update): the variant, sample pattern and geometry it was computed for, and the
-    // box padding of that geometry.  Cleared by daisy_formfactors_write_rows.
+    // box padding of that geometry.  Cleared by daisy_formfactors_write_rows.  Per CURRENT triangle, so that it follows the
+    // triangles through daisy_ctx_replace_mesh; triangles removed since the record leave their recorded boxes behind.
     struct {
         bool valid = false;
         int variant = 0, S = 0;
         float uv[2 * DAISY_MAX_SAMPLES];
-        std::vector<float> vertices, normals;
+        std::vector<float> tri;         // 18 floats per triangle: its 3 vertex positions, then its 3 normals, as recorded
+        std::vector<unsigned char> has; // per triangle: 1 = recorded, 0 = added since the record
+        std::vector<float4> ghost;      // 2 float4 per triangle removed since the record: its recorded padded box
         float pad = 0.f;
     } rec;
     // last daisy_formfactors_update
@@ -374,6 +378,9 @@ int dz_unoccluded_rows(daisy_ctx *ctx, int variant, int row0, int nrows, daisy_t
 struct daisy_solver;
 // same-process peers (daisy_group): device pointers handed over directly, peer access enabled by the caller
 int dz_ctx_set_peer_pointers(daisy_ctx *ctx, float *const *F, int nranks);                                           // api.cu
+// daisy_ctx_replace_mesh over ctx[0..n): one context, or every device of a group (rank i of n, F remapped through peer access)  // api.cu
+int dz_replace_mesh(daisy_ctx *const *ctx, int n, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                    const int32_t *previous, const char *what);
 int dz_solver_get_buffers(daisy_solver *s, float **res0, float **res1, unsigned long long **flags);                  // gather.cu
 int dz_solver_set_peer_pointers(daisy_solver *s, float *const *res0, float *const *res1, unsigned long long *const *flags, int nranks); // gather.cu
 // converge with the stop rule on the device over n solvers issued from one thread (one GPU, or a group's devices)   // gather.cu

@@ -29,8 +29,15 @@
 #define G_THREADS (G_WARPS * 32)
 #define G_TC 512 // residual tile width (columns)
 
+// a solver is sized by the mesh its context held at daisy_solver_create (N, row blocks, material ids); after
+// daisy_ctx_replace_mesh every call but destroy refuses it
+#define DZ_SOLVER_CURRENT(s, what)                                                                                           \
+    DZ_REQUIRE((s)->mesh_version == (s)->ctx->mesh_version, DAISY_E_STATE,                                                   \
+               what ": the context's mesh was replaced (daisy_ctx_replace_mesh) after this solver was created; create a new solver")
+
 struct daisy_solver {
     daisy_ctx *ctx = nullptr;
+    uint64_t mesh_version = 0; // the context's mesh_version at create: the mesh N, the row blocks and mat_idx belong to
     int K = 0, Kp = 0; // bands requested / bands the kernel is instantiated for
     int nmat = 0;
     int N = 0, n = 0, G = 1, rank = 0, nloc = 0, row0 = 0;
@@ -1372,7 +1379,7 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
         DZ_REQUIRE(mat_idx[p] >= 0 && mat_idx[p] < nmat, DAISY_E_INVALID, "daisy_solver_create: material index out of range");
     DZ_CUDA(cudaSetDevice(ctx->device));
     daisy_solver *s = new daisy_solver();
-    s->ctx = ctx; s->K = K; s->Kp = padded_K(K); s->nmat = nmat;
+    s->ctx = ctx; s->mesh_version = ctx->mesh_version; s->K = K; s->Kp = padded_K(K); s->nmat = nmat;
     s->N = ctx->N; s->n = ctx->rows_per_rank; s->G = ctx->nranks; s->rank = ctx->rank;
     s->row0 = ctx->row0; s->nloc = ctx->row1 - ctx->row0;
     int64_t body = (int64_t)s->Kp * s->n;
@@ -1449,6 +1456,7 @@ extern "C" void daisy_solver_destroy(daisy_solver *s) {
 
 extern "C" int daisy_solver_reset(daisy_solver *s) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_reset: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_reset");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
     size_t exb = sizeof(float) * (size_t)s->G * s->bstride;
@@ -1473,8 +1481,8 @@ extern "C" int daisy_solver_reset(daisy_solver *s) {
     return DAISY_OK;
 }
 
-extern "C" int daisy_solver_step_local(daisy_solver *s) {
-    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step_local: null solver");
+// the passes of daisy_solver_step_local / _step_finish; daisy_solver_step and _step_fused check the solver once per pass
+static int step_local(daisy_solver *s) {
     DzRange range_("gather pass");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
@@ -1488,12 +1496,14 @@ extern "C" int daisy_solver_step_local(daisy_solver *s) {
 
 extern "C" int daisy_solver_set_chained(daisy_solver *s, int on) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_set_chained: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_set_chained");
     s->chained = on != 0;
     return DAISY_OK;
 }
 
 extern "C" int daisy_solver_exchange_info(daisy_solver *s, void **d_next_buffer, int64_t *block_bytes, int64_t *total_bytes) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_exchange_info: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_exchange_info");
     if (d_next_buffer) *d_next_buffer = s->d_res[s->cur ^ 1];
     if (block_bytes) *block_bytes = (int64_t)sizeof(float) * s->bstride;
     if (total_bytes) *total_bytes = (int64_t)sizeof(float) * s->bstride * s->G;
@@ -1536,8 +1546,7 @@ static int fetch_sums(daisy_solver *s) {
 
 // band_sums == NULL: nothing is read back and the call does not wait for the device (back-to-back passes);
 // the sums are fetched lazily by daisy_solver_band_sums / daisy_solver_converge.
-extern "C" int daisy_solver_step_finish(daisy_solver *s, double *band_sums) {
-    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step_finish: null solver");
+static int step_finish(daisy_solver *s, double *band_sums) {
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     s->cur ^= 1;
     s->numpasses++;
@@ -1549,17 +1558,31 @@ extern "C" int daisy_solver_step_finish(daisy_solver *s, double *band_sums) {
     return DAISY_OK;
 }
 
+extern "C" int daisy_solver_step_local(daisy_solver *s) {
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step_local: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_step_local");
+    return step_local(s);
+}
+
+extern "C" int daisy_solver_step_finish(daisy_solver *s, double *band_sums) {
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step_finish: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_step_finish");
+    return step_finish(s, band_sums);
+}
+
 extern "C" int daisy_solver_step(daisy_solver *s, double *band_sums) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_step");
     DZ_REQUIRE(s->G == 1, DAISY_E_STATE, "daisy_solver_step: partitioned solver needs step_local / exchange / step_finish");
-    int rc = daisy_solver_step_local(s);
+    int rc = step_local(s);
     if (rc) return rc;
-    return daisy_solver_step_finish(s, band_sums);
+    return step_finish(s, band_sums);
 }
 
 // ---- fused exchange over peer memory (multi-GPU, one process per GPU) ------------------------------------------
 extern "C" int daisy_solver_ipc_handles(daisy_solver *s, void *handles192) {
     DZ_REQUIRE(s && handles192, DAISY_E_INVALID, "daisy_solver_ipc_handles: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_ipc_handles");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaIpcMemHandle_t h[3];
@@ -1572,6 +1595,7 @@ extern "C" int daisy_solver_ipc_handles(daisy_solver *s, void *handles192) {
 
 extern "C" int daisy_solver_set_peers(daisy_solver *s, const void *handles, int nranks) {
     DZ_REQUIRE(s && handles, DAISY_E_INVALID, "daisy_solver_set_peers: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_set_peers");
     DZ_REQUIRE(nranks == s->G && nranks <= 16, DAISY_E_INVALID, "daisy_solver_set_peers: nranks must match the partition (<= 16)");
     DZ_REQUIRE(!s->fused, DAISY_E_STATE, "daisy_solver_set_peers: peers already set");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
@@ -1621,6 +1645,7 @@ __global__ void k_raise_flags(int npeers, unsigned long long seq, const unsigned
 
 extern "C" int daisy_solver_write_slices(daisy_solver *s, const float *B_local, const float *residual_local) {
     DZ_REQUIRE(s && B_local && residual_local, DAISY_E_INVALID, "daisy_solver_write_slices: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_write_slices");
     DZ_REQUIRE(s->G == 1 || s->fused, DAISY_E_STATE, "daisy_solver_write_slices: a partitioned solver needs the fused exchange (daisy_solver_set_peers)");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
@@ -1659,6 +1684,7 @@ extern "C" int daisy_solver_write_slices(daisy_solver *s, const float *B_local, 
 // this rank's new block into every rank's next buffer and raise the flags.  No host synchronisation, no NCCL call.
 extern "C" int daisy_solver_step_fused(daisy_solver *s, double *band_sums) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_step_fused: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_step_fused");
     DZ_REQUIRE(s->fused, DAISY_E_STATE, "daisy_solver_step_fused: call daisy_solver_set_peers first");
     DzRange range_("gather pass + fused exchange");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
@@ -1675,7 +1701,7 @@ extern "C" int daisy_solver_step_fused(daisy_solver *s, double *band_sums) {
     if (rc) return rc;
     DZ_CUDA(cudaEventRecord(s->e1, st));
     s->events_recorded = true;
-    return daisy_solver_step_finish(s, band_sums);
+    return step_finish(s, band_sums);
 }
 
 static bool unconverged(const daisy_solver *s, double threshold, int per_band) {
@@ -1690,13 +1716,15 @@ static bool unconverged(const daisy_solver *s, double threshold, int per_band) {
 
 extern "C" int daisy_solver_converge(daisy_solver *s, double threshold, int per_band, int max_passes, int *passes_out) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_converge: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_converge");
     DZ_REQUIRE(s->G == 1, DAISY_E_STATE, "daisy_solver_converge: partitioned solver is driven by the host exchange loop (or daisy_group_solver_converge)");
     DzRange range_("daisy_solver_converge");
     int done = 0;
     std::vector<double> tmp(s->K);
     if (!s->sums_valid) { int rc = fetch_sums(s); if (rc) return rc; }
     while (unconverged(s, threshold, per_band) && (max_passes <= 0 || done < max_passes)) {
-        int rc = daisy_solver_step(s, tmp.data());
+        int rc = step_local(s);
+        if (!rc) rc = step_finish(s, tmp.data());
         if (rc) return rc;
         done++;
     }
@@ -1737,6 +1765,7 @@ int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per
     daisy_solver *s0 = ss[0];
     for (int i = 0; i < n; i++) {
         daisy_solver *s = ss[i];
+        DZ_SOLVER_CURRENT(s, "daisy_solver_converge_device");
         DZ_CUDA(cudaSetDevice(s->ctx->device));
         if (s->fused && s->h_abort && *reinterpret_cast<volatile unsigned long long *>(s->h_abort) != 0ull) return abort_error(s);
         int rc = ensure_stop_buffers(s);
@@ -1823,6 +1852,7 @@ int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per
 
 extern "C" int daisy_solver_converge_device(daisy_solver *s, double threshold, int per_band, int max_passes, int *passes_out) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_converge_device: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_converge_device");
     DZ_REQUIRE(s->G == 1 || s->fused, DAISY_E_STATE, "daisy_solver_converge_device: a partitioned solver needs the fused exchange (daisy_solver_set_peers)");
     DzRange range_("daisy_solver_converge_device");
     int rc = dz_converge_device(&s, 1, threshold, per_band, max_passes);
@@ -1831,10 +1861,15 @@ extern "C" int daisy_solver_converge_device(daisy_solver *s, double threshold, i
     return DAISY_OK;
 }
 
-extern "C" int daisy_solver_numpasses(daisy_solver *s) { return s ? s->numpasses : DAISY_E_INVALID; }
+extern "C" int daisy_solver_numpasses(daisy_solver *s) {
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_numpasses: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_numpasses");
+    return s->numpasses;
+}
 
 extern "C" int daisy_solver_band_sums(daisy_solver *s, double *band_sums) {
     DZ_REQUIRE(s && band_sums, DAISY_E_INVALID, "daisy_solver_band_sums: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_band_sums");
     if (!s->sums_valid) { DZ_CUDA(cudaSetDevice(s->ctx->device)); int rc = fetch_sums(s); if (rc) return rc; }
     memcpy(band_sums, s->sums.data(), sizeof(double) * s->K);
     return DAISY_OK;
@@ -1842,6 +1877,7 @@ extern "C" int daisy_solver_band_sums(daisy_solver *s, double *band_sums) {
 
 extern "C" int daisy_solver_read(daisy_solver *s, float *B, float *residual) {
     DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_read: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_read");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     // local rows only: out[k*nloc + pl]; both copies ride the solver's stream behind the passes, one synchronisation at the end
     cudaStream_t st = s->ctx->stream;
@@ -1856,6 +1892,7 @@ extern "C" int daisy_solver_read(daisy_solver *s, float *B, float *residual) {
 
 extern "C" int daisy_solver_write(daisy_solver *s, const float *B, const float *residual) {
     DZ_REQUIRE(s && B && residual, DAISY_E_INVALID, "daisy_solver_write: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_write");
     DZ_REQUIRE(s->G == 1, DAISY_E_STATE, "daisy_solver_write: single-GPU solvers only");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
@@ -1872,6 +1909,7 @@ extern "C" int daisy_solver_write(daisy_solver *s, const float *B, const float *
 // rank holds the whole residual vector, as after an exchange)
 extern "C" int daisy_solver_write_partitioned(daisy_solver *s, const float *B_local, const float *residual_full) {
     DZ_REQUIRE(s && B_local && residual_full, DAISY_E_INVALID, "daisy_solver_write_partitioned: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_write_partitioned");
     DZ_CUDA(cudaSetDevice(s->ctx->device));
     cudaStream_t st = s->ctx->stream;
     if (s->fused && s->seq > 0) { // peers' stores of the last pass have landed
@@ -1894,7 +1932,8 @@ extern "C" int daisy_solver_write_partitioned(daisy_solver *s, const float *B_lo
 
 // kernels one pass launches in this solver's configuration (the benchmark reports it)
 extern "C" int daisy_solver_launches_per_pass(daisy_solver *s) {
-    if (!s) return DAISY_E_INVALID;
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_launches_per_pass: null solver");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_launches_per_pass");
     if (s->fused_epi) return 1;                         // k_gather_tma with the epilogue and the exchange wait inside
     int n = 2;                                          // streaming kernel + k_gather_epilogue
     if (s->use_mma) n += 1;                             // k_split_residual
@@ -1904,6 +1943,7 @@ extern "C" int daisy_solver_launches_per_pass(daisy_solver *s) {
 
 extern "C" int daisy_solver_last_step_ms(daisy_solver *s, double *ms) {
     DZ_REQUIRE(s && ms, DAISY_E_INVALID, "daisy_solver_last_step_ms: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_last_step_ms");
     *ms = s->last_ms;
     return DAISY_OK;
 }
@@ -1913,6 +1953,7 @@ extern "C" int daisy_solver_last_step_ms(daisy_solver *s, double *ms) {
 // of the scan kernel
 extern "C" int daisy_solver_tile_map(daisy_solver *s, int32_t *dims2, uint8_t *occ, int64_t capacity, int64_t *occupied, double *scan_ms) {
     DZ_REQUIRE(s && dims2, DAISY_E_INVALID, "daisy_solver_tile_map: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_tile_map");
     const bool have = s->skip && !s->occ.empty();
     dims2[0] = have ? (int32_t)(s->occ.size() / (size_t)s->sk_S) : 0;
     dims2[1] = have ? s->sk_S : 0;

@@ -23,6 +23,7 @@ struct daisy_group {
 
 struct daisy_group_solver {
     daisy_group *g = nullptr;
+    uint64_t mesh_version = 0; // device 0's mesh_version at create (daisy_group_replace_mesh moves every device's)
     int K = 0;
     std::vector<daisy_solver *> s;
 };
@@ -164,6 +165,15 @@ extern "C" int daisy_group_formfactors_update(daisy_group *g, int variant) {
     return rc;
 }
 
+extern "C" int daisy_group_replace_mesh(daisy_group *g, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                                        const int32_t *previous) {
+    DZ_REQUIRE(g, DAISY_E_INVALID, "daisy_group_replace_mesh: null group");
+    DzRange range_("daisy_group_replace_mesh");
+    const int rc = dz_replace_mesh(g->ctx.data(), g->ndev, vertices, nv, normals, nn, tri_idx, ntri, previous, "daisy_group_replace_mesh");
+    g->N = g->ctx[0]->N;
+    return rc;
+}
+
 static int owner_of(daisy_group *g, int row) {
     const int n = g->ctx[0]->rows_per_rank;
     int o = n > 0 ? row / n : 0;
@@ -288,7 +298,7 @@ extern "C" int daisy_group_solver_create(daisy_group *g, int K, const float *E, 
     DZ_REQUIRE(g && out, DAISY_E_INVALID, "daisy_group_solver_create: null argument");
     *out = nullptr;
     daisy_group_solver *gs = new daisy_group_solver();
-    gs->g = g; gs->K = K;
+    gs->g = g; gs->K = K; gs->mesh_version = g->ctx[0]->mesh_version;
     gs->s.assign((size_t)g->ndev, nullptr);
     int rc = for_each_device(g, "daisy_group_solver_create", [&](int i) { return daisy_solver_create(g->ctx[(size_t)i], K, E, M, nmat, mat_idx, &gs->s[(size_t)i]); });
     if (!rc && g->ndev > 1) {
@@ -370,6 +380,8 @@ extern "C" int daisy_group_solver_converge_device(daisy_group_solver *gs, double
 // lightningvalues and residualvector of the whole scene, K x N band-major, assembled from the devices' row blocks
 extern "C" int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *residual) {
     DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_read: null solver");
+    DZ_REQUIRE(gs->mesh_version == gs->g->ctx[0]->mesh_version, DAISY_E_STATE,
+               "daisy_group_solver_read: the group's mesh was replaced after this solver was created; create a new solver");
     daisy_group *g = gs->g;
     const int N = g->N, K = gs->K;
     std::vector<float> b, r;
@@ -392,6 +404,8 @@ extern "C" int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *
 // slices reach the other devices over NVLink (daisy_solver_write_slices)
 extern "C" int daisy_group_solver_write(daisy_group_solver *gs, const float *B, const float *residual) {
     DZ_REQUIRE(gs && B && residual, DAISY_E_INVALID, "daisy_group_solver_write: null argument");
+    DZ_REQUIRE(gs->mesh_version == gs->g->ctx[0]->mesh_version, DAISY_E_STATE,
+               "daisy_group_solver_write: the group's mesh was replaced after this solver was created; create a new solver");
     daisy_group *g = gs->g;
     const int N = g->N, K = gs->K;
     if (g->ndev == 1) return daisy_solver_write(gs->s[0], B, residual);

@@ -255,6 +255,62 @@ def cornell_moved(scene: Scene, quads, offset=(0.0, 0.0, 0.0), angle_y: float = 
     return V32, VN32
 
 
+def cornell_panel(n_patches: int) -> Scene:
+    """A free-standing white panel for :func:`cornell_box` scenes of ``n_patches``: 1.1 x 1.4 at z = 4.6, facing the room (+z),
+    subdivided like one quad of the box (``n_patches / 16`` triangles).  The object the mesh-edit tests and tools add."""
+    nu, nv = cornell_subdivision(n_patches)
+    V, VN, T, M = [], [], [], []
+    _quad((0.6, 1.2, 4.6), (1.1, 0, 0), (0, 1.4, 0), nu, nv, (0, 0, 1), V, VN, T, M, 0)
+    white = next(m for m in CORNELL_MATERIALS if m["name"] == "white")
+    mats = [{k: (np.asarray(v, np.float32) if k != "name" else v) for k, v in white.items()}]
+    return Scene(np.asarray(V, np.float32), np.asarray(VN, np.float32), np.asarray(T, np.int32), np.asarray(M, np.int32), mats, "panel")
+
+
+def edit_scene(scene: Scene, remove=(), add: Scene | None = None, insert_at: int | None = None):
+    """``(edited scene, previous)``: ``scene`` without the triangles listed in ``remove``, with the triangles of ``add`` inserted
+    before surviving triangle ``insert_at`` (appended when ``None``); the vertex and normal arrays are compacted to the entries
+    the triangles use and renumbered (survivors keep their relative order).  Materials follow their triangles; a material of
+    ``add`` is matched to one of ``scene`` by name or appended.  ``previous[t]`` = the index in ``scene`` of the triangle new
+    triangle t continues, -1 for an added one: the ``previous`` argument of ``replaceMesh``."""
+    N = scene.numtriangles
+    remove = np.asarray(remove, np.int64).reshape(-1)
+    if remove.size and (remove.min() < 0 or remove.max() >= N):
+        raise ValueError("edit_scene: a removed triangle is not in the scene")
+    keep = np.ones(N, bool)
+    keep[remove] = False
+    kept = np.nonzero(keep)[0]
+    V = [np.asarray(scene.vertices, np.float32).reshape(-1, 3)]
+    VN = [np.asarray(scene.normals, np.float32).reshape(-1, 3)]
+    tri, mat, prev = scene.tri[kept].astype(np.int64), scene.mat_idx[kept].astype(np.int64), kept.astype(np.int64)
+    mats = list(scene.materials)
+    if add is not None:
+        names = {m["name"]: i for i, m in enumerate(mats)}
+        mat_map = []
+        for m in add.materials:
+            if m["name"] not in names:
+                names[m["name"]] = len(mats)
+                mats.append(m)
+            mat_map.append(names[m["name"]])
+        add_tri = add.tri.astype(np.int64) + np.array([V[0].shape[0]] * 3 + [VN[0].shape[0]] * 3, np.int64)
+        add_mat = np.asarray(mat_map, np.int64)[add.mat_idx] if len(mat_map) else np.asarray(add.mat_idx, np.int64)
+        at = len(kept) if insert_at is None else int(insert_at)
+        if not 0 <= at <= len(kept):
+            raise ValueError("edit_scene: insert_at is not a position in the surviving triangles")
+        tri = np.concatenate([tri[:at], add_tri, tri[at:]])
+        mat = np.concatenate([mat[:at], add_mat, mat[at:]])
+        prev = np.concatenate([prev[:at], np.full(add.numtriangles, -1, np.int64), prev[at:]])
+        V.append(np.asarray(add.vertices, np.float32).reshape(-1, 3))
+        VN.append(np.asarray(add.normals, np.float32).reshape(-1, 3))
+    V, VN = np.concatenate(V), np.concatenate(VN)
+    used_v, used_n = np.unique(tri[:, :3]), np.unique(tri[:, 3:])
+    vmap, nmap = np.full(V.shape[0], -1, np.int64), np.full(VN.shape[0], -1, np.int64)
+    vmap[used_v], nmap[used_n] = np.arange(used_v.size), np.arange(used_n.size)
+    tri = np.concatenate([vmap[tri[:, :3]], nmap[tri[:, 3:]]], 1)
+    out = Scene(np.ascontiguousarray(V[used_v]), np.ascontiguousarray(VN[used_n]), tri.astype(np.int32).reshape(-1, 6), mat.astype(np.int32),
+                mats, scene.name)
+    return out, prev.astype(np.int32)
+
+
 def write_obj(scene: Scene, directory: str, stem: str | None = None):
     """Write ``scene`` as OBJ + MTL (the inverse of :func:`load_obj`; float32 values survive the round trip).
     Lets the reference's own loader (``MeshS::loadFromFile``) read the synthetic scenes."""

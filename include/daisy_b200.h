@@ -166,6 +166,22 @@ int daisy_formfactors_stats(daisy_ctx *ctx, int64_t *pairs_traced, int64_t *pair
  * daisy_formfactors_update_stats: the last update's triangles changed, tiles and facing pairs this context re-traced, and
  * device milliseconds of the tile classification. */
 int daisy_ctx_update_geometry(daisy_ctx *ctx, const float *vertices, int nv, const float *normals, int nn);
+/* daisy_ctx_replace_mesh: a new mesh with any counts (objects deleted, added, the vertex array renumbered).  previous[t] (ntri
+ * entries) = index in the current mesh of the triangle that new triangle t continues (the same patch, possibly moved), or -1 for
+ * a new triangle; each current index appears at most once; current triangles nobody continues are removed.  Invalid input
+ * (what daisy_ctx_create rejects, previous out of range or with a duplicate): DAISY_E_INVALID, the context unchanged.
+ * Everything daisy_ctx_create derives from the mesh is rebuilt, so N, daisy_ctx_row_range, daisy_formfactors_ld, closest hit,
+ * daisy_trace_screen, daisy_visibility_masks and daisy_unoccluded_rows answer for the new mesh at once.  F is remapped at once
+ * (its shape always matches N): entry (r, c) = the old entry (previous[r], previous[c]), +0.0 where r or c is new; nothing else
+ * in F changes until daisy_formfactors_update, which re-traces only the pairs the edit can reach (pairs with a new or changed
+ * patch, and pairs whose shaft meets a moved, new or removed triangle) and gives F bit for bit as a fresh build -- provided the
+ * surviving triangles keep their relative order (previous increasing over its entries >= 0); otherwise that update traces
+ * everything.  The old and the new matrix coexist during the remap: when both do not fit, DAISY_E_NOMEM and the context is
+ * unchanged.  Solvers created on the context before the call return DAISY_E_STATE from every call but destroy: create new
+ * ones.  A context partitioned across processes (daisy_ctx_set_partition with nranks > 1) cannot replace its mesh (the other
+ * rows of its matrix live in the other processes): DAISY_E_STATE. */
+int daisy_ctx_replace_mesh(daisy_ctx *ctx, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                           const int32_t *previous);
 int daisy_formfactors_update(daisy_ctx *ctx, int variant);
 int daisy_formfactors_update_stats(daisy_ctx *ctx, int64_t *tris_changed, int64_t *tiles_retraced, int64_t *pairs_retraced, double *classify_ms);
 
@@ -293,6 +309,10 @@ int daisy_group_formfactors_stats(daisy_group *g, int64_t *pairs, int64_t *rays,
 /* daisy_ctx_update_geometry / daisy_formfactors_update on every device (each traces its share of the tiles the update reaches) */
 int daisy_group_update_geometry(daisy_group *g, const float *vertices, int nv, const float *normals, int nn);
 int daisy_group_formfactors_update(daisy_group *g, int variant);
+/* daisy_ctx_replace_mesh on every device: the new row blocks are computed and every device's new matrix allocated first, then
+ * each device remaps its block, reading the old rows from whichever device owned them over peer access */
+int daisy_group_replace_mesh(daisy_group *g, const float *vertices, int nv, const float *normals, int nn, const int32_t *tri_idx, int ntri,
+                             const int32_t *previous);
 int daisy_group_solver_create(daisy_group *g, int K, const float *E, const float *M, int nmat, const int32_t *mat_idx,
                               daisy_group_solver **out);
 void daisy_group_solver_destroy(daisy_group_solver *gs);

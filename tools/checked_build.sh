@@ -11,6 +11,7 @@ timeout 1800 python -m pytest tests/test_gpu_parity.py tests/test_gpu_gather_sha
 timeout 1800 python -m pytest tests/test_gpu_far_geometry.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_converge_device.py -x -q -m gpu -k "not group and not two_process and not shim" 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_geometry_update.py -x -q -m gpu -k "not group" 2>&1 | tail -4
+timeout 1800 python -m pytest tests/test_gpu_mesh_edit.py -x -q -m gpu -k "not group" 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_matrix_cache.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_wide_bands.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_ff_limits.py -x -q -m gpu 2>&1 | tail -4
