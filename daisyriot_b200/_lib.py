@@ -114,6 +114,12 @@ SYMBOLS = {
     "daisy_solver_step_finish": (_i, [_vp, _dp]),
     "daisy_solver_last_step_ms": (_i, [_vp, _dp]),
     "daisy_solver_set_chained": (_i, [_vp, _i]),
+    "daisy_solver_restart": (_i, [_vp, _fp]),
+    "daisy_solver_set_emission": (_i, [_vp, _fp]),
+    "daisy_solver_set_materials": (_i, [_vp, _fp, _i, _ip]),
+    "daisy_group_solver_restart": (_i, [_vp, _fp]),
+    "daisy_group_solver_set_emission": (_i, [_vp, _fp]),
+    "daisy_group_solver_set_materials": (_i, [_vp, _fp, _i, _ip]),
 }
 
 _LIB = None

@@ -477,6 +477,55 @@ class GroupSolver:
         R = np.ascontiguousarray(R, np.float32)
         _lib.check(_lib.lib().daisy_group_solver_write(self._s, _lib.fptr(B), _lib.fptr(R)), "group_solver_write")
 
+    def restart(self, B0=None):
+        """:meth:`Lightning.restart` over every device; ``B0`` is K x N (whole scene) or ``None`` for the current B."""
+        b = None
+        if B0 is not None:
+            b = np.ascontiguousarray(B0, np.float32)
+            if b.shape != (self.K, self.group.N):
+                raise ValueError("restart: B0 must be K x N, got %s" % (b.shape,))
+        _lib.check(_lib.lib().daisy_group_solver_restart(self._s, None if b is None else _lib.fptr(b)), "group_solver_restart")
+
+    def set_emission(self, E):
+        E = np.ascontiguousarray(E, np.float32)
+        if E.shape != (self.K, self.group.N):
+            raise ValueError("set_emission: E must be K x N, got %s" % (E.shape,))
+        _lib.check(_lib.lib().daisy_group_solver_set_emission(self._s, _lib.fptr(E)), "group_solver_set_emission")
+
+    def set_materials(self, M, mat_idx):
+        M, mat = _material_arrays(M, mat_idx, self.K, self.group.N)
+        _lib.check(_lib.lib().daisy_group_solver_set_materials(self._s, _lib.fptr(M), M.shape[0], _lib.iptr(mat)), "group_solver_set_materials")
+
+
+def remap_bands(B_old, previous, E_new) -> np.ndarray:
+    """A warm start for the solver of an edited mesh (:meth:`OptixPrimeFunctionality.replaceMesh`): column t of the result is
+    ``B_old[:, previous[t]]`` for a triangle that continues old triangle ``previous[t]``, and ``E_new[:, t]`` for a new one
+    (``previous[t] == -1``).  K x N_new float32."""
+    B_old = np.asarray(B_old, np.float32)
+    E_new = np.asarray(E_new, np.float32)
+    p = np.asarray(previous)
+    if B_old.ndim != 2 or E_new.ndim != 2 or B_old.shape[0] != E_new.shape[0]:
+        raise ValueError("remap_bands: B_old (K x N_old) and E_new (K x N_new) need the same band count")
+    if p.ndim != 1 or p.shape[0] != E_new.shape[1]:
+        raise ValueError("remap_bands: previous needs one entry per triangle of the new mesh")
+    if p.size and not np.issubdtype(p.dtype, np.integer):
+        raise ValueError("remap_bands: previous holds triangle indices (integers)")
+    if p.size and (p.min() < -1 or p.max() >= B_old.shape[1]):
+        raise ValueError("remap_bands: previous holds an index outside [-1, N_old)")
+    out = np.array(E_new, np.float32, copy=True)
+    kept = p >= 0
+    out[:, kept] = B_old[:, p[kept]]
+    return np.ascontiguousarray(out)
+
+
+def _material_arrays(M, mat_idx, K: int, N: int):
+    """Contiguous float32 nmat x K x K materials and int32 ids, checked for their shapes (the ids' range the library checks)."""
+    M = np.ascontiguousarray(M, np.float32)
+    mat = np.ascontiguousarray(mat_idx, np.int32).reshape(-1)
+    if M.ndim != 3 or M.shape[1:] != (K, K) or mat.size != N:
+        raise ValueError("set_materials: M must be nmat x K x K and mat_idx hold N ids")
+    return M, mat
+
 
 def _csc_arrays(values, inner, outer, n: int):
     """Contiguous float32 / int32 copies of CSC arrays, checked for their lengths (the values themselves the library checks)."""
@@ -620,17 +669,25 @@ class Lightning:
             self.initMat(mesh, optixP)
         else:
             self.initMatFromFile(mesh, optixP, matfile)
-        E = np.ascontiguousarray(E, np.float32)
-        M = np.ascontiguousarray(M, np.float32)
-        mat = np.ascontiguousarray(mesh.materialIndexPerTriangle, np.int32)
-        self.K = E.shape[0]
-        self._s = C.c_void_p()
-        _lib.check(_lib.lib().daisy_solver_create(optixP._ctx, self.K, _lib.fptr(E), _lib.fptr(M), M.shape[0], _lib.iptr(mat),
-                                                  C.byref(self._s)), "solver_create")
-        self.emission = E
+        self._create_solver(E, M)
         self.reset()
         if converge:
             self.converge_lightning()
+
+    def _create_solver(self, E, M):
+        """A solver on the context's current matrix for ``self.mesh_`` (emission E, materials M)."""
+        E = np.ascontiguousarray(E, np.float32)
+        M = np.ascontiguousarray(M, np.float32)
+        mat = np.ascontiguousarray(self.mesh_.materialIndexPerTriangle, np.int32)
+        self.K = E.shape[0]
+        self._s = C.c_void_p()
+        _lib.check(_lib.lib().daisy_solver_create(self.optixP._ctx, self.K, _lib.fptr(E), _lib.fptr(M), M.shape[0], _lib.iptr(mat),
+                                                  C.byref(self._s)), "solver_create")
+        self.emission = E
+
+    def _derive_inputs(self, emissionval):
+        """(E, M) of ``self.mesh_`` by the flavour's own rule (set_sampled_emission / set_reflection*, Lightning.h:263-292)."""
+        raise NotImplementedError
 
     def initMat(self, mesh, optixP):  # Lightning.h:75-83
         self.RadMat = optixP.cudaCalculateRadiosityMatrix() if self.cuda_on else optixP.calculateRadiosityMatrix()
@@ -697,6 +754,52 @@ class Lightning:
         self._after_update()
         return passes.value
 
+    # -- warm restart: the solve continues from the current (or a given) B after the matrix, emission or materials changed ----
+    def restart(self, B0=None):
+        """One pass that starts the iteration from ``B0`` (K x N of this context's rows) or, ``None``, from the current B:
+        B = E + M F B0, residual = B - B0 (``daisy_solver_restart``).  Band sums then total |residual| until the next
+        :meth:`reset`.  Returns those band sums."""
+        b = None
+        if B0 is not None:
+            r0, r1 = self.optixP.row_range
+            b = np.ascontiguousarray(B0, np.float32)
+            if b.shape != (self.K, r1 - r0):
+                raise ValueError("restart: B0 must be K x N (this context's rows), got %s" % (b.shape,))
+        _lib.check(_lib.lib().daisy_solver_restart(self._s, None if b is None else _lib.fptr(b)), "solver_restart")
+        self._after_update()
+        return self.band_sums()
+
+    def reconverge(self, max_passes: int = 0, on_device: bool = False):
+        """Restart from the current B and converge: the passes of the new solve, restart pass included."""
+        self.restart()
+        return self.converge_lightning(max_passes, on_device)
+
+    def set_emission_value(self, emissionval):
+        """Re-derive E for a new emission value with the flavour's own rule; B and the residual are untouched until
+        :meth:`restart` (or :meth:`reset`)."""
+        E, _ = self._derive_inputs(emissionval)
+        E = np.ascontiguousarray(E, np.float32)
+        _lib.check(_lib.lib().daisy_solver_set_emission(self._s, _lib.fptr(E)), "solver_set_emission")
+        self.emission, self.emission_value = E, emissionval
+
+    def set_materials(self):
+        """Re-derive M (and the material ids) from ``mesh.materials`` after a material changed; takes effect at the next pass."""
+        _, M = self._derive_inputs(self.emission_value)
+        M = np.ascontiguousarray(M, np.float32)
+        mat = np.ascontiguousarray(self.mesh_.materialIndexPerTriangle, np.int32)
+        _lib.check(_lib.lib().daisy_solver_set_materials(self._s, _lib.fptr(M), M.shape[0], _lib.iptr(mat)), "solver_set_materials")
+
+    def after_mesh_edit(self, mesh, previous, B_before, converge: bool = True):
+        """Follow ``optixP.replaceMesh(mesh, previous)`` + ``updateRadiosityMatrix()``: a new solver on the context's current
+        matrix (no rebuild, no reload), restarted from ``B_before`` (the B read before the edit) remapped by
+        :func:`remap_bands`; then converged unless ``converge=False``.  Returns the passes of the new solve."""
+        self.close()
+        self.mesh_, self.numpatches = mesh, mesh.numtriangles
+        E, M = self._derive_inputs(self.emission_value)
+        self._create_solver(E, M)
+        self.restart(remap_bands(B_before, previous, self.emission))
+        return self.converge_lightning() if converge else self.numpasses
+
     def _after_update(self):
         pass
 
@@ -716,6 +819,9 @@ class SpectralLightning(Lightning):
         E, M = _mat.spectral_inputs(mesh.materials, mesh.materialIndexPerTriangle, emissionval)  # :263-292
         self._cache = None
         self._init(mesh, optixP, E, M, cuda_enabled, matfile, converge)
+
+    def _derive_inputs(self, emissionval):
+        return _mat.spectral_inputs(self.mesh_.materials, self.mesh_.materialIndexPerTriangle, emissionval)
 
     def _after_update(self):
         self._cache = None
@@ -746,8 +852,12 @@ class RGBLightning(Lightning):
 
     def __init__(self, mesh, optixP, emissionval, cuda_enabled=False, matfile=None, converge=True):
         self.numsamples = 3
+        self.emission_value = emissionval
         E, M = _mat.rgb_inputs(mesh.materials, mesh.materialIndexPerTriangle, emissionval)  # :359-382
         self._init(mesh, optixP, E, M, cuda_enabled, matfile, converge)
+
+    def _derive_inputs(self, emissionval):
+        return _mat.rgb_inputs(self.mesh_.materials, self.mesh_.materialIndexPerTriangle, emissionval)
 
     def get_color_of_patch(self, index):
         return self.lightningvalues[:, index].copy()
@@ -760,8 +870,12 @@ class BWLightning(Lightning):
 
     def __init__(self, mesh, optixP, emissionval, matfile=None, converge=True):
         self.numsamples = 1
+        self.emission_value = emissionval
         E, M = _mat.bw_inputs(mesh.materials, mesh.materialIndexPerTriangle, emissionval)  # :434-442
         self._init(mesh, optixP, E, M, False, matfile, converge)
+
+    def _derive_inputs(self, emissionval):
+        return _mat.bw_inputs(self.mesh_.materials, self.mesh_.materialIndexPerTriangle, emissionval)
 
     def get_color_of_patch(self, index):
         v = self.lightningvalues[0, index]

@@ -385,6 +385,8 @@ int dz_solver_get_buffers(daisy_solver *s, float **res0, float **res1, unsigned 
 int dz_solver_set_peer_pointers(daisy_solver *s, float *const *res0, float *const *res1, unsigned long long *const *flags, int nranks); // gather.cu
 // converge with the stop rule on the device over n solvers issued from one thread (one GPU, or a group's devices)   // gather.cu
 int dz_converge_device(daisy_solver *const *ss, int n, double threshold, int per_band, int max_passes);
+// the restart pass without reading its band sums back (a group launches it on every device before any waits)   // gather.cu
+int dz_solver_restart_launch(daisy_solver *s, const float *B0_local);
 // upd != null: only the pairs the update can reach are traced and stored (ctx->upd_tiles, upd_classify_ms report it)
 int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mrow0, int mrow1, bool write_F,
                          const DzUpdate *upd = nullptr);                                                    // formfactor.cu

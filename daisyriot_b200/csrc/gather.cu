@@ -39,7 +39,8 @@ struct daisy_solver {
     daisy_ctx *ctx = nullptr;
     uint64_t mesh_version = 0; // the context's mesh_version at create: the mesh N, the row blocks and mat_idx belong to
     int K = 0, Kp = 0; // bands requested / bands the kernel is instantiated for
-    int nmat = 0;
+    int nmat = 0, nmat_cap = 0; // materials in use / material matrices d_M has room for (daisy_solver_set_materials)
+    bool abs_sums = false;      // restart mode: the passes total |r| (from daisy_solver_restart to the next reset / write)
     int N = 0, n = 0, G = 1, rank = 0, nloc = 0, row0 = 0;
     int64_t bstride = 0;   // floats per exchange block
     int64_t sums_off = 0;  // float offset of the K doubles inside a block
@@ -376,6 +377,10 @@ struct FusedEpi {
     int G;
     unsigned long long wait_seq;     // 0: nothing to wait for
     unsigned long long timeout_ns;
+    // restart pass (read only by the ABS instantiation): the pass reads B_old, and the epilogue forms B_new = y + E and
+    // r = B_new - B_old from this rank's emission block instead of B += y
+    int restart;
+    const float *E_block;
 };
 
 // acquire flag[g] >= wait_seq: rank g's block of the previous pass has landed here and rank g has finished reading the buffer
@@ -482,7 +487,9 @@ __host__ __device__ __forceinline__ bool next_piece(const GatherParams &P, int c
     return true;
 }
 
-template <int K>
+// ABS (restart mode, DESIGN 3.3b): the band sums total |r| instead of r, and E.restart selects the restart epilogue.  A template
+// parameter rather than a flag, so that the kernel of an ordinary pass is the one it always was.
+template <int K, bool ABS = false>
 __global__ void __launch_bounds__((TmaCfg<K>::NCW + 3) * 32, 1)
 k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __grid_constant__ CUtensorMap tmRes, const __grid_constant__ FusedEpi E) {
     constexpr int NST = tma_nstage<K>();
@@ -618,16 +625,41 @@ k_gather_tma(GatherParams P, const __grid_constant__ CUtensorMap tmF, const __gr
 #pragma unroll
                         for (int j = 0; j < K; j++) v = fmaf(__ldg(Mp + j * K + k), b[j], v);
                         y[k] = v;
-                        loc[k] = (double)v;
+                        if constexpr (!ABS) loc[k] = (double)v;
                     }
+                    if constexpr (ABS) {
+                        // y = M (F B_old): B_new = y + E, r = B_new - B_old (restart pass); otherwise B += r, r = y
 #pragma unroll
-                    for (int k = 0; k < K; k++) {
-                        if (E.npeers > 0) {
-                            for (int g = 0; g < E.npeers; g++) E.peer_out[g][(size_t)k * P.n + row] = y[k]; // NVLink stores into every rank's buffer
-                        } else {
-                            E.res_out_block[(size_t)k * P.n + row] = y[k];                   // residualvector[j][i] = result[j]
+                        for (int k = 0; k < K; k++) {
+                            float bn;
+                            if (E.restart) {
+                                bn = __fadd_rn(y[k], __ldg(E.E_block + (size_t)k * P.n + row));
+                                y[k] = __fsub_rn(bn, Bv[k]);
+                            } else {
+                                bn = __fadd_rn(Bv[k], y[k]);
+                            }
+                            Bv[k] = bn;
+                            loc[k] = fabs((double)y[k]);
                         }
-                        E.B[(size_t)k * P.n + row] = Bv[k] + y[k];                           // lightningvalues += residual   :221-223
+#pragma unroll
+                        for (int k = 0; k < K; k++) {
+                            if (E.npeers > 0) {
+                                for (int g = 0; g < E.npeers; g++) E.peer_out[g][(size_t)k * P.n + row] = y[k];
+                            } else {
+                                E.res_out_block[(size_t)k * P.n + row] = y[k];
+                            }
+                            E.B[(size_t)k * P.n + row] = Bv[k];
+                        }
+                    } else {
+#pragma unroll
+                        for (int k = 0; k < K; k++) {
+                            if (E.npeers > 0) {
+                                for (int g = 0; g < E.npeers; g++) E.peer_out[g][(size_t)k * P.n + row] = y[k]; // NVLink stores into every rank's buffer
+                            } else {
+                                E.res_out_block[(size_t)k * P.n + row] = y[k];                   // residualvector[j][i] = result[j]
+                            }
+                            E.B[(size_t)k * P.n + row] = Bv[k] + y[k];                           // lightningvalues += residual   :221-223
+                        }
                     }
                     if (E.npeers > 0) __threadfence_system(); else __threadfence();
                 }
@@ -812,9 +844,12 @@ struct EpiParams {
     unsigned long long seq;
     const unsigned long long *abort_marker; // flag word 16 of this rank (null: single GPU)
     unsigned int *stop_state;               // device converge: {stopped, passes} (the streaming kernel decided), else null
+    int restart;                            // restart pass (ABS instantiation only): B_new = y + E_block, r = B_new - B_old
+    const float *E_block;
 };
 
-template <int K>
+// ABS: restart mode, band sums of |r| (see k_gather_tma)
+template <int K, bool ABS = false>
 __global__ void __launch_bounds__(256) k_gather_epilogue(EpiParams P) {
     __shared__ double s_sum[8][K];
     __shared__ bool s_last;
@@ -839,6 +874,24 @@ __global__ void __launch_bounds__(256) k_gather_epilogue(EpiParams P) {
             float y = 0.0f;
 #pragma unroll
             for (int j = 0; j < K; j++) y = fmaf(Mp[j * K + k], b[j], y);
+            if constexpr (ABS) {
+                const float bo = P.B[(size_t)k * P.n + row];
+                float bn;
+                if (P.restart) {
+                    bn = __fadd_rn(y, P.E_block[(size_t)k * P.n + row]);
+                    y = __fsub_rn(bn, bo);
+                } else {
+                    bn = __fadd_rn(bo, y);
+                }
+                if (P.npeers > 0) {
+                    for (int g = 0; g < P.npeers; g++) P.peer_out[g][(size_t)k * P.n + row] = y;
+                } else {
+                    P.res_out_block[(size_t)k * P.n + row] = y;
+                }
+                P.B[(size_t)k * P.n + row] = bn;
+                loc[k] += fabs((double)y);
+                continue;
+            }
             if (P.npeers > 0) {
                 for (int g = 0; g < P.npeers; g++) P.peer_out[g][(size_t)k * P.n + row] = y; // NVLink stores into every rank's buffer
             } else {
@@ -935,8 +988,9 @@ static int launch_partial(daisy_solver *s, const GatherParams &P) {
 // wait_seq != 0 (fused exchange): the blocks of pass wait_seq must have arrived before the residual is read.  The fused TMA
 // kernel waits by itself, block by block; the other kernels get a k_wait_flags launch in front.
 // stop != null: a pass of a device converge (state, rule and threshold set by the caller; the tails are filled in here)
+// restart: the restart pass (daisy_solver_restart); s->abs_sums selects the epilogues that total |r|
 template <int K>
-static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const DevStop *stop) {
+static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const DevStop *stop, bool restart) {
     daisy_ctx *c = s->ctx;
     if (wait_seq != 0ull && !s->fused_epi) {
         k_wait_flags<<<1, 32, 0, c->stream>>>(s->d_flags, s->G, wait_seq, s->timeout_ns, s->d_abort_host, stop ? stop->state : nullptr);
@@ -977,10 +1031,13 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
     } else if (s->use_tma) {
         constexpr int NST = tma_nstage<K>();
         size_t smem = (size_t)NST * tma_stage_bytes<K>() + 2 * NST * sizeof(uint64_t) + tma_epi_bytes<K>();
-        static bool attr_done[64] = { false }; // per device
-        if (!attr_done[c->device & 63]) {
-            DZ_CUDA(cudaFuncSetAttribute(k_gather_tma<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            attr_done[c->device & 63] = true;
+        // restart mode runs the ABS instantiation; only the fused epilogue reads it (otherwise the epilogue warps return at once)
+        const bool abs_kernel = s->abs_sums && s->fused_epi;
+        auto kern = abs_kernel ? k_gather_tma<K, true> : k_gather_tma<K, false>;
+        static bool attr_done[2][64] = { { false } }; // per instantiation and device
+        if (!attr_done[abs_kernel][c->device & 63]) {
+            DZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            attr_done[abs_kernel][c->device & 63] = true;
         }
         P.nrb = s->nrb_tma; // (nloc + tma_rows<K>() - 1) / tma_rows<K>(), and 1 for a rank without rows (plan())
         P.sk = s->fused_epi ? 1 : 0; P.sk_S = s->sk_S; P.sk_L = s->sk_L; P.sk_total = s->sk_total;
@@ -997,6 +1054,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
             F.res_out_block = next; F.block_sums = reinterpret_cast<double *>(next + s->sums_off);
             F.seq = s->seq; F.flags = s->d_flags; F.host_abort = s->d_abort_host; F.G = s->G;
             F.wait_seq = wait_seq; F.timeout_ns = s->timeout_ns;
+            F.restart = restart ? 1 : 0; F.E_block = s->d_E + (size_t)s->rank * s->bstride;
             if (s->fused) {
                 F.npeers = s->G;
                 for (int g = 0; g < s->G; g++) {
@@ -1019,7 +1077,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
             at[0].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = at;
             cfg.numAttrs = (s->fused_epi && (s->chained || stop) && s->G == 1) ? 1 : 0;
-            DZ_CUDA(cudaLaunchKernelEx(&cfg, k_gather_tma<K>, P, s->tmF, s->tmRes[s->cur], F));
+            DZ_CUDA(cudaLaunchKernelEx(&cfg, kern, P, s->tmF, s->tmRes[s->cur], F));
         }
         DZ_CUDA(cudaGetLastError());
         if (s->fused_epi) return DAISY_OK; // the whole pass was that one launch
@@ -1037,6 +1095,7 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
     E.cta_sums = s->d_cta_sums; E.block_sums = reinterpret_cast<double *>(next + s->sums_off); E.done = s->d_done;
     E.npeers = 0; E.seq = s->seq; E.abort_marker = s->fused ? s->d_flags + 16 : nullptr;
     E.stop_state = P.stop.state;
+    E.restart = restart ? 1 : 0; E.E_block = s->d_E + (size_t)s->rank * s->bstride;
     if (s->fused) {
         E.npeers = s->G;
         for (int g = 0; g < s->G; g++) {
@@ -1049,25 +1108,26 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
     int egrid = (s->nloc + 255) / 256;
     if (egrid > 148) egrid = 148;
     if (egrid < 1) egrid = 1;
-    k_gather_epilogue<K><<<egrid, 256, 0, c->stream>>>(E);
+    if (s->abs_sums) k_gather_epilogue<K, true><<<egrid, 256, 0, c->stream>>>(E);
+    else k_gather_epilogue<K, false><<<egrid, 256, 0, c->stream>>>(E);
     DZ_CUDA(cudaGetLastError());
     return DAISY_OK;
 }
 
 static int scan_and_plan(daisy_solver *s);
 
-static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull, const DevStop *stop = nullptr) {
+static int launch_pass(daisy_solver *s, unsigned long long wait_seq = 0ull, const DevStop *stop = nullptr, bool restart = false) {
     if (s->skip && s->scanned_version != s->ctx->F_version) { // F was written since the last scan (a host integer compare per pass)
         int rc = scan_and_plan(s);
         if (rc) return rc;
     }
     switch (s->Kp) {
-    case 1: return launch_pass_K<1>(s, wait_seq, stop);
-    case 3: return launch_pass_K<3>(s, wait_seq, stop);
-    case 9: return launch_pass_K<9>(s, wait_seq, stop);
-    case 16: return launch_pass_K<16>(s, wait_seq, stop);
-    case 32: return launch_pass_K<32>(s, wait_seq, stop);
-    case 64: return launch_pass_K<64>(s, wait_seq, stop);
+    case 1: return launch_pass_K<1>(s, wait_seq, stop, restart);
+    case 3: return launch_pass_K<3>(s, wait_seq, stop, restart);
+    case 9: return launch_pass_K<9>(s, wait_seq, stop, restart);
+    case 16: return launch_pass_K<16>(s, wait_seq, stop, restart);
+    case 32: return launch_pass_K<32>(s, wait_seq, stop, restart);
+    case 64: return launch_pass_K<64>(s, wait_seq, stop, restart);
     }
     daisy_set_error("unsupported padded band count %d", s->Kp);
     return DAISY_E_INVALID;
@@ -1355,6 +1415,14 @@ static double host_sum(const float *x, size_t n) {
     return ((a[0] + a[1]) + (a[2] + a[3])) + ((a[4] + a[5]) + (a[6] + a[7]));
 }
 
+// M (nmat x K x K column-major) padded to Kp x Kp: the extra bands are inert (zero rows and columns)
+static void pad_materials(const daisy_solver *s, const float *M, int nmat, std::vector<float> &Mp) {
+    Mp.assign((size_t)nmat * s->Kp * s->Kp, 0.0f);
+    for (int m = 0; m < nmat; m++)
+        for (int j = 0; j < s->K; j++)
+            for (int i = 0; i < s->K; i++) Mp[((size_t)m * s->Kp + j) * s->Kp + i] = M[((size_t)m * s->K + j) * s->K + i];
+}
+
 static int compute_sums_from_host(daisy_solver *s, const float *res /* K x N */) {
     // band sums of a residual supplied by the host (reset / write): same quantity the kernels total on device
     s->sums.assign(s->K, 0.0);
@@ -1379,7 +1447,7 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
         DZ_REQUIRE(mat_idx[p] >= 0 && mat_idx[p] < nmat, DAISY_E_INVALID, "daisy_solver_create: material index out of range");
     DZ_CUDA(cudaSetDevice(ctx->device));
     daisy_solver *s = new daisy_solver();
-    s->ctx = ctx; s->mesh_version = ctx->mesh_version; s->K = K; s->Kp = padded_K(K); s->nmat = nmat;
+    s->ctx = ctx; s->mesh_version = ctx->mesh_version; s->K = K; s->Kp = padded_K(K); s->nmat = s->nmat_cap = nmat;
     s->N = ctx->N; s->n = ctx->rows_per_rank; s->G = ctx->nranks; s->rank = ctx->rank;
     s->row0 = ctx->row0; s->nloc = ctx->row1 - ctx->row0;
     int64_t body = (int64_t)s->Kp * s->n;
@@ -1428,11 +1496,8 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
         std::vector<float> ex;
         to_exchange(s, E, ex);
         SC(cudaMemcpy(s->d_E, ex.data(), exb, cudaMemcpyHostToDevice));
-        // M padded to Kp x Kp (extra bands are inert: zero rows/columns)
-        std::vector<float> Mp((size_t)nmat * s->Kp * s->Kp, 0.0f);
-        for (int m = 0; m < nmat; m++)
-            for (int j = 0; j < K; j++)
-                for (int i = 0; i < K; i++) Mp[((size_t)m * s->Kp + j) * s->Kp + i] = M[((size_t)m * K + j) * K + i];
+        std::vector<float> Mp;
+        pad_materials(s, M, nmat, Mp);
         SC(cudaMemcpy(s->d_M, Mp.data(), sizeof(float) * Mp.size(), cudaMemcpyHostToDevice));
         if (s->nloc > 0) SC(cudaMemcpy(s->d_mat, mat_idx + s->row0, sizeof(int) * (size_t)s->nloc, cudaMemcpyHostToDevice));
     }
@@ -1476,8 +1541,9 @@ extern "C" int daisy_solver_reset(daisy_solver *s) {
     DZ_CUDA(cudaMemcpyAsync(s->d_B, s->d_E + (size_t)s->rank * s->bstride, sizeof(float) * (size_t)s->Kp * s->n, cudaMemcpyDeviceToDevice, st));
     DZ_CUDA(cudaStreamSynchronize(st));
     s->numpasses = 0;
-    s->sums = s->e_sums; // band sums of E, totalled once at create
+    s->sums = s->e_sums; // band sums of E (totalled at create and by daisy_solver_set_emission)
     s->sums_valid = true;
+    s->abs_sums = false;
     return DAISY_OK;
 }
 
@@ -1677,6 +1743,7 @@ extern "C" int daisy_solver_write_slices(daisy_solver *s, const float *B_local, 
     DZ_CUDA(cudaGetLastError());
     s->cur = nxt;
     s->sums_valid = false;
+    s->abs_sums = false;
     return DAISY_OK;
 }
 
@@ -1902,6 +1969,7 @@ extern "C" int daisy_solver_write(daisy_solver *s, const float *B, const float *
     compute_sums_from_host(s, residual); // while the copies are in flight
     DZ_CUDA(cudaStreamSynchronize(st));
     s->sums_valid = true;
+    s->abs_sums = false;
     return DAISY_OK;
 }
 
@@ -1927,6 +1995,107 @@ extern "C" int daisy_solver_write_partitioned(daisy_solver *s, const float *B_lo
     compute_sums_from_host(s, residual_full); // while the copies are in flight
     DZ_CUDA(cudaStreamSynchronize(st));
     s->sums_valid = true;
+    s->abs_sums = false;
+    return DAISY_OK;
+}
+
+// ---- warm restart (DESIGN 3.3b) ----------------------------------------------------------------------------------------
+// The restart pass streams F once with B_old as the input vector: y = M (F B_old) with the arithmetic of an ordinary pass,
+// B_new = y + E, r = B_new - B_old.  B_old (this rank's K x nloc rows, or the solver's own B when B0_local is NULL) goes into
+// d_B and, as the pass's input, into this rank's block of the buffer the pass reads -- with the fused exchange also into every
+// peer's copy of that buffer, published with flag[rank] the way daisy_solver_write_slices publishes a residual, so the pass's
+// own flag waits cover it.  From here on the solver is in restart mode: every pass totals |r|.
+int dz_solver_restart_launch(daisy_solver *s, const float *B0_local) {
+    DZ_SOLVER_CURRENT(s, "daisy_solver_restart");
+    DZ_REQUIRE(s->G == 1 || s->fused, DAISY_E_STATE,
+               "daisy_solver_restart: a partitioned solver needs the fused exchange (daisy_solver_set_peers); a partition exchanged by the host cannot restart");
+    DZ_CUDA(cudaSetDevice(s->ctx->device));
+    if (s->fused && s->h_abort && *reinterpret_cast<volatile unsigned long long *>(s->h_abort) != 0ull) return abort_error(s);
+    cudaStream_t st = s->ctx->stream;
+    // fused exchange: every rank has finished the last pass, and with it every read of the buffer about to be overwritten
+    if (s->fused && s->seq > 0) {
+        k_wait_flags<<<1, 32, 0, st>>>(s->d_flags, s->G, s->seq, s->timeout_ns, s->d_abort_host);
+        DZ_CUDA(cudaGetLastError());
+    }
+    if (B0_local && s->nloc > 0) {
+        DZ_CUDA(cudaMemcpy2DAsync(s->d_B, sizeof(float) * s->n, B0_local, sizeof(float) * s->nloc, sizeof(float) * s->nloc, s->K, cudaMemcpyHostToDevice, st));
+        DZ_CUDA(cudaStreamSynchronize(st)); // B0_local is pageable host memory the caller may reuse at once
+    }
+    // the padded bands and the columns nloc..n-1 of d_B are zero (reset copies the zero-padded emission block; no pass writes them)
+    const int in = s->fused ? (s->cur ^ 1) : s->cur;
+    float *own = s->d_res[in] + (size_t)s->rank * s->bstride;
+    DZ_CUDA(cudaMemcpyAsync(own, s->d_B, sizeof(float) * (size_t)s->Kp * s->n, cudaMemcpyDeviceToDevice, st));
+    if (s->fused) {
+        for (int g = 0; g < s->G; g++) {
+            if (g == s->rank) continue;
+            DZ_CUDA(cudaMemcpyAsync(s->peer_res[in][g] + (size_t)s->rank * s->bstride, own, sizeof(float) * (size_t)s->Kp * s->n, cudaMemcpyDeviceToDevice, st));
+        }
+        s->seq++;
+        unsigned long long *f[16];
+        for (int g = 0; g < 16; g++) f[g] = (g < s->G) ? s->peer_flags[g] + s->rank : nullptr;
+        k_raise_flags<<<1, 32, 0, st>>>(s->G, s->seq, s->d_flags + 16, f[0], f[1], f[2], f[3], f[4], f[5], f[6], f[7], f[8], f[9], f[10], f[11], f[12],
+                                        f[13], f[14], f[15]);
+        DZ_CUDA(cudaGetLastError());
+        s->cur = in;
+    }
+    if (!s->chained) DZ_CUDA(cudaEventRecord(s->e0, st));
+    const unsigned long long wait_seq = s->fused ? s->seq : 0ull; // the B_old blocks just published
+    if (s->fused) s->seq++;
+    s->abs_sums = true;
+    int rc = launch_pass(s, wait_seq, nullptr, true);
+    if (rc) return rc;
+    if (!s->chained) DZ_CUDA(cudaEventRecord(s->e1, st));
+    s->events_recorded = !s->chained;
+    s->numpasses = 0; // the restart pass counts as the first pass of the new solve
+    return step_finish(s, nullptr);
+}
+
+extern "C" int daisy_solver_restart(daisy_solver *s, const float *B0) {
+    DZ_REQUIRE(s, DAISY_E_INVALID, "daisy_solver_restart: null solver");
+    DzRange range_("daisy_solver_restart");
+    int rc = dz_solver_restart_launch(s, B0);
+    if (rc) return rc;
+    return fetch_sums(s); // the band sums of the restart pass: sum |r|
+}
+
+extern "C" int daisy_solver_set_emission(daisy_solver *s, const float *E) {
+    DZ_REQUIRE(s && E, DAISY_E_INVALID, "daisy_solver_set_emission: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_set_emission");
+    DZ_CUDA(cudaSetDevice(s->ctx->device));
+    cudaStream_t st = s->ctx->stream;
+    std::vector<float> ex;
+    to_exchange(s, E, ex);
+    DZ_CUDA(cudaStreamSynchronize(st)); // a restart pass enqueued earlier may still read the old emission
+    DZ_CUDA(cudaMemcpyAsync(s->d_E, ex.data(), sizeof(float) * ex.size(), cudaMemcpyHostToDevice, st));
+    std::vector<double> es((size_t)s->K);
+    for (int k = 0; k < s->K; k++) es[(size_t)k] = host_sum(E + (size_t)k * s->N, (size_t)s->N);
+    DZ_CUDA(cudaStreamSynchronize(st)); // `ex` is pageable host memory
+    s->e_sums = es;
+    return DAISY_OK;
+}
+
+extern "C" int daisy_solver_set_materials(daisy_solver *s, const float *M, int nmat, const int32_t *mat_idx) {
+    DZ_REQUIRE(s && M && mat_idx, DAISY_E_INVALID, "daisy_solver_set_materials: null argument");
+    DZ_SOLVER_CURRENT(s, "daisy_solver_set_materials");
+    DZ_REQUIRE(nmat >= 1, DAISY_E_INVALID, "daisy_solver_set_materials: need at least one material");
+    for (int p = 0; p < s->N; p++)
+        DZ_REQUIRE(mat_idx[p] >= 0 && mat_idx[p] < nmat, DAISY_E_INVALID, "daisy_solver_set_materials: material index out of range");
+    DZ_CUDA(cudaSetDevice(s->ctx->device));
+    cudaStream_t st = s->ctx->stream;
+    DZ_CUDA(cudaStreamSynchronize(st)); // no pass in flight reads d_M or d_mat below
+    if (nmat > s->nmat_cap) {
+        float *d = nullptr;
+        DZ_CUDA(cudaMalloc(&d, sizeof(float) * (size_t)nmat * s->Kp * s->Kp)); // on failure the solver keeps its old matrices
+        cudaFree(s->d_M);
+        s->d_M = d;
+        s->nmat_cap = nmat;
+    }
+    std::vector<float> Mp;
+    pad_materials(s, M, nmat, Mp);
+    DZ_CUDA(cudaMemcpyAsync(s->d_M, Mp.data(), sizeof(float) * Mp.size(), cudaMemcpyHostToDevice, st));
+    if (s->nloc > 0) DZ_CUDA(cudaMemcpyAsync(s->d_mat, mat_idx + s->row0, sizeof(int) * (size_t)s->nloc, cudaMemcpyHostToDevice, st));
+    DZ_CUDA(cudaStreamSynchronize(st)); // `Mp` is pageable host memory
+    s->nmat = nmat;
     return DAISY_OK;
 }
 

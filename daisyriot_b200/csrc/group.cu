@@ -377,6 +377,49 @@ extern "C" int daisy_group_solver_converge_device(daisy_group_solver *gs, double
     return rc;
 }
 
+// daisy_solver_restart over every device: B0 (K x N whole scene, or NULL for the current B) is split into the devices' rows, the
+// restart pass is launched on every device before any device waits, and device 0 answers the band sums when they are asked for
+extern "C" int daisy_group_solver_restart(daisy_group_solver *gs, const float *B0) {
+    DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_restart: null solver");
+    DZ_REQUIRE(gs->mesh_version == gs->g->ctx[0]->mesh_version, DAISY_E_STATE,
+               "daisy_group_solver_restart: the group's mesh was replaced after this solver was created; create a new solver");
+    daisy_group *g = gs->g;
+    if (g->ndev == 1) return daisy_solver_restart(gs->s[0], B0);
+    nvtxRangePushA("daisy_group_solver_restart");
+    const int N = g->N, K = gs->K;
+    std::vector<float> b;
+    int rc = DAISY_OK;
+    for (int i = 0; i < g->ndev && !rc; i++) {
+        daisy_ctx *c = g->ctx[(size_t)i];
+        const int nloc = c->row1 - c->row0;
+        if (B0) {
+            b.assign((size_t)K * (nloc > 0 ? nloc : 1), 0.f);
+            for (int k = 0; k < K && nloc > 0; k++) memcpy(b.data() + (size_t)k * nloc, B0 + (size_t)k * N + c->row0, sizeof(float) * (size_t)nloc);
+        }
+        rc = dz_solver_restart_launch(gs->s[(size_t)i], B0 ? b.data() : nullptr);
+    }
+    nvtxRangePop();
+    return rc;
+}
+
+extern "C" int daisy_group_solver_set_emission(daisy_group_solver *gs, const float *E) {
+    DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_set_emission: null solver");
+    for (daisy_solver *s : gs->s) { // the same input on every device: the first one refuses invalid input before any changes
+        int rc = daisy_solver_set_emission(s, E);
+        if (rc) return rc;
+    }
+    return DAISY_OK;
+}
+
+extern "C" int daisy_group_solver_set_materials(daisy_group_solver *gs, const float *M, int nmat, const int32_t *mat_idx) {
+    DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_set_materials: null solver");
+    for (daisy_solver *s : gs->s) {
+        int rc = daisy_solver_set_materials(s, M, nmat, mat_idx);
+        if (rc) return rc;
+    }
+    return DAISY_OK;
+}
+
 // lightningvalues and residualvector of the whole scene, K x N band-major, assembled from the devices' row blocks
 extern "C" int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *residual) {
     DZ_REQUIRE(gs, DAISY_E_INVALID, "daisy_group_solver_read: null solver");

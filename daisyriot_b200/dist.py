@@ -187,6 +187,30 @@ class PartitionedSolver:
             passes += 1
         return passes
 
+    def restart(self, B0_local=None):
+        """``daisy_solver_restart`` on this rank (every rank calls it): ``B0_local`` holds this rank's K x (row1 - row0) rows
+        of the B to restart from, ``None`` restarts from the current B.  Needs the fused exchange with more than one rank
+        (a partition exchanged through NCCL gets DAISY_E_STATE).  Returns the band sums (sum of |residual|)."""
+        b = None
+        if B0_local is not None:
+            r0, r1 = self.p.row_range
+            b = np.ascontiguousarray(B0_local, np.float32)
+            if b.shape != (self.K, r1 - r0):
+                raise ValueError("restart: B0_local must be K x (row1 - row0), got %s" % (b.shape,))
+        _lib.check(_lib.lib().daisy_solver_restart(self._s, None if b is None else _lib.fptr(b)), "solver_restart")
+        return self.band_sums()
+
+    def set_emission(self, E):
+        """The whole scene's K x N emission (every rank passes the same); used at the next reset or restart."""
+        E = np.ascontiguousarray(E, np.float32)
+        _lib.check(_lib.lib().daisy_solver_set_emission(self._s, _lib.fptr(E)), "solver_set_emission")
+
+    def set_materials(self, M, mat_idx):
+        """nmat x K x K material matrices and the N material ids of the whole scene; used from the next pass."""
+        M = np.ascontiguousarray(M, np.float32)
+        mat = np.ascontiguousarray(mat_idx, np.int32)
+        _lib.check(_lib.lib().daisy_solver_set_materials(self._s, _lib.fptr(M), M.shape[0], _lib.iptr(mat)), "solver_set_materials")
+
     def read_local(self):
         r0, r1 = self.p.row_range
         B = np.empty((self.K, r1 - r0), np.float32)

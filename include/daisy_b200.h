@@ -225,6 +225,25 @@ int daisy_solver_band_sums(daisy_solver *s, double *band_sums);
 int daisy_solver_read(daisy_solver *s, float *B, float *residual);
 /* overwrite the current residual and B from host (K x N band-major) -- used by the end-to-end benchmark */
 int daisy_solver_write(daisy_solver *s, const float *B, const float *residual);
+/* Warm restart (after the matrix, the emission or the materials changed): one pass that starts the iteration from B_old instead
+ * of from E.  B_old = B0 (K x N band-major; a partitioned solver: this rank's K x (row1-row0) rows, as in write_slices), or the
+ * solver's current B when B0 == NULL.  The pass streams F once with B_old as its input and, per row and band, forms
+ *   y = M_p (F B_old)   (the arithmetic of an ordinary pass),   B_new = y + E,   r = B_new - B_old   (FP32, round to nearest)
+ * and stores B = B_new, residual = r; the ordinary passes then continue (r <- M F r, B += r) towards the fixed point
+ * B* = E + M F B* of a cold solve.  numpasses becomes 1.  r carries FP32 cancellation noise of about ulp(B) per entry, which
+ * the passes contract like any residual.
+ * From the restart to the next daisy_solver_reset / _write / _write_slices / _write_partitioned the solver is in restart mode:
+ * every band sum (step, band_sums, converge, converge_device) is sum_p |r| -- the residual of a warm start has both signs, and
+ * the reference's criteria applied to signed sums could stop while B is still off.  For a cold solve (E, M, F >= 0) that is the
+ * same number.  Single GPU, or a partitioned solver with the fused exchange (every rank calls it); DAISY_E_STATE for a
+ * partition exchanged by the host. */
+int daisy_solver_restart(daisy_solver *s, const float *B0);
+/* replace the emission (K x N, whole scene) or the material matrices (nmat x K x K; nmat may grow) and the N material ids: the
+ * solver-side set_sampled_emission / set_reflectionvalues / set_reflectionmatrix (Lightning.h:263-292).  B and the residual
+ * are untouched; the emission takes effect at the next reset or restart, the materials at the next pass.  Invalid input:
+ * DAISY_E_INVALID and the solver unchanged. */
+int daisy_solver_set_emission(daisy_solver *s, const float *E);
+int daisy_solver_set_materials(daisy_solver *s, const float *M, int nmat, const int32_t *mat_idx);
 
 /* ---- multi-GPU plumbing (one process per GPU; the host does the exchange with NCCL / torch.distributed) -----
  * With daisy_ctx_set_partition(rank, nranks) the residual lives in an exchange buffer of `nranks` equal blocks,
@@ -325,6 +344,10 @@ int daisy_group_solver_numpasses(daisy_group_solver *gs);
 int daisy_group_solver_band_sums(daisy_group_solver *gs, double *band_sums);
 int daisy_group_solver_read(daisy_group_solver *gs, float *B, float *residual);   /* K x N band-major, whole scene */
 int daisy_group_solver_write(daisy_group_solver *gs, const float *B, const float *residual);
+/* daisy_solver_restart over every device (B0: K x N whole scene, or NULL), and the two setters on every device */
+int daisy_group_solver_restart(daisy_group_solver *gs, const float *B0);
+int daisy_group_solver_set_emission(daisy_group_solver *gs, const float *E);
+int daisy_group_solver_set_materials(daisy_group_solver *gs, const float *M, int nmat, const int32_t *mat_idx);
 
 #ifdef __cplusplus
 }

@@ -37,6 +37,18 @@ public:
         numpasses = 0;
         fetch();
     }
+    // warm restart after the matrix (updateGeometry + updateRadiosityMatrix), the emission or the materials changed: one pass
+    // from the current lightningvalues instead of from the emission (daisy_group_solver_restart); numpasses becomes 1
+    void restart() {
+        check(daisy_group_solver_restart(solver, nullptr));
+        numpasses = daisy_group_solver_numpasses(solver);
+        fetch();
+    }
+    // restart + converge_lightning: the stop rule then looks at the sum of |residual| (a warm residual has both signs)
+    void reconverge_lightning() {
+        check(daisy_group_solver_restart(solver, nullptr));
+        converge_lightning();
+    }
     virtual ~Lightning() { daisy_group_solver_destroy(solver); }
     int numpasses = 0;
     std::vector<std::vector<float>> lightningvalues, residualvector; // K x N, band-major (Lightning.h:107-109)

@@ -103,6 +103,13 @@ int main(int argc, char **argv) {
         l->reset();
         l->converge_lightning_on_device();
     }
+    // DAISY_DEMO_RECONVERGE=1: one warm restart from the converged values (reconverge_lightning); RESTART reports its passes
+    if (getenv("DAISY_DEMO_RECONVERGE")) {
+        l->reconverge_lightning();
+        double sr = 0;
+        for (auto &band : l->lightningvalues) for (float v : band) sr += v;
+        printf("RESTART passes=%d sumB=%.9e\n", l->numpasses, sr);
+    }
     const double solve_s = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
     double sum = 0;
     for (auto &band : l->lightningvalues) for (float v : band) sum += v;
