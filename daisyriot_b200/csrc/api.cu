@@ -325,7 +325,7 @@ static void free_mesh_arrays(MeshArrays &m) {
     cudaFree(m.vertices); cudaFree(m.normals); cudaFree(m.tri); cudaFree(m.geom); cudaFree(m.plane); cudaFree(m.nbr); cudaFree(m.vadj_off); cudaFree(m.vadj);
     m = MeshArrays();
 }
-static int alloc_mesh_arrays(const int32_t *tri_idx, int nv, int nn, int ntri, MeshArrays &m) {
+static int alloc_mesh_arrays(const int32_t *tri_idx, int nv, int nn, int ntri, cudaStream_t st, MeshArrays &m) {
     m = MeshArrays();
 #define CC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { daisy_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); free_mesh_arrays(m); return DAISY_E_CUDA; } } while (0)
     CC(cudaMalloc(&m.vertices, sizeof(float) * 3 * (size_t)(nv > 0 ? nv : 1)));
@@ -334,7 +334,7 @@ static int alloc_mesh_arrays(const int32_t *tri_idx, int nv, int nn, int ntri, M
     CC(cudaMalloc(&m.geom, sizeof(PatchGeom) * (size_t)(ntri > 0 ? ntri : 1)));
     CC(cudaMalloc(&m.plane, sizeof(float4) * (size_t)(ntri > 0 ? ntri : 1)));
     CC(cudaMalloc(&m.nbr, sizeof(int) * 32 * (size_t)(ntri > 0 ? ntri : 1)));
-    if (ntri) CC(cudaMemcpy(m.tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice));
+    if (ntri) CC(cudaMemcpyAsync(m.tri, tri_idx, sizeof(int) * 6 * (size_t)ntri, cudaMemcpyHostToDevice, st));
     {
         // MeshS::trianglesPerVertex (MeshS.cpp:107-109) as CSR, lists in ascending triangle order: Drawer::interpolate sums
         // the patch colours of a vertex in exactly that order
@@ -347,8 +347,9 @@ static int alloc_mesh_arrays(const int32_t *tri_idx, int nv, int nn, int ntri, M
             for (int k = 0; k < 3; k++) adj[(size_t)fill[tri_idx[6 * (size_t)i + k]]++] = i;
         CC(cudaMalloc(&m.vadj_off, sizeof(int) * off.size()));
         CC(cudaMalloc(&m.vadj, sizeof(int) * adj.size()));
-        CC(cudaMemcpy(m.vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice));
-        CC(cudaMemcpy(m.vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice));
+        CC(cudaMemcpyAsync(m.vadj_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice, st));
+        CC(cudaMemcpyAsync(m.vadj, adj.data(), sizeof(int) * adj.size(), cudaMemcpyHostToDevice, st));
+        CC(cudaStreamSynchronize(st)); // `off` and `adj` are pageable host memory
     }
 #undef CC
     return DAISY_OK;
@@ -384,7 +385,7 @@ extern "C" int daisy_ctx_create(const float *vertices, int nv, const float *norm
     cudaDeviceProp prop;
     DZ_CUDA(cudaGetDeviceProperties(&prop, device));
     MeshArrays m;
-    rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, m);
+    rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, 0, m); // a new context runs on the default stream until daisy_ctx_set_stream
     if (rc) return rc;
     daisy_ctx *c = new daisy_ctx();
     c->device = device;
@@ -427,10 +428,10 @@ static int build_geometry(daisy_ctx *c) {
     // round by far less than those margins.  When the coordinates round at more than 1/256 of 1e-4 x the extent (a scene
     // many times its own size away from the origin), neither is used: every plane id stays 0, so nothing is skipped.
     const bool far_from_origin = 1e-4f * ext < 256.0f * ulp;
-    if (nv) DZ_CUDA(cudaMemcpy(c->d_vertices, vertices, sizeof(float) * 3 * (size_t)nv, cudaMemcpyHostToDevice));
-    if (nn) DZ_CUDA(cudaMemcpy(c->d_normals, normals, sizeof(float) * 3 * (size_t)nn, cudaMemcpyHostToDevice));
+    if (nv) DZ_CUDA(cudaMemcpyAsync(c->d_vertices, vertices, sizeof(float) * 3 * (size_t)nv, cudaMemcpyHostToDevice, c->stream));
+    if (nn) DZ_CUDA(cudaMemcpyAsync(c->d_normals, normals, sizeof(float) * 3 * (size_t)nn, cudaMemcpyHostToDevice, c->stream));
+    std::vector<int> pid; // pageable host memory: lives until the stream synchronisation below
     {
-        std::vector<int> pid;
         if (far_from_origin) pid.assign((size_t)(ntri > 0 ? ntri : 1), 0);
         else assign_plane_ids(vertices, tri_idx, ntri, ext, pid);
         dz_free_faces(c);
@@ -438,7 +439,7 @@ static int build_geometry(daisy_ctx *c) {
         cudaFree(c->d_pid);
         c->d_pid = nullptr;
         DZ_CUDA(cudaMalloc(&c->d_pid, sizeof(int) * pid.size()));
-        DZ_CUDA(cudaMemcpy(c->d_pid, pid.data(), sizeof(int) * pid.size(), cudaMemcpyHostToDevice));
+        DZ_CUDA(cudaMemcpyAsync(c->d_pid, pid.data(), sizeof(int) * pid.size(), cudaMemcpyHostToDevice, c->stream));
     }
     int rc = dz_build_lbvh(c);
     if (!rc) rc = dz_precompute_geom(c);
@@ -493,7 +494,7 @@ extern "C" int daisy_ctx_row_range(daisy_ctx *ctx, int *row0, int *row1, int *ro
 extern "C" int daisy_ctx_set_stream(daisy_ctx *ctx, void *cuda_stream) {
     DZ_REQUIRE(ctx, DAISY_E_INVALID, "daisy_ctx_set_stream: null context");
     DZ_CUDA(cudaSetDevice(ctx->device));
-    DZ_CUDA(cudaDeviceSynchronize()); // work enqueued on the previous stream (context set-up) is complete before the new one is used
+    DZ_CUDA(cudaStreamSynchronize(ctx->stream)); // work enqueued on the previous stream is complete before the new one is used
     ctx->stream = (cudaStream_t)cuda_stream;
     return DAISY_OK;
 }
@@ -592,8 +593,6 @@ extern "C" int daisy_formfactors_build(daisy_ctx *ctx, int variant) {
     int rc = dz_ensure_F(ctx);
     if (rc) return rc;
     if (timing) { cudaStreamSynchronize(ctx->stream); fprintf(stderr, "daisy_formfactors_build: matrix allocation + zero fill %.3f s\n", std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count()); }
-    rc = dz_set_samples_const(ctx);
-    if (rc) return rc;
     const auto t1 = std::chrono::steady_clock::now();
     rc = dz_build_formfactors(ctx, variant, nullptr, 0, 0, true);
     if (rc) return rc;
@@ -618,8 +617,6 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
     DzRange range_("daisy_formfactors_update: dirty set, tile classification, partial k_ff_tiles");
     DZ_CUDA(cudaSetDevice(ctx->device));
     int rc = dz_ensure_F(ctx);
-    if (rc) return rc;
-    rc = dz_set_samples_const(ctx);
     if (rc) return rc;
     const int N = ctx->N;
     ctx->upd_classify_ms = 0.0;
@@ -701,10 +698,11 @@ extern "C" int daisy_formfactors_update(daisy_ctx *ctx, int variant) {
         if (e == cudaSuccess) e = cudaMalloc(&d_leaf, sizeof(float4) * (leaf.empty() ? 1 : leaf.size()));
         if (e == cudaSuccess) e = cudaMalloc(&d_cbox, sizeof(float4) * (cbox.empty() ? 1 : cbox.size()));
         if (e == cudaSuccess) e = cudaMalloc(&d_crange, sizeof(int2) * (crange.empty() ? 1 : crange.size()));
-        if (e == cudaSuccess) e = cudaMemcpy(d_changed, changed.data(), changed.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && !leaf.empty()) e = cudaMemcpy(d_leaf, leaf.data(), sizeof(float4) * leaf.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && !cbox.empty()) e = cudaMemcpy(d_cbox, cbox.data(), sizeof(float4) * cbox.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && !crange.empty()) e = cudaMemcpy(d_crange, crange.data(), sizeof(int2) * crange.size(), cudaMemcpyHostToDevice);
+        // (the host vectors outlive dz_build_formfactors, which ends in a stream synchronisation)
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d_changed, changed.data(), changed.size(), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess && !leaf.empty()) e = cudaMemcpyAsync(d_leaf, leaf.data(), sizeof(float4) * leaf.size(), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess && !cbox.empty()) e = cudaMemcpyAsync(d_cbox, cbox.data(), sizeof(float4) * cbox.size(), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess && !crange.empty()) e = cudaMemcpyAsync(d_crange, crange.data(), sizeof(int2) * crange.size(), cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess) {
             DzUpdate upd;
             upd.changed = d_changed; upd.leaf = d_leaf; upd.cbox = d_cbox; upd.crange = d_crange; upd.nclusters = (int)crange.size();
@@ -835,7 +833,7 @@ int dz_replace_mesh(daisy_ctx *const *ctx, int n, const float *vertices, int nv,
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream); // nothing enqueued may still read what is replaced
         if (e != cudaSuccess) return cuda_fail(e, "device");
         lay[(size_t)i] = row_layout(ntri, c->rank, c->nranks);
-        rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, arr[(size_t)i]);
+        rc = alloc_mesh_arrays(tri_idx, nv, nn, ntri, c->stream, arr[(size_t)i]);
         if (rc) { discard(); return rc; }
         if (!remap) continue;
         const RowLayout &l = lay[(size_t)i];
@@ -848,7 +846,7 @@ int dz_replace_mesh(daisy_ctx *const *ctx, int n, const float *vertices, int nv,
             return DAISY_E_NOMEM;
         }
         if (e == cudaSuccess) e = cudaMalloc(&d_prev[(size_t)i], sizeof(int) * (size_t)(ntri > 0 ? ntri : 1));
-        if (e == cudaSuccess && ntri) e = cudaMemcpy(d_prev[(size_t)i], previous, sizeof(int) * (size_t)ntri, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess && ntri) e = cudaMemcpyAsync(d_prev[(size_t)i], previous, sizeof(int) * (size_t)ntri, cudaMemcpyHostToDevice, c->stream);
         if (e != cudaSuccess) return cuda_fail(e, "allocation");
     }
     // (2) remap on every device, reading the old rows where they live (a group's devices through peer access)
@@ -995,9 +993,9 @@ extern "C" int daisy_formfactors_read_rows(daisy_ctx *ctx, int row0, int nrows, 
     DZ_REQUIRE(nrows >= 0 && row0 >= ctx->row0 && row0 + nrows <= ctx->row1, DAISY_E_INVALID, "daisy_formfactors_read_rows: rows outside this context's range");
     if (nrows == 0) return DAISY_OK;
     DZ_CUDA(cudaSetDevice(ctx->device));
+    DZ_CUDA(cudaMemcpy2DAsync(out, sizeof(float) * (size_t)ctx->N, ctx->d_F + (size_t)(row0 - ctx->row0) * ctx->ldF, sizeof(float) * (size_t)ctx->ldF,
+                              sizeof(float) * (size_t)ctx->N, (size_t)nrows, cudaMemcpyDeviceToHost, ctx->stream));
     DZ_CUDA(cudaStreamSynchronize(ctx->stream));
-    DZ_CUDA(cudaMemcpy2D(out, sizeof(float) * (size_t)ctx->N, ctx->d_F + (size_t)(row0 - ctx->row0) * ctx->ldF, sizeof(float) * (size_t)ctx->ldF,
-                         sizeof(float) * (size_t)ctx->N, (size_t)nrows, cudaMemcpyDeviceToHost));
     return DAISY_OK;
 }
 
@@ -1064,8 +1062,7 @@ extern "C" int daisy_visibility_masks(daisy_ctx *ctx, int variant, int row0, int
     if (nrows == 0 || ctx->N == 0) return DAISY_OK;
     DzRange range_("daisy_visibility_masks");
     DZ_CUDA(cudaSetDevice(ctx->device));
-    int rc = dz_set_samples_const(ctx);
-    if (rc) return rc;
+    int rc = DAISY_OK;
     uint64_t *d = nullptr;
     size_t bytes = sizeof(uint64_t) * (size_t)nrows * ctx->N;
     DZ_CUDA(cudaMalloc(&d, bytes));

@@ -230,7 +230,9 @@ int dz_csc_export(daisy_ctx *const *ctx, int n, int64_t *nnz, float *values, int
         std::vector<int64_t> s(outer.begin(), outer.end() - 1);
         for (int g = 0; g < n; g++) {
             CSC_CUDA(mem.alloc(ctx[g]->device, (void **)&start[(size_t)g], sizeof(int64_t) * (size_t)N), what);
-            CSC_CUDA(cudaMemcpy(start[(size_t)g], s.data(), sizeof(int64_t) * (size_t)N, cudaMemcpyHostToDevice), what);
+            CSC_CUDA(cudaSetDevice(ctx[g]->device), what);
+            CSC_CUDA(cudaMemcpyAsync(start[(size_t)g], s.data(), sizeof(int64_t) * (size_t)N, cudaMemcpyHostToDevice, ctx[g]->stream), what);
+            CSC_CUDA(cudaStreamSynchronize(ctx[g]->stream), what); // `s` is pageable host memory, advanced below
             for (int c = 0; c < N; c++) s[(size_t)c] += h_cnt[(size_t)g][(size_t)c];
         }
     }

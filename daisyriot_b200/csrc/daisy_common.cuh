@@ -290,7 +290,6 @@ struct daisy_ctx {
     int rank = 0, nranks = 1, rows_per_rank = 0, row0 = 0, row1 = 0;
     int S = 0;
     float h_uv[2 * DAISY_MAX_SAMPLES];
-    int n_nonedge = 0;     // samples [0, n_nonedge) of the device-side (permuted) pattern lie well inside the triangle
     // device mesh
     float *d_vertices = nullptr, *d_normals = nullptr;
     int *d_tri = nullptr;
@@ -373,7 +372,6 @@ int dz_launch_closest(daisy_ctx *ctx, int n, const float *d_rays, daisy_hit *d_h
 int dz_precompute_geom(daisy_ctx *ctx);                              // formfactor.cu
 int dz_build_faces(daisy_ctx *c, const float *vertices, const int32_t *tri_idx, int ntri, std::vector<int> &pid); // faces.cu
 void dz_free_faces(daisy_ctx *c);                                    // faces.cu
-int dz_set_samples_const(daisy_ctx *ctx);                            // formfactor.cu
 int dz_unoccluded_rows(daisy_ctx *ctx, int variant, int row0, int nrows, daisy_tripl *d_out); // formfactor.cu
 struct daisy_solver;
 // same-process peers (daisy_group): device pointers handed over directly, peer access enabled by the caller

@@ -335,9 +335,10 @@ int dz_build_faces(daisy_ctx *c, const float *vertices, const int32_t *tri_idx, 
     DZ_CUDA(cudaMalloc(&c->d_faces, sizeof(DzFace) * faces.size()));
     DZ_CUDA(cudaMalloc(&c->d_face_cells, sizeof(int) * cells.size()));
     DZ_CUDA(cudaMalloc(&c->d_face_lists, sizeof(int) * (lists.empty() ? 1 : lists.size())));
-    DZ_CUDA(cudaMemcpy(c->d_faces, faces.data(), sizeof(DzFace) * faces.size(), cudaMemcpyHostToDevice));
-    DZ_CUDA(cudaMemcpy(c->d_face_cells, cells.data(), sizeof(int) * cells.size(), cudaMemcpyHostToDevice));
-    if (!lists.empty()) DZ_CUDA(cudaMemcpy(c->d_face_lists, lists.data(), sizeof(int) * lists.size(), cudaMemcpyHostToDevice));
+    DZ_CUDA(cudaMemcpyAsync(c->d_faces, faces.data(), sizeof(DzFace) * faces.size(), cudaMemcpyHostToDevice, c->stream));
+    DZ_CUDA(cudaMemcpyAsync(c->d_face_cells, cells.data(), sizeof(int) * cells.size(), cudaMemcpyHostToDevice, c->stream));
+    if (!lists.empty()) DZ_CUDA(cudaMemcpyAsync(c->d_face_lists, lists.data(), sizeof(int) * lists.size(), cudaMemcpyHostToDevice, c->stream));
+    DZ_CUDA(cudaStreamSynchronize(c->stream)); // the tables are pageable host memory
     c->nfaces = (int)faces.size();
     c->face_cells = (int64_t)cells.size();
     c->face_list_ints = (int64_t)lists.size();

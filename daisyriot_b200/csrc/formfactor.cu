@@ -33,32 +33,29 @@
 #define PI_F 3.14159265358979323846f
 
 // Sample pattern in DEVICE order: samples whose barycentric margin min(u, v, 1-u-v) is at least EDGE_MARGIN come first
-// ("inner" samples), the rest ("edge" samples) last; c_perm maps a device position back to the caller's sample index
+// ("inner" samples), the rest ("edge" samples) last; perm maps a device position back to the caller's sample index
 // (= bit position in the visibility mask).  Rays of inner samples leave and reach the two patches well inside them, which
-// is what lets coplanar neighbours be skipped for them (see k_tri_planes / shaft_candidates).
+// is what lets coplanar neighbours be skipped for them (see k_tri_planes / shaft_candidates).  The pattern travels in the
+// kernel's parameters, so every launch carries its own context's pattern: two contexts on one device never see each other's.
 #define EDGE_MARGIN 0.02f
-__constant__ float c_uv[2 * DAISY_MAX_SAMPLES];
-__constant__ int c_perm[DAISY_MAX_SAMPLES];
 #ifdef DAISY_FF_STATS
 __device__ unsigned long long g_ffstats[48];
 #endif
 
-int dz_set_samples_const(daisy_ctx *ctx) {
-    float uv[2 * DAISY_MAX_SAMPLES] = { 0 };
-    int perm[DAISY_MAX_SAMPLES] = { 0 };
-    int n = 0;
+// fills uv and perm (DAISY_MAX_SAMPLES entries each, zero past S) and returns the number of inner samples
+static int samples_device_order(const daisy_ctx *ctx, float *uv, unsigned char *perm) {
+    memset(uv, 0, sizeof(float) * 2 * DAISY_MAX_SAMPLES);
+    memset(perm, 0, DAISY_MAX_SAMPLES);
+    int n = 0, n_inner = 0;
     for (int pass = 0; pass < 2; pass++) {
         for (int i = 0; i < ctx->S; i++) {
             const float u = ctx->h_uv[2 * i], v = ctx->h_uv[2 * i + 1];
             const bool inner = fminf(fminf(u, v), 1.0f - u - v) >= EDGE_MARGIN;
-            if (inner == (pass == 0)) { uv[2 * n] = u; uv[2 * n + 1] = v; perm[n] = i; n++; }
+            if (inner == (pass == 0)) { uv[2 * n] = u; uv[2 * n + 1] = v; perm[n] = (unsigned char)i; n++; }
         }
-        if (pass == 0) ctx->n_nonedge = n;
+        if (pass == 0) n_inner = n;
     }
-    DZ_CUDA(cudaMemcpyToSymbolAsync(c_uv, uv, sizeof(uv), 0, cudaMemcpyHostToDevice, ctx->stream));
-    DZ_CUDA(cudaMemcpyToSymbolAsync(c_perm, perm, sizeof(perm), 0, cudaMemcpyHostToDevice, ctx->stream));
-    DZ_CUDA(cudaStreamSynchronize(ctx->stream));
-    return DAISY_OK;
+    return n_inner;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -981,6 +978,8 @@ struct FFParams {
     // update runs (PARTIAL, see dz_build_formfactors): the dirty set and, per job, the dirty clusters its tile's shaft meets
     DzUpdate upd;
     const int *tile_dirty; // (UPD_CAP + 1) ints per job: count (-1 = more than UPD_CAP: every pair of the tile is dirty), cluster ids
+    float uv[2 * DAISY_MAX_SAMPLES];      // sample pattern in device order (samples_device_order)
+    unsigned char perm[DAISY_MAX_SAMPLES]; // device position -> caller's sample index
 };
 
 // Tile slots: [0, 64) = the row-tile's patches, [64, 128) = the column-tile's patches.  A listed pair is (rl, cl) plus a
@@ -1037,8 +1036,8 @@ __global__ void __launch_bounds__(FF_THREADS, FF_MINBLOCKS) k_ff_tiles(FFParams 
     int &s_nlist = sm.nlist, &s_next = sm.next, &s_job = sm.job, &s_nown = sm.nown, &s_nheavy = sm.nheavy, &s_hnext = sm.hnext;
     const int tid = threadIdx.x;
     const int lane = tid & 31;
-    if (tid < 2 * DAISY_MAX_SAMPLES) sm.uv[tid] = c_uv[tid];
-    if (tid < DAISY_MAX_SAMPLES) sm.perm[tid] = (unsigned char)c_perm[tid];
+    if (tid < 2 * DAISY_MAX_SAMPLES) sm.uv[tid] = P.uv[tid];
+    if (tid < DAISY_MAX_SAMPLES) sm.perm[tid] = P.perm[tid];
     int *my_cand = P.scratch + ((size_t)blockIdx.x * FF_THREADS + tid) * SHAFT_CAP;
     int *warp_cand = P.scratch + ((size_t)blockIdx.x * FF_THREADS + (tid & ~31)) * SHAFT_CAP;
 #ifdef DAISY_FF_STATS
@@ -1371,7 +1370,7 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
     FFParams P;
     P.geom = ctx->d_geom; P.tv = ctx->d_triverts; P.tribox = ctx->d_tribox; P.scratch = nullptr; P.nodes = ctx->d_nodes; P.root = ctx->root; P.N = N; P.S = ctx->S;
     P.order = ctx->d_order;
-    P.plane = ctx->d_plane; P.pid = ctx->d_pid; P.nbr = ctx->d_nbr; P.n_inner = ctx->n_nonedge;
+    P.plane = ctx->d_plane; P.pid = ctx->d_pid; P.nbr = ctx->d_nbr; P.n_inner = samples_device_order(ctx, P.uv, P.perm);
     P.faces = ctx->d_faces; P.face_cells = ctx->d_face_cells; P.face_lists = ctx->d_face_lists; P.nfaces = ctx->nfaces; P.face_tm = 4.0f * ctx->pad;
     P.face_ncells = ctx->face_cells; P.face_nlist = ctx->face_list_ints;
 
@@ -1446,7 +1445,8 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
 #ifdef DAISY_FF_STATS
     {
         unsigned long long h[48];
-        cudaMemcpyFromSymbol(h, g_ffstats, sizeof(h));
+        cudaMemcpyFromSymbolAsync(h, g_ffstats, sizeof(h), 0, cudaMemcpyDeviceToHost, st);
+        cudaStreamSynchronize(st);
         const char *nm[4] = { "simple(n_main=0)", "occluded", "visible", "partial" };
         for (int c = 0; c < 4; c++)
             fprintf(stderr, "ffstats %-18s pairs %12llu  mean n_main %7.1f  mean n_ring %6.1f\n", nm[c], h[c], h[c] ? (double)h[4 + c] / h[c] : 0.0, h[c] ? (double)h[8 + c] / h[c] : 0.0);
@@ -1464,7 +1464,8 @@ int dz_build_formfactors(daisy_ctx *ctx, int variant, uint64_t *d_masks, int mro
             for (int i = 0; i < 7; i++) fprintf(stderr, "ffstats warp-cycles %-18s %6.2f %%\n", ph[i], tot ? 100.0 * (double)h[24 + i] / (double)tot : 0.0);
         }
         unsigned long long z[48] = { 0 };
-        cudaMemcpyToSymbol(g_ffstats, z, sizeof(z));
+        cudaMemcpyToSymbolAsync(g_ffstats, z, sizeof(z), 0, cudaMemcpyHostToDevice, st);
+        cudaStreamSynchronize(st);
     }
 #endif
     if (write_F) { ctx->ff_ms = ms; ctx->pairs_traced = (int64_t)pairs[0]; ctx->pairs_owned = (int64_t)pairs[1]; ctx->pairs_heavy = (int64_t)pairs[2]; }

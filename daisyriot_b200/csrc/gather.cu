@@ -22,7 +22,9 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <atomic>
 #include <cmath>
+#include <mutex>
 #include <vector>
 
 #define G_WARPS 8
@@ -975,10 +977,12 @@ __global__ void k_wait_flags(unsigned long long *flags, int G, unsigned long lon
 template <int K, int R>
 static int launch_partial(daisy_solver *s, const GatherParams &P) {
     size_t smem = 2 * K * G_TC * sizeof(float) + 64;
-    static bool attr_done[64] = { false }; // per device: a function attribute belongs to the device's context
-    if (!attr_done[s->ctx->device & 63]) {
+    // per device: a function attribute belongs to the device's context.  Solvers may run from several host threads; setting
+    // the attribute twice is harmless, a torn flag is not.
+    static std::atomic<bool> attr_done[64];
+    if (!attr_done[s->ctx->device & 63].load()) {
         DZ_CUDA(cudaFuncSetAttribute(k_gather_partial<K, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_done[s->ctx->device & 63] = true;
+        attr_done[s->ctx->device & 63].store(true);
     }
     k_gather_partial<K, R><<<s->grid, G_THREADS, smem, s->ctx->stream>>>(P);
     DZ_CUDA(cudaGetLastError());
@@ -1013,10 +1017,10 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
     if (s->use_mma && (K == 16 || K == 32 || K == 64)) {
         if constexpr (K == 16 || K == 32 || K == 64) {
             constexpr size_t smem = mm_smem_bytes<K>();
-            static bool attr_done[64] = { false }; // per device
-            if (!attr_done[c->device & 63]) {
+            static std::atomic<bool> attr_done[64]; // per device
+            if (!attr_done[c->device & 63].load()) {
                 DZ_CUDA(cudaFuncSetAttribute(k_gather_mma<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                attr_done[c->device & 63] = true;
+                attr_done[c->device & 63].store(true);
             }
             k_split_residual<K><<<(s->ncolsP + 255) / 256, 256, 0, c->stream>>>(s->d_res[s->cur], s->bstride, s->n, s->G * s->n, s->ncolsP, s->d_split, P.stop);
             DZ_CUDA(cudaGetLastError());
@@ -1034,10 +1038,10 @@ static int launch_pass_K(daisy_solver *s, unsigned long long wait_seq, const Dev
         // restart mode runs the ABS instantiation; only the fused epilogue reads it (otherwise the epilogue warps return at once)
         const bool abs_kernel = s->abs_sums && s->fused_epi;
         auto kern = abs_kernel ? k_gather_tma<K, true> : k_gather_tma<K, false>;
-        static bool attr_done[2][64] = { { false } }; // per instantiation and device
-        if (!attr_done[abs_kernel][c->device & 63]) {
+        static std::atomic<bool> attr_done[2][64]; // per instantiation and device
+        if (!attr_done[abs_kernel][c->device & 63].load()) {
             DZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            attr_done[abs_kernel][c->device & 63] = true;
+            attr_done[abs_kernel][c->device & 63].store(true);
         }
         P.nrb = s->nrb_tma; // (nloc + tma_rows<K>() - 1) / tma_rows<K>(), and 1 for a rank without rows (plan())
         P.sk = s->fused_epi ? 1 : 0; P.sk_S = s->sk_S; P.sk_L = s->sk_L; P.sk_total = s->sk_total;
@@ -1138,13 +1142,14 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
                                     const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static PFN_encodeTiled get_encode() {
+    static std::once_flag once; // solvers may be created from several host threads
     static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
+    std::call_once(once, [] {
         void *p = nullptr;
         cudaDriverEntryPointQueryResult q;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
             fn = (PFN_encodeTiled)p;
-    }
+    });
     return fn;
 }
 
@@ -1360,8 +1365,9 @@ static int scan_and_plan(daisy_solver *s) {
         DZ_CUDA(cudaMalloc(&s->d_partial, sizeof(float) * (size_t)sp.maxp * (s->nloc > 0 ? s->nloc : 1) * s->Kp));
         s->partial_splits = sp.maxp;
     }
-    DZ_CUDA(cudaMemcpy(s->d_sk_list, sp.list.data(), sizeof(int) * sp.list.size(), cudaMemcpyHostToDevice));
-    DZ_CUDA(cudaMemcpy(s->d_sk_off, sp.off.data(), sizeof(int) * sp.off.size(), cudaMemcpyHostToDevice));
+    DZ_CUDA(cudaMemcpyAsync(s->d_sk_list, sp.list.data(), sizeof(int) * sp.list.size(), cudaMemcpyHostToDevice, st));
+    DZ_CUDA(cudaMemcpyAsync(s->d_sk_off, sp.off.data(), sizeof(int) * sp.off.size(), cudaMemcpyHostToDevice, st));
+    DZ_CUDA(cudaStreamSynchronize(st)); // `sp` is pageable host memory
     s->sk_total = sp.total; s->sk_grid = sp.grid; s->sk_L = sp.L; s->sk_maxp = sp.maxp;
     s->occupied = sp.occupied;
     s->pin16 = pin16_for(s, (double)sp.occupied * trows * tcols * 4.0); // the bytes a pass actually streams
@@ -1446,6 +1452,7 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     for (int p = 0; p < ctx->N; p++)
         DZ_REQUIRE(mat_idx[p] >= 0 && mat_idx[p] < nmat, DAISY_E_INVALID, "daisy_solver_create: material index out of range");
     DZ_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
     daisy_solver *s = new daisy_solver();
     s->ctx = ctx; s->mesh_version = ctx->mesh_version; s->K = K; s->Kp = padded_K(K); s->nmat = s->nmat_cap = nmat;
     s->N = ctx->N; s->n = ctx->rows_per_rank; s->G = ctx->nranks; s->rank = ctx->rank;
@@ -1467,13 +1474,13 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     SC(cudaMalloc(&s->d_partial, sizeof(float) * (size_t)s->partial_splits * (s->nloc > 0 ? s->nloc : 1) * s->Kp));
     SC(cudaMalloc(&s->d_cta_sums, sizeof(double) * 148 * s->Kp));
     SC(cudaMalloc(&s->d_done, sizeof(unsigned int)));
-    SC(cudaMemset(s->d_done, 0, sizeof(unsigned int)));
+    SC(cudaMemsetAsync(s->d_done, 0, sizeof(unsigned int), st));
     {
         const int trows = (s->Kp == 32) ? 32 : 64; // = tma_rows<Kp>()
         s->nrb_tma = (s->nloc + trows - 1) / trows;
         if (s->nrb_tma < 1) s->nrb_tma = 1; // a rank without rows runs one row block over zero rows (plan())
         SC(cudaMalloc(&s->d_rb_arrive, sizeof(unsigned int) * (size_t)s->nrb_tma));
-        SC(cudaMemset(s->d_rb_arrive, 0, sizeof(unsigned int) * (size_t)s->nrb_tma));
+        SC(cudaMemsetAsync(s->d_rb_arrive, 0, sizeof(unsigned int) * (size_t)s->nrb_tma, st));
         SC(cudaMalloc(&s->d_rb_sums, sizeof(double) * (size_t)s->nrb_tma * s->Kp));
         SC(cudaHostAlloc(reinterpret_cast<void **>(&s->h_abort), sizeof(unsigned long long), cudaHostAllocMapped));
         *s->h_abort = 0ull;
@@ -1482,9 +1489,9 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
         if (e && atof(e) > 0.0) s->timeout_ns = (unsigned long long)(atof(e) * 1e6);
     }
     SC(cudaMalloc(&s->d_flags, sizeof(unsigned long long) * 17));
-    SC(cudaMemset(s->d_flags, 0, sizeof(unsigned long long) * 17));
-    SC(cudaMemset(s->d_res[0], 0, exb));
-    SC(cudaMemset(s->d_res[1], 0, exb));
+    SC(cudaMemsetAsync(s->d_flags, 0, sizeof(unsigned long long) * 17, st));
+    SC(cudaMemsetAsync(s->d_res[0], 0, exb, st));
+    SC(cudaMemsetAsync(s->d_res[1], 0, exb, st));
     SC(cudaEventCreate(&s->e0));
     SC(cudaEventCreate(&s->e1));
     if (s->use_mma) {
@@ -1493,18 +1500,15 @@ extern "C" int daisy_solver_create(daisy_ctx *ctx, int K, const float *E, const 
     }
     if (s->use_tma) { int mrc = make_maps(s); if (mrc) { free_solver(s); return mrc; } }
     {
-        std::vector<float> ex;
+        std::vector<float> ex, Mp;
         to_exchange(s, E, ex);
-        SC(cudaMemcpy(s->d_E, ex.data(), exb, cudaMemcpyHostToDevice));
-        std::vector<float> Mp;
+        SC(cudaMemcpyAsync(s->d_E, ex.data(), exb, cudaMemcpyHostToDevice, st));
         pad_materials(s, M, nmat, Mp);
-        SC(cudaMemcpy(s->d_M, Mp.data(), sizeof(float) * Mp.size(), cudaMemcpyHostToDevice));
-        if (s->nloc > 0) SC(cudaMemcpy(s->d_mat, mat_idx + s->row0, sizeof(int) * (size_t)s->nloc, cudaMemcpyHostToDevice));
+        SC(cudaMemcpyAsync(s->d_M, Mp.data(), sizeof(float) * Mp.size(), cudaMemcpyHostToDevice, st));
+        if (s->nloc > 0) SC(cudaMemcpyAsync(s->d_mat, mat_idx + s->row0, sizeof(int) * (size_t)s->nloc, cudaMemcpyHostToDevice, st));
+        SC(cudaStreamSynchronize(st)); // `ex` and `Mp` are pageable host memory
     }
 #undef SC
-    // the set-up above used synchronous copies and legacy-stream memsets; the solver's kernels run on ctx->stream, which may be
-    // a non-blocking stream (daisy_ctx_set_stream): make sure everything has landed before anything is enqueued there
-    { cudaError_t e_ = cudaDeviceSynchronize(); if (e_ != cudaSuccess) { daisy_set_error("daisy_solver_create: %s", cudaGetErrorString(e_)); free_solver(s); return DAISY_E_CUDA; } }
     if (s->skip) { rc = scan_and_plan(s); if (rc) { free_solver(s); return rc; } }
     compute_sums_from_host(s, E);
     s->e_sums = s->sums;

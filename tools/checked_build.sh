@@ -16,3 +16,4 @@ timeout 1800 python -m pytest tests/test_gpu_matrix_cache.py -x -q -m gpu 2>&1 |
 timeout 1800 python -m pytest tests/test_gpu_wide_bands.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_ff_limits.py -x -q -m gpu 2>&1 | tail -4
 timeout 1800 python -m pytest tests/test_gpu_warm_restart.py -x -q -m gpu -k "not group" 2>&1 | tail -4
+timeout 1800 python -m pytest tests/test_gpu_streams.py -x -q -m gpu 2>&1 | tail -4
